@@ -90,8 +90,8 @@ __device__ __forceinline__ void fused_rgb_epilogue(const LayerArgs& a, const uin
         const float t = apply_act(__fadd_rn(__fmaf_rn(u[col], 1.0f / 2048.0f, v[col]), bias3[c]), a.act);
         y[px * 3 + c] = tic_denorm_clip(t, a.mean[c], a.stdv[c]);
       }
-    if (a.out_mode == IO_DENORM_U8 && X + 1 < g.W && !(off & 1)) {
-      // both pixels inside the image and 2-byte aligned (X is even: any even W): three 2-byte stores
+    if (a.out_mode == IO_DENORM_U8 && X + 1 < g.W && !((reinterpret_cast<uintptr_t>(a.out) + off) & 1)) {
+      // both pixels inside the image and 2-byte aligned (X is even: any even W, and an even base address): three 2-byte stores
       uint32_t q[6];
 #pragma unroll
       for (int i = 0; i < 6; ++i) q[i] = (uint32_t)(int)rintf(y[i]);

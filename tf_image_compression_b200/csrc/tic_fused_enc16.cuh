@@ -559,11 +559,20 @@ fused_enc_kernel(const __grid_constant__ CUtensorMap tm_img, const __grid_consta
   }
 }
 
+// The builders' operand is the exact integer x - m_c with m_c = round(mean_c): it must stay inside the exact fp16 integer
+// range the weight image was laid out for.
+inline bool fused_enc_mean_ok(float mean) {
+  const long m = lrintf(mean);
+  return m >= -768 && m <= 1023;
+}
+
 // Which layer pairs take the fused kernel: the u8 image through conv 3 -> 32 stride 2 (TMA-fed windowed first layer)
-// followed by conv 32 -> 32 stride 2 into pair planes.
+// followed by conv 32 -> 32 stride 2 into pair planes.  Other channel means take the first-layer + u16 kernels.
 inline bool fused_enc_supported(const LayerArgs& a1, int kind1, int stride1, const LayerArgs& a2, int kind2, int stride2) {
   if (kind1 != 0 || kind2 != 0 || stride1 != 2 || stride2 != 2) return false;
   if (a1.in_mode != IO_U8_NORM || a1.cin != 3 || a1.cout != 32 || a2.cin != 32 || a2.cout != 32) return false;
+  for (int c = 0; c < 3; ++c)
+    if (!fused_enc_mean_ok(a1.mean[c])) return false;
   if (a1.res || a2.res || a2.out_mode != IO_ACT16) return false;
   if (a1.hin != a1.win || a1.hin % 64 != 0 || a1.hin / 32 > kFusedMaxTilesX) return false;
   if (a1.hout * 2 != a1.hin || a2.hin != a1.hout || a2.hout * 2 != a2.hin || a2.wout * 2 != a2.win) return false;
@@ -601,7 +610,7 @@ inline int launch_fused_enc(cudaStream_t stream, const LayerArgs& a1, const Laye
     nm.mean[c] = a1.mean[c];
     nm.stdv[c] = a1.stdv[c];
     nm.m[c] = (int)lrintf(a1.mean[c]);
-    if (nm.m[c] < -768 || nm.m[c] > 1023) return fail("fused encoder: channel mean outside the exact fp16 integer range", -5);
+    if (!fused_enc_mean_ok(a1.mean[c])) return fail("fused encoder: channel mean outside the exact fp16 integer range", -5);
   }
   if (!fw->w1 || memcmp(&fw->nm, &nm, sizeof(nm)) != 0) {
     // (a rebuild on the same stream is ordered behind the launches that still read the old image)

@@ -232,8 +232,9 @@ __device__ __forceinline__ void store_pixel(const LayerArgs& a, int n, int y, in
     case IO_QUANT_U8:
     case IO_QUANT_F32: {
       const long long gp = (((long long)a.geo.n0 + n) * a.hout + y) * a.wout + x;
-      if (a.out_mode == IO_QUANT_U8 && NV == 16 && oc + NV <= a.cout && (a.cout & 15) == 0) {
-        // 16 symbols of one pixel are 16 consecutive bytes of the symbol tensor: one 16-byte store
+      if (a.out_mode == IO_QUANT_U8 && NV == 16 && oc + NV <= a.cout && (a.cout & 15) == 0 &&
+          (reinterpret_cast<uintptr_t>(a.out) & 15) == 0) {
+        // 16 symbols of one pixel are 16 consecutive bytes of a 16-byte aligned symbol tensor: one 16-byte store
         uint32_t w[4] = {0u, 0u, 0u, 0u};
 #pragma unroll
         for (int i = 0; i < NV; ++i) {

@@ -367,8 +367,8 @@ __device__ __forceinline__ void u16_epilogue_tile(const LayerArgs& a, const int 
       const int Y = g.oy + (int)gy * g.P + 2 * yt + half, X = g.ox + (int)gx * g.P + 2 * xt;
       if (Y >= g.H) return;
       const long long off = (((long long)img * g.H + Y) * g.W + X) * 3;
-      if (a.out_mode == IO_DENORM_U8 && X + 1 < g.W && !(off & 1)) {
-        // both pixels inside the image and 2-byte aligned (X is even: any even W): three 2-byte stores instead of six bytes
+      if (a.out_mode == IO_DENORM_U8 && X + 1 < g.W && !((reinterpret_cast<uintptr_t>(a.out) + off) & 1)) {
+        // both pixels inside the image and 2-byte aligned (X is even: any even W, and an even base address): three 2-byte stores instead of six bytes
         uint32_t q[6];
 #pragma unroll
         for (int px = 0; px < 2; ++px)
