@@ -192,6 +192,21 @@ int tic_entropy_encode(tic_codec* h, const uint8_t* symbols, int64_t n_streams, 
 int tic_entropy_decode(tic_codec* h, const uint8_t* in, int64_t n_streams, int64_t in_stride, const int64_t* in_bytes,
                        const uint32_t* cum_freq, int n_cum, uint8_t* symbols, int64_t stream_len, int mem);
 
+/* ---- rate-distortion evaluation ------------------------------------------ */
+/* encode.py -> decode.py -> processing_utils/evaluate.py (scipt_bash/encode_decode_evaluate.sh) without files:
+ * images [n_images,H,W,3] u8 -> code_bytes[i] = stored length of image i's range-coded stream (== tic_entropy_encode's
+ * out_bytes == the size of the file entry.compress writes), sq_err[i] = sum over H*W*3 of (recon - image)^2 with recon
+ * the u8 reconstruction tic_decode_images(TIC_U8) returns; recon may be NULL (not written).  cum_freq: host array, as in
+ * tic_entropy_encode.  mem applies to images, code_bytes, sq_err and recon.
+ * Chunks of whole images run encoder -> range coder (lengths only) -> decoder -> squared error on the device; symbols,
+ * reconstructions and squared errors stay in HBM.  Host buffers: the H2D of chunk i+1 overlaps the kernels of chunk i
+ * (as in tic_roundtrip_images), the per-image results come back once at the end, errors are returned.  Device buffers:
+ * asynchronous on the handle's stream; a symbol outside the table or of zero probability surfaces at tic_check_status.
+ * The symbol histogram accumulates as on every encoder call.  n_images == 0 writes nothing. */
+int tic_evaluate_images(tic_codec* h, const uint8_t* images, int64_t n_images, int H, int W, int P,
+                        const uint32_t* cum_freq, int n_cum, int64_t* code_bytes, uint64_t* sq_err,
+                        uint8_t* recon, int mem);
+
 /* ---- introspection (measurement) ----------------------------------------- */
 /* Kernels launched by this handle since creation (bench.py's gpu_launches). */
 int64_t tic_launch_count(const tic_codec* h);

@@ -60,6 +60,8 @@ SIGNATURES = {
                                      C.c_void_p, C.c_int]),
     "tic_entropy_decode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                      C.c_int64, C.c_int]),
+    "tic_evaluate_images": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int,
+                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "tic_launch_count": (C.c_int64, [C.c_void_p]),
     "tic_last_kernel_ms": (C.c_float, [C.c_void_p]),
     "tic_profile_enable": (C.c_int, [C.c_void_p, C.c_int]),

@@ -471,6 +471,37 @@ class Codec:
                                                 int(stream_len), src.mem))
         return out
 
+    # ---- rate-distortion evaluation -------------------------------------------------------------
+    def evaluate_images(self, images, patch_size, cum_freq, out=None):
+        """encode.py -> decode.py -> processing_utils/evaluate.py on the device, without files: [B,H,W,3] uint8 ->
+        (code_bytes int64[B], sq_err uint64[B], out | None).  code_bytes[i] is the size of the range-coded file of image i
+        (entropy_encode's nbytes, entry.compress's file), sq_err[i] the integer sum of squared differences between image i
+        and its uint8 reconstruction (decode_images), written to `out` [B,H,W,3] uint8 when one is given.  CUDA tensors in
+        give CUDA tensors out (sq_err as int64; asynchronous, errors surface through check_status())."""
+        if images.ndim == 3:
+            images = images[None]
+        B, H, W = int(images.shape[0]), int(images.shape[1]), int(images.shape[2])
+        if tuple(images.shape[3:]) != (3,):
+            raise ValueError(f"images must be [B,H,W,3], got {tuple(images.shape)}")
+        src = _Buf(images, np.uint8, self.device, self)
+        cum = np.ascontiguousarray(np.asarray([int(v) for v in cum_freq], dtype=np.uint32))
+        dst = None
+        if out is not None:
+            self._expect_shape("out", out, (B, H, W, 3))
+            dst = _Buf(out, np.uint8, self.device)
+            if dst.mem != src.mem:
+                raise ValueError("input and output must both be host or both be device buffers")
+        if _is_torch(images) and images.is_cuda:
+            code_bytes = torch.zeros(B, dtype=torch.int64, device=images.device)
+            sq_err = torch.zeros(B, dtype=torch.int64, device=images.device)
+            cb_ptr, se_ptr = code_bytes.data_ptr(), sq_err.data_ptr()
+        else:
+            code_bytes, sq_err = np.zeros(B, dtype=np.int64), np.zeros(B, dtype=np.uint64)
+            cb_ptr, se_ptr = code_bytes.ctypes.data, sq_err.ctypes.data
+        self._check(self.lib.tic_evaluate_images(self._h, src.ptr, B, H, W, int(patch_size), cum.ctypes.data, cum.size, cb_ptr,
+                                                 se_ptr, dst.ptr if dst is not None else None, src.mem))
+        return code_bytes, sq_err, out
+
     def check_status(self):
         """Synchronise the codec's stream and raise if a tensor-mode ('f16x3') run left the fp16 range (|activation| >=
         65504): device-buffer calls are asynchronous, so their status surfaces here or at the next call."""

@@ -17,6 +17,7 @@
 #include "tic_fused16.cuh"
 #include "tic_fused_enc16.cuh"
 #include "tic_entropy.cuh"
+#include "tic_eval.cuh"
 
 using namespace tic;
 
@@ -92,6 +93,8 @@ struct tic_codec {
   uint8_t* d_seg = nullptr;         // entropy stage: worst-case slots of a segmented call's pieces (grow-only)
   long long* d_seg_bytes = nullptr; //   and their stored lengths
   int64_t seg_cap = 0;              //   pieces both hold
+  long long* d_eval = nullptr;      // tic_evaluate_images with host buffers: per-image stored lengths, then squared errors
+  int64_t eval_cap = 0;             //   images it holds (grow-only)
   cudaEvent_t ev_switch = nullptr;  // orders the old stream before the new one in tic_set_stream
   std::string err;
 };
@@ -692,6 +695,30 @@ std::vector<int64_t> host_chunk_schedule(int64_t units, int64_t cap, double patc
   return out;
 }
 
+// Device-buffer calls have no staging to overlap with: fewer, longer launch sequences (up to 16384 patches of 128x128
+// each), equal-sized.
+std::vector<int64_t> device_chunk_schedule(int64_t units, int64_t cap) {
+  cap *= 4;
+  const int64_t upc = (units + (units + cap - 1) / cap - 1) / ((units + cap - 1) / cap);
+  std::vector<int64_t> out;
+  for (int64_t u0 = 0; u0 < units; u0 += upc) out.push_back(std::min<int64_t>(upc, units - u0));
+  return out;
+}
+
+// Both buffers of a staging set hold at least `need` bytes (grow-only; the device is drained before a buffer is freed).
+int grow_pair(tic_codec* h, void** bufs, size_t* have, size_t need) {
+  if (*have >= need) return TIC_OK;
+  TIC_CUDA(h, cudaDeviceSynchronize());
+  for (int b = 0; b < 2; ++b) {
+    if (bufs[b]) cudaFree(bufs[b]);
+    bufs[b] = nullptr;
+  }
+  *have = 0;
+  for (int b = 0; b < 2; ++b) TIC_CUDA(h, cudaMalloc(&bufs[b], need));
+  *have = need;
+  return TIC_OK;
+}
+
 // Generic chunked driver.  `units` are processed `upc` (units per chunk) at a time; a unit is a
 // patch or a whole image.  in_unit_bytes / out_unit_bytes describe the caller's buffers; run()
 // executes one chunk given device pointers (chunk-local when staged from host) and the unit offset.
@@ -703,12 +730,11 @@ int drive(tic_codec* h, int mem, const void* in, void* out, int64_t units, int64
   if (int st = overflow_status(h)) return st;
   TIC_CUDA(h, cudaEventRecord(h->ev_t0, h->stream));
   if (mem == TIC_MEM_DEVICE) {
-    upc *= 4;  // no staging to overlap with: fewer, longer launch sequences (up to 16384 patches of 128x128 each)
-    upc = (units + (units + upc - 1) / upc - 1) / ((units + upc - 1) / upc);  // equal-sized sequences
-    for (int64_t u0 = 0; u0 < units; u0 += upc) {
-      int64_t nu = std::min<int64_t>(upc, units - u0);
+    int64_t u0 = 0;
+    for (const int64_t nu : device_chunk_schedule(units, upc)) {
       int rc = run(in, out, u0, nu, /*local=*/false);
       if (rc != TIC_OK) return rc;
+      u0 += nu;
     }
     TIC_CUDA(h, cudaEventRecord(h->ev_t1, h->stream));
     return TIC_OK;
@@ -903,6 +929,7 @@ void tic_destroy(tic_codec* h) {
   if (h->d_cum) cudaFree(h->d_cum);
   if (h->d_seg) cudaFree(h->d_seg);
   if (h->d_seg_bytes) cudaFree(h->d_seg_bytes);
+  if (h->d_eval) cudaFree(h->d_eval);
   if (h->ev_switch) cudaEventDestroy(h->ev_switch);
   if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
   if (h->s_h2d) cudaStreamDestroy(h->s_h2d);
@@ -1238,21 +1265,9 @@ int tic_roundtrip_images(tic_codec* h, const uint8_t* images, int64_t n_images, 
   const size_t img_unit = (size_t)H * W * 3;
   const size_t sym_unit = (size_t)ppi * hb * wb * cb;
   const size_t rec_unit = img_unit * (out_dtype == TIC_U8 ? 1 : 4);
-  auto grow = [&](void** bufs, size_t* have, size_t need) -> int {
-    if (*have >= need) return TIC_OK;
-    TIC_CUDA(h, cudaDeviceSynchronize());
-    for (int b = 0; b < 2; ++b) {
-      if (bufs[b]) cudaFree(bufs[b]);
-      bufs[b] = nullptr;
-    }
-    *have = 0;
-    for (int b = 0; b < 2; ++b) TIC_CUDA(h, cudaMalloc(&bufs[b], need));
-    *have = need;
-    return TIC_OK;
-  };
-  if ((rc = grow(h->stage_in, &h->stage_in_bytes, (size_t)ipc * img_unit)) != TIC_OK) return rc;
-  if ((rc = grow(h->stage_sym, &h->stage_sym_bytes, (size_t)ipc * sym_unit)) != TIC_OK) return rc;
-  if ((rc = grow(h->stage_out, &h->stage_out_bytes, (size_t)ipc * rec_unit)) != TIC_OK) return rc;
+  if ((rc = grow_pair(h, h->stage_in, &h->stage_in_bytes, (size_t)ipc * img_unit)) != TIC_OK) return rc;
+  if ((rc = grow_pair(h, h->stage_sym, &h->stage_sym_bytes, (size_t)ipc * sym_unit)) != TIC_OK) return rc;
+  if ((rc = grow_pair(h, h->stage_out, &h->stage_out_bytes, (size_t)ipc * rec_unit)) != TIC_OK) return rc;
   // Three streams, two staging sets: H2D of chunk i+1 (one PCIe direction) runs under the kernels of chunk i and
   // the D2H of chunk i-1 (the other direction).
   if (int st = overflow_status(h)) return st;
@@ -1557,13 +1572,35 @@ int tic_profile_read(tic_codec* h, int graph, float* ms, int64_t* launches, int 
 // ---- GPU entropy stage ------------------------------------------------------------------------
 int64_t tic_entropy_bound(int64_t stream_len) { return (tic_rc_bound(stream_len < 0 ? 0 : stream_len) + 15) & ~(int64_t)15; }
 
-static int entropy_table(tic_codec* h, const uint32_t* cum, int n_cum) {
+static int entropy_table_check(tic_codec* h, const uint32_t* cum, int n_cum) {
   if (!cum || n_cum < 2 || n_cum - 1 > kEntropyMaxSymbols) return fail(h, TIC_ERR_INVALID, "entropy stage: tables of 1..256 symbols");
   if (cum[0] != 0) return fail(h, TIC_ERR_INVALID, "entropy stage: cumulative frequencies must start at 0");
   for (int i = 1; i < n_cum; ++i)
     if (cum[i] < cum[i - 1]) return fail(h, TIC_ERR_INVALID, "entropy stage: cumulative frequencies must not decrease");
   if (cum[n_cum - 1] == 0 || cum[n_cum - 1] > TIC_RC_MAX_TOTAL) return fail(h, TIC_ERR_INVALID, "entropy stage: frequency total must be in [1, 65536]");
+  return TIC_OK;
+}
+
+static int entropy_table(tic_codec* h, const uint32_t* cum, int n_cum) {
+  int rc = entropy_table_check(h, cum, n_cum);
+  if (rc != TIC_OK) return rc;
   TIC_CUDA(h, cudaMemcpyAsync(h->d_cum, cum, (size_t)n_cum * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+  return TIC_OK;
+}
+
+// Grow-only scratch of `pieces` worst-case segment slots and their stored lengths.  The stream is drained first: earlier
+// calls may still be reading the old buffer.
+static int ensure_seg_scratch(tic_codec* h, int64_t pieces) {
+  if (pieces <= h->seg_cap) return TIC_OK;
+  TIC_CUDA(h, cudaStreamSynchronize(h->stream));
+  if (h->d_seg) cudaFree(h->d_seg);
+  if (h->d_seg_bytes) cudaFree(h->d_seg_bytes);
+  h->d_seg = nullptr;
+  h->d_seg_bytes = nullptr;
+  h->seg_cap = 0;
+  TIC_CUDA(h, cudaMalloc(&h->d_seg, (size_t)(pieces * kEntropySegSlot)));
+  TIC_CUDA(h, cudaMalloc(&h->d_seg_bytes, (size_t)pieces * sizeof(long long)));
+  h->seg_cap = pieces;
   return TIC_OK;
 }
 
@@ -1593,18 +1630,7 @@ int tic_entropy_encode(tic_codec* h, const uint8_t* symbols, int64_t n_streams, 
   }
   const int64_t nseg = tic_rc_segments(stream_len);
   if (nseg > 0x7fffffffLL / std::max<int64_t>(1, n_streams)) return fail(h, TIC_ERR_INVALID, "too many segments");
-  if (nseg > 0 && n_streams * nseg > h->seg_cap) {
-    // grow-only scratch: the stream is drained first, earlier calls may still be packing out of the old buffer
-    TIC_CUDA(h, cudaStreamSynchronize(h->stream));
-    if (h->d_seg) cudaFree(h->d_seg);
-    if (h->d_seg_bytes) cudaFree(h->d_seg_bytes);
-    h->d_seg = nullptr;
-    h->d_seg_bytes = nullptr;
-    h->seg_cap = 0;
-    TIC_CUDA(h, cudaMalloc(&h->d_seg, (size_t)(n_streams * nseg * kEntropySegSlot)));
-    TIC_CUDA(h, cudaMalloc(&h->d_seg_bytes, (size_t)(n_streams * nseg) * sizeof(long long)));
-    h->seg_cap = n_streams * nseg;
-  }
+  if (nseg > 0 && (rc = ensure_seg_scratch(h, n_streams * nseg)) != TIC_OK) return rc;
   TIC_CUDA(h, cudaEventRecord(h->ev_t0, h->stream));
   if (nseg == 0) {
     rc_encode_kernel<<<(unsigned)n_streams, 32, 0, h->stream>>>(dsym, stream_len, stream_len, 1, h->d_cum, n_cum, dout, out_stride, dbytes,
@@ -1689,6 +1715,167 @@ int tic_entropy_decode(tic_codec* h, const uint8_t* in, int64_t n_streams, int64
   }
   if (e != cudaSuccess) return fail(h, TIC_ERR_CUDA, "entropy decode failed: %s", cudaGetErrorString(e));
   return TIC_OK;
+}
+
+// ---- rate-distortion evaluation -----------------------------------------------------------------
+int tic_evaluate_images(tic_codec* h, const uint8_t* images, int64_t n_images, int H, int W, int P, const uint32_t* cum_freq,
+                        int n_cum, int64_t* code_bytes, uint64_t* sq_err, uint8_t* recon, int mem) {
+  if (!h) return TIC_ERR_INVALID;
+  if (n_images < 0 || H <= 0 || W <= 0 || P <= 0 || (n_images > 0 && (!images || !code_bytes || !sq_err)))
+    return fail(h, TIC_ERR_INVALID, "bad arguments");
+  if ((H % P != 0 && H < 2) || (W % P != 0 && W < 2)) return fail(h, TIC_ERR_INVALID, "reflect padding needs at least 2 pixels");
+  int rc = check_graph_ready(h, TIC_GRAPH_ENCODER, true);
+  if (rc != TIC_OK) return rc;
+  rc = check_graph_ready(h, TIC_GRAPH_DECODER, true);
+  if (rc != TIC_OK) return rc;
+  if (h->q < 2) return fail(h, TIC_ERR_STATE, "quantiser not configured (tic_set_quantizer)");
+  if (h->g[TIC_GRAPH_ENCODER].layers[0].d.cin != 3) return fail(h, TIC_ERR_INVALID, "encoder must take 3 channels");
+  int hb, wb, cb;
+  rc = tic_bottleneck_shape(h, P, &hb, &wb, &cb);
+  if (rc != TIC_OK) return rc;
+  Graph& gd = h->g[TIC_GRAPH_DECODER];
+  Shape so;
+  if (gd.layers[0].d.cin != cb || graph_out_shape(gd, Shape{hb, wb, cb}, &so, nullptr) != 0 || so.c != 3 || so.h != P || so.w != P)
+    return fail(h, TIC_ERR_INVALID, "decoder graph does not map the encoder's %dx%dx%d symbols back to %dx%d RGB", hb, wb, cb, P, P);
+  if ((rc = entropy_table_check(h, cum_freq, n_cum)) != TIC_OK) return rc;
+  if (n_images == 0) return TIC_OK;
+  TIC_CUDA(h, cudaSetDevice(h->device));
+  const bool host = mem == TIC_MEM_HOST;
+  const Geo g0 = image_geo(H, W, P, 0);
+  const int ppi = g0.gh * g0.gw;
+  const int64_t cap = std::max<int64_t>(1, patches_per_chunk(h, P) / ppi);
+  const std::vector<int64_t> sched =
+      host ? host_chunk_schedule(n_images, cap, (double)ppi * P * P / 16384.0) : device_chunk_schedule(n_images, cap);
+  const int64_t ipc = *std::max_element(sched.begin(), sched.end());
+  const size_t img_unit = (size_t)H * W * 3;
+  const int64_t stream_len = (int64_t)ppi * hb * wb * cb;  // one image's symbols: one range-coded stream
+  const int64_t nseg = tic_rc_segments(stream_len);
+  const int64_t npiece = std::max<int64_t>(1, nseg);
+  // A piece (one segment, or one plain stream) is a serial chain: a coder launch takes about as long as one piece, however
+  // few pieces it has (one launch per 4-image chunk of config 2 made the host-buffer call 2.5x slower, DESIGN.md §4.10).
+  // So the range coder runs over the symbols of several chunks at once: they accumulate in the symbol workspace until at
+  // least kCoderPieces pieces are pending (config 2: all 64 images, 1536 pieces, one launch) or the last chunk is encoded.
+  constexpr int64_t kCoderPieces = 2048;
+  const int64_t coder_imgs = (kCoderPieces + npiece - 1) / npiece;
+  const int64_t sym_cap = std::min<int64_t>(n_images, coder_imgs - 1 + ipc);
+  if (sym_cap * npiece > 0x7fffffffLL) return fail(h, TIC_ERR_INVALID, "too many segments");
+  if ((rc = grow_pair(h, h->stage_sym, &h->stage_sym_bytes, (size_t)sym_cap * stream_len)) != TIC_OK) return rc;
+  if (host || !recon)
+    if ((rc = grow_pair(h, h->stage_out, &h->stage_out_bytes, (size_t)ipc * img_unit)) != TIC_OK) return rc;
+  if (host) {
+    if ((rc = grow_pair(h, h->stage_in, &h->stage_in_bytes, (size_t)ipc * img_unit)) != TIC_OK) return rc;
+    if (n_images > h->eval_cap) {
+      TIC_CUDA(h, cudaStreamSynchronize(h->stream));
+      if (h->d_eval) cudaFree(h->d_eval);
+      h->d_eval = nullptr;
+      h->eval_cap = 0;
+      TIC_CUDA(h, cudaMalloc(&h->d_eval, (size_t)n_images * 2 * sizeof(long long)));
+      h->eval_cap = n_images;
+    }
+  }
+  if ((rc = ensure_seg_scratch(h, sym_cap * npiece)) != TIC_OK) return rc;
+  if (int st = overflow_status(h)) return st;
+  long long* d_bytes = host ? h->d_eval : reinterpret_cast<long long*>(code_bytes);
+  unsigned long long* d_sse = host ? reinterpret_cast<unsigned long long*>(h->d_eval + n_images) : reinterpret_cast<unsigned long long*>(sq_err);
+  // Per chunk, all on the handle's stream: encoder -> symbols -> decoder -> u8 reconstruction -> squared error against
+  // the input still in place, then (see kCoderPieces) the range coder, stored lengths only, over the pending symbols.
+  // With host buffers the staging follows tic_roundtrip_images: H2D of chunk i+1 under the kernels of chunk i, the
+  // reconstruction's D2H (when asked for) on the other side stream.  Only n_images * 16 bytes of results come back.
+  const int rc_pipe = [&]() -> int {
+  TIC_CUDA(h, cudaEventRecord(h->ev_t0, h->stream));
+  if ((rc = entropy_table(h, cum_freq, n_cum)) != TIC_OK) return rc;
+  TIC_CUDA(h, cudaMemsetAsync(d_sse, 0, (size_t)n_images * sizeof(unsigned long long), h->stream));
+  int64_t u0 = 0, p0 = 0;  // images [p0, u0) are encoded and wait for the range coder
+  for (int64_t idx = 0; idx < (int64_t)sched.size(); u0 += sched[idx], ++idx) {
+    const int b = host ? (int)(idx & 1) : 0;
+    const int64_t nu = sched[idx];
+    // chunk-local staging buffers are indexed from patch 0, the caller's device buffers from the chunk's first patch
+    const uint8_t* img = images;
+    int64_t img0 = u0;
+    uint8_t* rec = recon;
+    int64_t rec0 = u0;
+    if (host) {
+      if (idx >= 2) TIC_CUDA(h, cudaStreamWaitEvent(h->s_h2d, h->ev_enc[b], 0));  // chunk idx-2 is done with stage_in[b]
+      TIC_CUDA(h, cudaMemcpyAsync(h->stage_in[b], images + (size_t)u0 * img_unit, (size_t)nu * img_unit, cudaMemcpyHostToDevice,
+                                  h->s_h2d));
+      TIC_CUDA(h, cudaEventRecord(h->ev_in[b], h->s_h2d));
+      TIC_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_in[b], 0));
+      if (idx >= 2 && recon) TIC_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_out[b], 0));  // stage_out[b] drained
+      img = (const uint8_t*)h->stage_in[b];
+      img0 = 0;
+    }
+    if (host || !recon) {
+      rec = (uint8_t*)h->stage_out[b];
+      rec0 = 0;
+    }
+    uint8_t* sym = (uint8_t*)h->stage_sym[0] + (size_t)(u0 - p0) * stream_len;
+    IoSpec i, o;
+    i.mode = IO_U8_NORM;
+    i.in = img;
+    i.geo = image_geo(H, W, P, img0 * ppi);
+    o.mode = IO_QUANT_U8;
+    o.out = sym;
+    o.geo = image_geo(H, W, P, 0);
+    if ((rc = run_graph(h, TIC_GRAPH_ENCODER, i, o, (int)(nu * ppi), P, P)) != TIC_OK) return rc;
+    IoSpec di, dout;
+    di.mode = IO_U8_SYMLUT;
+    di.in = sym;
+    di.geo = image_geo(H, W, P, 0);
+    dout.mode = IO_DENORM_U8;
+    dout.out = rec;
+    dout.geo = image_geo(H, W, P, rec0 * ppi);
+    if ((rc = run_graph(h, TIC_GRAPH_DECODER, di, dout, (int)(nu * ppi), hb, wb)) != TIC_OK) return rc;
+    // enough blocks to keep every SM streaming (8 per SM over the chunk), at least 2048 16-byte loads each
+    const int64_t nvec = (int64_t)(img_unit + 15) / 16;
+    const int parts = (int)std::max<int64_t>(1, std::min<int64_t>((nvec + 2047) / 2048, (8LL * h->num_sms + nu - 1) / nu));
+    sse_u8_kernel<<<(unsigned)(nu * parts), kSseThreads, 0, h->stream>>>(img + (size_t)img0 * img_unit, rec + (size_t)rec0 * img_unit,
+                                                                         (long long)img_unit, parts, d_sse + u0);
+    h->launches++;
+    TIC_CUDA(h, cudaGetLastError());
+    if (host) {
+      TIC_CUDA(h, cudaEventRecord(h->ev_enc[b], h->stream));
+      if (recon) {
+        TIC_CUDA(h, cudaStreamWaitEvent(h->s_d2h, h->ev_enc[b], 0));
+        TIC_CUDA(h, cudaMemcpyAsync(recon + (size_t)u0 * img_unit, h->stage_out[b], (size_t)nu * img_unit, cudaMemcpyDeviceToHost,
+                                    h->s_d2h));
+        TIC_CUDA(h, cudaEventRecord(h->ev_out[b], h->s_d2h));
+      }
+    }
+    const int64_t pend = u0 + nu - p0;
+    if (pend >= coder_imgs || idx + 1 == (int64_t)sched.size()) {
+      // the stored length of each image's stream, exactly tic_entropy_encode's out_bytes: plain streams report it
+      // directly, segmented ones through their segment lengths.  The next chunk's encoder overwrites the symbols
+      // after these kernels in stream order.
+      const uint8_t* s0 = (const uint8_t*)h->stage_sym[0];
+      if (nseg == 0) {
+        rc_encode_kernel<<<(unsigned)pend, 32, 0, h->stream>>>(s0, stream_len, stream_len, 1, h->d_cum, n_cum, h->d_seg, kEntropySegSlot,
+                                                               d_bytes + p0, h->d_oflow + 1);
+        h->launches++;
+      } else {
+        rc_encode_kernel<<<(unsigned)(pend * nseg), 32, 0, h->stream>>>(s0, stream_len, TIC_RC_SEGMENT_SYMBOLS, (int)nseg, h->d_cum, n_cum,
+                                                                        h->d_seg, kEntropySegSlot, h->d_seg_bytes, h->d_oflow + 1);
+        rc_stored_length_kernel<<<(unsigned)pend, 256, 0, h->stream>>>(h->d_seg_bytes, (int)nseg, d_bytes + p0);
+        h->launches += 2;
+      }
+      TIC_CUDA(h, cudaGetLastError());
+      p0 = u0 + nu;
+    }
+  }
+  TIC_CUDA(h, cudaEventRecord(h->ev_t1, h->stream));
+  if (host) {
+    TIC_CUDA(h, cudaMemcpyAsync(code_bytes, h->d_eval, (size_t)n_images * sizeof(int64_t), cudaMemcpyDeviceToHost, h->stream));
+    TIC_CUDA(h, cudaMemcpyAsync(sq_err, h->d_eval + n_images, (size_t)n_images * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
+    TIC_CUDA(h, cudaStreamSynchronize(h->s_d2h));
+    TIC_CUDA(h, cudaStreamSynchronize(h->stream));
+  }
+  return TIC_OK;
+  }();
+  if (!host) return rc_pipe;
+  if (rc_pipe != TIC_OK) {
+    quiesce(h);
+    return rc_pipe;
+  }
+  return overflow_status(h);
 }
 
 #ifdef TIC_ABLATE

@@ -167,15 +167,11 @@ __global__ void __launch_bounds__(32) rc_encode_kernel(const uint8_t* __restrict
   else if (sink.overflow) atomicCAS(status, 0u, 2u);
 }
 
-// Segmented call, second step: block stream * nseg + j writes header entry j (little-endian uint32 byte count) and copies
-// body j behind the bodies before it:  out slot = [ nseg x uint32 | body 0 | body 1 | ... ].
-__global__ void __launch_bounds__(256) rc_pack_kernel(const uint8_t* __restrict__ seg, const long long* __restrict__ seg_bytes, int nseg,
-                                                      uint8_t* __restrict__ out, long long out_stride, long long* __restrict__ out_bytes,
-                                                      unsigned int* status) {
+// Byte offset of body j in a segmented stream's container [ nseg x uint32 | body 0 | body 1 | ... ]: the header plus the
+// stored lengths of the bodies before j (lens = the stream's nseg segment lengths).  j = nseg gives the stored length of
+// the whole stream.  Called once by every thread of a 256-thread block; all of them get the value.
+__device__ __forceinline__ long long rc_container_offset(const long long* __restrict__ lens, int nseg, int j) {
   __shared__ long long s_part[8];
-  const long long stream = blockIdx.x / nseg;
-  const int j = (int)(blockIdx.x - stream * nseg);
-  const long long* lens = seg_bytes + stream * nseg;
   long long before = 0;
   for (int i = threadIdx.x; i < j; i += 256) before += lens[i];
   for (int o = 16; o > 0; o >>= 1) before += __shfl_down_sync(0xffffffffu, before, o);
@@ -184,8 +180,19 @@ __global__ void __launch_bounds__(256) rc_pack_kernel(const uint8_t* __restrict_
   before = 0;
 #pragma unroll
   for (int w = 0; w < 8; ++w) before += s_part[w];
+  return 4LL * nseg + before;
+}
+
+// Segmented call, second step: block stream * nseg + j writes header entry j (little-endian uint32 byte count) and copies
+// body j behind the bodies before it:  out slot = [ nseg x uint32 | body 0 | body 1 | ... ].
+__global__ void __launch_bounds__(256) rc_pack_kernel(const uint8_t* __restrict__ seg, const long long* __restrict__ seg_bytes, int nseg,
+                                                      uint8_t* __restrict__ out, long long out_stride, long long* __restrict__ out_bytes,
+                                                      unsigned int* status) {
+  const long long stream = blockIdx.x / nseg;
+  const int j = (int)(blockIdx.x - stream * nseg);
+  const long long* lens = seg_bytes + stream * nseg;
   const long long len = lens[j];
-  const long long at = 4LL * nseg + before;
+  const long long at = rc_container_offset(lens, nseg, j);
   uint8_t* slot = out + stream * out_stride;
   if (at + len > out_stride) {
     if (threadIdx.x == 0) {
@@ -204,6 +211,14 @@ __global__ void __launch_bounds__(256) rc_pack_kernel(const uint8_t* __restrict_
     slot[4 * j + 3] = (uint8_t)(v >> 24);
     if (j == nseg - 1) out_bytes[stream] = at + len;
   }
+}
+
+// Segmented call without an output slot: block `stream` writes the stored length rc_pack_kernel would give the stream
+// (out_bytes of tic_entropy_encode) from its segment lengths; no body is copied.
+__global__ void __launch_bounds__(256) rc_stored_length_kernel(const long long* __restrict__ seg_bytes, int nseg,
+                                                               long long* __restrict__ out_bytes) {
+  const long long v = rc_container_offset(seg_bytes + (long long)blockIdx.x * nseg, nseg, nseg);
+  if (threadIdx.x == 0) out_bytes[blockIdx.x] = v;
 }
 
 // One block (= one warp) per piece, as in rc_encode_kernel.  nseg = 0: plain streams.  nseg > 0: the slot starts with

@@ -197,6 +197,35 @@ def cal_distribution(codec, patches, batch_size=64):
     return np.asarray(prob), encoded_order, seq_prob
 
 
+def evaluate(codec, images, config, prob, group=None):
+    """scipt_bash/encode_decode_evaluate.sh without files: encode.py + decode.py + processing_utils/evaluate.py over a list
+    of uint8 [H,W,3] images (any sizes), on the device (Codec.evaluate_images per group of equal-sized images, the table
+    of encode.py:76-91).  Returns {"bpp", "psnr", "code_bytes", "sq_err"}: the set-level figures of evaluate.py (:10-49)
+    computed from exact integer sums in the float64 expressions of bpp() / psnr(), and the per-image file sizes and
+    integer squared errors in input order.  With `group`, the sums are all-reduced over its ranks first, so every rank
+    returns the figures of the whole dataset (the PSNR of a union is not a function of the per-rank PSNRs)."""
+    P = int(config["patch_size"])
+    cum = cum_freq_table(prob, int(config["resolution"]))
+    code_bytes = np.zeros(len(images), np.int64)
+    sq_err = np.zeros(len(images), np.uint64)
+    by_shape = {}
+    for i, im in enumerate(images):
+        by_shape.setdefault(tuple(im.shape), []).append(i)
+    for shape, idx in by_shape.items():
+        batch = np.ascontiguousarray(np.stack([images[i] for i in idx]), dtype=np.uint8)
+        nb, se, _ = codec.evaluate_images(batch, P, cum)
+        code_bytes[idx] = nb
+        sq_err[idx] = se
+    pixels = sum(int(im.shape[0]) * int(im.shape[1]) for im in images)
+    totals = np.array([int(code_bytes.sum()), int(sq_err.sum()), pixels, 3 * pixels], np.int64)
+    if group is not None:
+        totals = parallel.allreduce_counts(totals, group)
+    n_bytes, se, hw, hwc = (int(v) for v in totals)
+    return {"bpp": 8.0 * float(n_bytes) / float(hw),
+            "psnr": 20.0 * np.log10(255.0) - 10.0 * np.log10(float(se) / hwc),
+            "code_bytes": code_bytes, "sq_err": sq_err}
+
+
 def psnr(originals, reconstructions):
     """processing_utils/evaluate.py:10-30: 20 log10(255) - 10 log10(sum SE / sum HWC) over the whole set."""
     se, cnt = 0.0, 0
