@@ -4,9 +4,6 @@ boundaries, every first-layer / fused-pair dispatch path (checked by the names o
 quan_scale > 2.  Tolerances as in test_gpu_parity.py: symbol mismatch rate <= 1e-5 and every mismatch where the fp64
 logit is within fp32 noise of the sigmoid == 0.5 threshold; reconstruction within 1e-3 max-abs as float32, within one
 grey level at a rate < 1e-4 as uint8."""
-import json
-import os
-import tempfile
 import time
 
 import numpy as np
@@ -14,18 +11,12 @@ import pytest
 import torch
 
 from oracle import codec_oracle as O
-from gpu_common import MEAN, STD, make_codec, params_for
+from gpu_common import MEAN, STD, device_view, fmt, kernels_of, make_codec, params_for, ran, seeded_u8
 import tf_image_compression_b200 as T
 
 pytestmark = pytest.mark.gpu
 
 ORACLE_BATCH = 192  # patches per oracle call: one 2048x1536 image at P = 128 (a whole batch of them would need GBs)
-
-
-def seeded_u8(shape, seed):
-    """Uniform u8 noise from a seeded torch generator, as bench.py makes its images."""
-    g = torch.Generator(device="cpu").manual_seed(seed)
-    return torch.randint(0, 256, shape, dtype=torch.uint8, generator=g).numpy()
 
 
 def crops(images, P):
@@ -78,44 +69,6 @@ def check_recon(rec_f, rec_u8, want_f):
 def oracle_images(symbols, H, W, P, variant, dec, mean=MEAN, std=STD):
     """The oracle decoder of [B, gh*gw, ...] symbols, stitched and cropped like utils.concat_patches: [B,H,W,3] f32."""
     return np.stack([O.concat_patches(list(oracle_decoder(s, variant, dec, mean, std)), H, W, P) for s in symbols])
-
-
-def _short(name):
-    name = name.replace("(anonymous namespace)::", "").removeprefix("void ")
-    return name.split("(")[0].rsplit("::", 1)[-1].strip()
-
-
-def kernels_of(codec, fn):
-    """The names of the kernels one call fn() launches, without their parameter lists ('fused_enc_kernel',
-    'f16_first_s2_tma_kernel<true>', ...), from torch.profiler with CUDA activities.  fn() runs once before, so that
-    lazily built weight images are not counted; a torch kernel opens the profiled window, and the kernels recorded must
-    be as many as the codec counts (codec.launch_count), so that a kernel the profiler missed cannot pass for a path
-    that was not taken."""
-    fn()
-    torch.cuda.synchronize()
-    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
-        torch.zeros(1, device="cuda").add_(1)
-        n0 = codec.launch_count
-        fn()
-        torch.cuda.synchronize()
-        launched = codec.launch_count - n0
-    with tempfile.TemporaryDirectory() as d:
-        path = os.path.join(d, "trace.json")
-        prof.export_chrome_trace(path)
-        with open(path) as f:
-            events = json.load(f)["traceEvents"]
-    names = [_short(e["name"]) for e in events if e.get("cat") == "kernel" and "at::native" not in e["name"]]
-    assert len(names) == launched, f"torch.profiler recorded {len(names)} kernels, the codec launched {launched}: {names}"
-    return set(names)
-
-
-def ran(names, kernel):
-    """kernel ('fused_enc_kernel', or with template arguments: 'f16_first_s2_tma_kernel<true>') is among names."""
-    return kernel in names or kernel in {n.split("<")[0] for n in names}
-
-
-def fmt(names):
-    return ", ".join(sorted(names))
 
 
 # ---- A. the benchmark workload --------------------------------------------------------------------------------------
@@ -227,18 +180,6 @@ DISPATCH_CASES = [
     ("ragged129x385", (129, 385, 2), 0, {"f16_first_s2_kernel"}, {"fused_enc_kernel"}, {"fused_dec_kernel"}),
     ("ragged1356x2040", (1356, 2040, 1), 0, {"f16_first_s2_kernel"}, {"fused_enc_kernel"}, {"fused_dec_kernel"}),
 ]
-
-
-def device_view(host, offset, dtype=torch.uint8):
-    """host's values on the device, at byte `offset` from a 512-byte aligned allocation."""
-    t = torch.from_numpy(np.ascontiguousarray(host))
-    esz = t.element_size()
-    assert offset % esz == 0
-    buf = torch.zeros(t.numel() + 64 // esz, dtype=dtype, device="cuda")
-    v = buf[offset // esz:offset // esz + t.numel()].view(tuple(t.shape))
-    v.copy_(t.to("cuda"))
-    assert v.data_ptr() % 512 == offset and v.is_contiguous()
-    return v
 
 
 @pytest.mark.parametrize("case", DISPATCH_CASES, ids=[c[0] for c in DISPATCH_CASES])

@@ -352,6 +352,9 @@ class Codec:
         """rmbe.rmbe in place over float32 [B,H,W,3] (or [H,W,3]) images."""
         if self.post_layers is None:
             raise TicError("post-filter not configured (set_postfilter)")
+        # the C side reads and writes H*W*3 floats per image: any other layout must fail here
+        if images.ndim not in (3, 4) or tuple(images.shape[-1:]) != (3,):
+            raise ValueError(f"images must be [B,H,W,3] or [H,W,3], got {tuple(images.shape)}")
         x = images if images.ndim == 4 else images[None]
         B, H, W = int(x.shape[0]), int(x.shape[1]), int(x.shape[2])
         buf = _Buf(x, np.float32, self.device, self)
