@@ -1,5 +1,7 @@
-"""Shared fixtures for the -m gpu parity tests: seeded parameters, normalisation, inputs, device views and the names of
-the kernels a call launches."""
+"""Shared fixtures for the -m gpu parity tests: seeded parameters, normalisation, inputs, device views, the names of
+the kernels a call launches, the oracle of whole batches with the parity bars of the tensor path, and the rmbe
+post-filter's weights and oracle."""
+import collections
 import json
 import os
 import tempfile
@@ -65,8 +67,8 @@ def _short(name):
     return name.split("(")[0].rsplit("::", 1)[-1].strip()
 
 
-def kernels_of(codec, fn):
-    """The names of the kernels one call fn() launches, without their parameter lists ('fused_enc_kernel',
+def kernel_counts(codec, fn):
+    """How often each kernel is launched by one call fn(), by name without the parameter list ('fused_enc_kernel',
     'f16_first_s2_tma_kernel<true>', ...), from torch.profiler with CUDA activities.  fn() runs once before, so that
     lazily built weight images are not counted; a torch kernel opens the profiled window, and the kernels recorded must
     be as many as the codec counts (codec.launch_count), so that a kernel the profiler missed cannot pass for a path
@@ -86,7 +88,12 @@ def kernels_of(codec, fn):
             events = json.load(f)["traceEvents"]
     names = [_short(e["name"]) for e in events if e.get("cat") == "kernel" and "at::native" not in e["name"]]
     assert len(names) == launched, f"torch.profiler recorded {len(names)} kernels, the codec launched {launched}: {names}"
-    return set(names)
+    return collections.Counter(names)
+
+
+def kernels_of(codec, fn):
+    """The names of the kernels one call fn() launches (kernel_counts without the counts)."""
+    return set(kernel_counts(codec, fn))
 
 
 def ran(names, kernel):
@@ -96,3 +103,78 @@ def ran(names, kernel):
 
 def fmt(names):
     return ", ".join(sorted(names))
+
+
+# ---- oracle references of whole batches and the parity bars of the tensor path -------------------------------------
+ORACLE_BATCH = 192  # patches per oracle call: one 2048x1536 image at P = 128 (a whole batch of them would need GBs)
+
+
+def crops(images, P):
+    return np.stack([p for im in images for p in O.crop_image_input_patches(im, P)])
+
+
+def oracle_encoder(patches, variant, enc, mean=MEAN, std=STD, q=2):
+    return np.concatenate([O.encoder(patches[i:i + ORACLE_BATCH].astype(np.float32), variant, enc, mean, std, q)
+                           for i in range(0, len(patches), ORACLE_BATCH)])
+
+
+def oracle_decoder(symbols, variant, dec, mean=MEAN, std=STD, q=2):
+    return np.concatenate([O.decoder(symbols[i:i + ORACLE_BATCH], variant, dec, mean, std, q)
+                           for i in range(0, len(symbols), ORACLE_BATCH)])
+
+
+def logits64(patches, variant, enc, mean, std):
+    return np.concatenate([O.encoder_logits(patches[i:i + ORACLE_BATCH].astype(np.float32), variant, enc, mean, std,
+                                            dtype=torch.float64) for i in range(0, len(patches), ORACLE_BATCH)])
+
+
+def check_symbols(got, ref, patches, variant, enc, mean=MEAN, std=STD):
+    """q = 2: at most 1e-5 of the symbols (or one) differ from the oracle, and each difference sits where the fp64 logit
+    is within fp32 noise of 0 (test_gpu_parity.py's rule).  fp64 logits are evaluated for the patches with a mismatch only.
+    Returns (mismatches, largest |fp64 logit| at a mismatch)."""
+    got = np.asarray(got).reshape(ref.shape)
+    diff = got != ref
+    nm = int(diff.sum())
+    assert nm <= max(1, 1e-5 * ref.size), f"{nm}/{ref.size} symbol mismatches"
+    if not nm:
+        return 0, 0.0
+    bad = np.flatnonzero(diff.reshape(len(ref), -1).any(1))
+    l64 = logits64(patches[bad], variant, enc, mean, std)
+    at = np.abs(l64[diff[bad]])
+    bound = 1.5e-7 + 4e-6 * np.abs(l64).max()
+    assert at.max() < bound, f"mismatch at |fp64 logit| {at.max():.3e} outside the dead zone (< {bound:.3e})"
+    return nm, float(at.max())
+
+
+def check_recon(rec_f, rec_u8, want_f):
+    """float32 within 1e-3 max-abs of the oracle, uint8 within one grey level of np.around of it at a rate < 1e-4.
+    Returns (max-abs float error, fraction of u8 values that differ)."""
+    err = float(np.abs(np.asarray(rec_f) - want_f).max())
+    assert err <= 1e-3, f"reconstruction max-abs error {err:.3e}"
+    d = np.abs(np.asarray(rec_u8).astype(np.int32) - O.around_u8(want_f).astype(np.int32))
+    assert d.max() <= 1 and (d != 0).mean() < 1e-4, (int(d.max()), float((d != 0).mean()))
+    return err, float((d != 0).mean())
+
+
+def oracle_images(symbols, H, W, P, variant, dec, mean=MEAN, std=STD):
+    """The oracle decoder of [B, gh*gw, ...] symbols, stitched and cropped like utils.concat_patches: [B,H,W,3] f32."""
+    return np.stack([O.concat_patches(list(oracle_decoder(s, variant, dec, mean, std)), H, W, P) for s in symbols])
+
+
+# ---- the rmbe post-filter: fan-in weights, their normalisation and the fp32 oracle on whole images --------------------
+PM = np.array([110.0, 108.0, 99.0], np.float32)  # post-filter normalisation of the fan-in weight set
+PS = np.array([55.0, 57.0, 60.0], np.float32)
+ORACLE_TILES = 64  # tiles per oracle call (a 2048x1536 pass at once would need GBs of activations)
+
+
+def post_params(name="rmbe"):
+    """Fan-in weights: far from the identity, so a tile read before or after the other pass's write shows."""
+    return O.init_params(O.POSTFILTERS[name], 3, 77 if name == "rmbe" else 78, "fanin")
+
+
+def in_tiles(run, tiles):
+    return np.concatenate([run(tiles[i:i + ORACLE_TILES]) for i in range(0, len(tiles), ORACLE_TILES)])
+
+
+def oracle32(img, name, pp, mean=PM, std=PS):
+    return O.rmbe(img, lambda t: in_tiles(lambda x: O.postfilter(x, name, pp, mean, std), t))

@@ -8,7 +8,8 @@ from tf_image_compression_b200 import variants as V
 
 
 class OracleCodec:
-    def __init__(self, variant, quan_scale, mean, std, enc_params, dec_params):
+    def __init__(self, variant, quan_scale, mean, std, enc_params, dec_params, post_params=None, post_mean=None,
+                 post_std=None, post_name="rmbe"):
         self.variant = V.resolve(variant)
         self.quan_scale = int(quan_scale)
         self.mean, self.std = np.asarray(mean, np.float32), np.asarray(std, np.float32)
@@ -17,6 +18,11 @@ class OracleCodec:
         self.dec_layers = V.decoder_layers(self.variant)
         self.device = 0
         self.calls = []
+        # the rmbe post-filter of submit/2 (Codec.set_postfilter): weights, normalisation and net
+        self.post_params = None if post_params is None else dict(post_params)
+        self.post_mean = self.mean if post_mean is None else np.asarray(post_mean, np.float32)
+        self.post_std = self.std if post_std is None else np.asarray(post_std, np.float32)
+        self.post_name = post_name
 
     # ---- Codec surface used by ModelModule / entry / checkpoint ------------------------------------------------
     def bottleneck_shape(self, patch_size):
@@ -54,3 +60,15 @@ class OracleCodec:
             img = O.concat_patches(list(rec), height, width, patch_size)
             out.append(O.around_u8(img) if out_dtype == np.uint8 else img.astype(np.float32))
         return np.stack(out)
+
+    def postfilter_images(self, images):
+        """O.rmbe in place over float32 [B,H,W,3] (or [H,W,3]) images."""
+        if self.post_params is None:
+            raise RuntimeError("post-filter not configured")
+        x = images if images.ndim == 4 else images[None]
+        for im in x:
+            im[...] = O.rmbe(im, lambda t: O.postfilter(t, self.post_name, self.post_params, self.post_mean, self.post_std))
+        return images
+
+    def round_u8(self, x, out=None):
+        return O.around_u8(np.asarray(x))

@@ -181,3 +181,35 @@ def test_reference_entry_points_run_unmodified_on_the_oracle_codec(tmp_path):
     if HAVE_REF:  # the stored config is the reference's, as far as the flows read it
         assert {k: cfg[k] for k in stored_cfg} == stored_cfg
     assert all(entry.parse_encoded_name(s[0], stored_cfg)[1] == (16, 16, 64) for s in stored_roundtrip()[1])
+
+
+def test_uncompress_with_postfilter_on_the_oracle_codec(tmp_path):
+    """The submit/2 decode flow (decode -> stitch -> rmbe -> np.around, submit/2/decoder.py:183-198) through
+    entry.uncompress(postfilter=True) over the oracle codec of model_3, with the host and the serial coder: it equals
+    the oracle chain composed by hand from the symbols, exactly; postfilter=False equals decode_images(..., uint8).
+    200x300 is a multiple neither of the 128-pixel patch nor of the rmbe tile grid."""
+    from oracle_codec import OracleCodec
+    from gpu_common import PM, PS, post_params
+    ov = O.VARIANTS["model_3"]
+    enc = O.init_params(ov["enc"], 3, 1234, "fanin")
+    dec = O.condition_decoder("model_3", O.init_params(ov["dec"], ov["bottleneck"], 1235, "fanin"), 2)
+    pp = post_params()
+    codec = OracleCodec("model_3", 2, MEAN, STD, enc, dec, post_params=pp, post_mean=PM, post_std=PS)
+    cfg = dict(entry.DEFAULT_CONFIG, patch_size=128)
+    P, prob = cfg["patch_size"], np.array([0.55, 0.45])
+    images = {"a": O.synthetic_image(256, 384, 11), "b": O.synthetic_image(200, 300, 12)}
+    entry.compress(codec, list(images.values()), list(images), cfg, prob, str(tmp_path), coder="host")
+    want, plain = {}, {}
+    for nm, im in images.items():
+        H, W, _ = im.shape
+        sym = codec.encode_images(im[None], P)[0]
+        stitched = O.concat_patches(list(O.decoder(sym, "model_3", dec, MEAN, STD, 2)), H, W, P)
+        want[nm] = O.around_u8(O.rmbe(stitched, lambda t: O.postfilter(t, "rmbe", pp, PM, PS)))
+        plain[nm] = codec.decode_images(sym[None], H, W, P)[0]
+        assert not np.array_equal(want[nm], plain[nm])  # the filter changes the image
+    for c in ("host", "serial"):
+        got = entry.uncompress(codec, str(tmp_path), cfg, prob, postfilter=True, coder=c)
+        got_plain = entry.uncompress(codec, str(tmp_path), cfg, prob, coder=c)
+        for nm in images:
+            assert got[nm].dtype == np.uint8 and np.array_equal(got[nm], want[nm]), (c, nm)
+            assert np.array_equal(got_plain[nm], plain[nm]), (c, nm)

@@ -51,10 +51,12 @@ def test_against_the_file_flow(mode, tmp_path):
     codec.close()
 
 
-@pytest.mark.parametrize("variant,P", [("model_1", 256), ("base_model/reduced_btn_32", 128)])
+@pytest.mark.parametrize("variant,P", [("model_1", 256), ("base_model/reduced_btn_32", 128), ("model_3", 128),
+                                       ("model_2", 128)])
 def test_other_variants(variant, P):
-    """model_1 at P = 256, and a 32-channel bottleneck whose decoder tail is not the fused pair: lengths equal
-    entropy_encode's, squared errors equal those of decode_images."""
+    """model_1 at P = 256, a 32-channel bottleneck whose decoder tail is not the fused pair, and the submitted codecs
+    model_3 (80-channel bottleneck, CUDA-core decode_4) and model_2 (stride-2 quantiser, decoder from symbols): lengths
+    equal entropy_encode's, squared errors equal those of decode_images."""
     codec, _, _ = make_codec(variant, "fanin", compute="tensor")
     batch = np.stack([O.synthetic_image(512, 768, 60 + i) for i in range(3)])
     small = O.synthetic_image(200, 300, 70)[None]

@@ -19,25 +19,29 @@ pytestmark = pytest.mark.gpu
 
 # ---- decoder parity at realistic dynamic range (VERDICT r1, weak #3) ----------------------------------------------
 @pytest.mark.parametrize("mode", ["fp32", "tensor"])
-@pytest.mark.parametrize("variant", ["model_0", "model_1"])
+@pytest.mark.parametrize("variant", ["model_0", "model_1", "model_3", "model_2"])
 def test_decoder_parity_at_realistic_range(variant, mode):
     """A trained decoder's pre-denormalisation output has std ~ 1 (the data is normalised to unit variance,
     model_0/model.py:44,251) and the 0..255 clip is active.  condition_decoder(target_std=1.0) gives a random decoder
-    that range; P = 256 (the reference's config.json patch size).  The fp64 evaluation of the same graph is the arbiter:
-    the GPU result must be as close to it as the fp32 oracle is, and within the north-star bound of the fp32 oracle."""
+    that range; P = 256 (the reference's config.json patch size) for model_0 / model_1, P = 128 for the submitted codecs
+    model_3 (submit/2, submit/3) and model_2 (submit/1).  The fp64 evaluation of the same graph is the arbiter: the GPU
+    result must be as close to it as the fp32 oracle is, and within the north-star bound of the fp32 oracle.  The fp16
+    range guard of the tensor path must not trip at this range."""
+    P = 128 if variant in ("model_3", "model_2") else 256
     ov = O.VARIANTS[variant]
     dec = O.condition_decoder(variant, O.init_params(ov["dec"], ov["bottleneck"], 1235, "fanin"), 2, target_std=1.0)
     enc = O.init_params(ov["enc"], 3, 1234, "fanin")
     codec = T.Codec(variant, quan_scale=2, mean=MEAN, std=STD, enc_params=enc, dec_params=dec, compute=mode)
-    sym = np.random.RandomState(21).randint(0, 2, size=(3, 16, 16, 64)).astype(np.uint8)
+    sym = np.random.RandomState(21).randint(0, 2, size=(3, *codec.bottleneck_shape(P))).astype(np.uint8)
     got = codec.decode_patches(sym)
+    codec.check_status()
     ref32 = O.decoder(sym, variant, dec, MEAN, STD, 2)
     ref64 = O.decoder(sym, variant, dec, MEAN, STD, 2, dtype=torch.float64)
     clipped = float(((ref64 <= 0.0) | (ref64 >= 255.0)).mean())
     e_gpu64, e_ref64, e_gpu32 = (float(np.abs(got - ref64).max()), float(np.abs(ref32 - ref64).max()),
                                  float(np.abs(got - ref32).max()))
-    print(f"[{variant}@256 {mode}] clipped {clipped:.3f}; |gpu-f64| {e_gpu64:.3e}  |oracle32-f64| {e_ref64:.3e}  |gpu-oracle32| {e_gpu32:.3e}")
-    assert got.shape == (3, 256, 256, 3)
+    print(f"[{variant}@{P} {mode}] clipped {clipped:.3f}; |gpu-f64| {e_gpu64:.3e}  |oracle32-f64| {e_ref64:.3e}  |gpu-oracle32| {e_gpu32:.3e}")
+    assert got.shape == (3, P, P, 3)
     assert 0.005 < clipped < 0.5, clipped        # clipping is active but the image is not saturated
     assert float(np.std(ref64)) > 40.0           # realistic spread on the 0..255 scale
     assert e_gpu32 <= 1e-3                       # north_star: reconstruction within 1e-3 max-abs of the fp32 reference

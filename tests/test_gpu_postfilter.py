@@ -16,15 +16,12 @@ import torch
 
 from oracle import codec_oracle as O
 import tf_image_compression_b200 as T
-from gpu_common import MEAN, STD, device_view, fmt, kernels_of, make_codec, ran
+from gpu_common import MEAN, PM, PS, STD, device_view, fmt, in_tiles, kernels_of, make_codec, oracle32, post_params, ran
 
 pytestmark = pytest.mark.gpu
 
 MODES = ["fp32", "tensor"]
 P, OFF = 128, 64  # rmbe tile edge and grid offset (submit/2/rmbe/rmbe.py:12,16)
-PM = np.array([110.0, 108.0, 99.0], np.float32)  # post-filter normalisation of the fan-in weight set
-PS = np.array([55.0, 57.0, 60.0], np.float32)
-ORACLE_TILES = 64  # tiles per oracle call (a 2048x1536 pass at once would need GBs of activations)
 
 _cache = {}
 
@@ -34,11 +31,6 @@ def cached(key, fn):
     if key not in _cache:
         _cache[key] = fn()
     return _cache[key]
-
-
-def post_params(name="rmbe"):
-    """Fan-in weights: far from the identity, so a tile read before or after the other pass's write shows."""
-    return O.init_params(O.POSTFILTERS[name], 3, 77 if name == "rmbe" else 78, "fanin")
 
 
 def pf_codec(mode, name="rmbe", pp=None):
@@ -77,14 +69,6 @@ def untouched(H, W):
     return m
 
 
-def _batched(run, tiles):
-    return np.concatenate([run(tiles[i:i + ORACLE_TILES]) for i in range(0, len(tiles), ORACLE_TILES)])
-
-
-def oracle32(img, name, pp, mean=PM, std=PS):
-    return O.rmbe(img, lambda t: _batched(lambda x: O.postfilter(x, name, pp, mean, std), t))
-
-
 def arbiter64(img, name, pp, mean=PM, std=PS):
     """O.rmbe's two passes in float64: normalisation, the layers and the denormalisation + clip in float64, and the image
     kept in float64 between the passes.  The weights, means and stds are the float32 values the codec holds."""
@@ -100,7 +84,7 @@ def arbiter64(img, name, pp, mean=PM, std=PS):
         if hn * wn == 0:
             continue
         tiles = np.stack([image[oy + i * P:oy + (i + 1) * P, ox + j * P:ox + (j + 1) * P] for i in range(hn) for j in range(wn)])
-        new = _batched(run, tiles)
+        new = in_tiles(run, tiles)
         for i in range(hn):
             for j in range(wn):
                 image[oy + i * P:oy + (i + 1) * P, ox + j * P:ox + (j + 1) * P] = new[i * wn + j]

@@ -11,65 +11,11 @@ import pytest
 import torch
 
 from oracle import codec_oracle as O
-from gpu_common import MEAN, STD, device_view, fmt, kernels_of, make_codec, params_for, ran, seeded_u8
+from gpu_common import (MEAN, STD, check_recon, check_symbols, crops, device_view, fmt, kernels_of, logits64, make_codec,
+                        oracle_decoder, oracle_encoder, oracle_images, params_for, ran, seeded_u8)
 import tf_image_compression_b200 as T
 
 pytestmark = pytest.mark.gpu
-
-ORACLE_BATCH = 192  # patches per oracle call: one 2048x1536 image at P = 128 (a whole batch of them would need GBs)
-
-
-def crops(images, P):
-    return np.stack([p for im in images for p in O.crop_image_input_patches(im, P)])
-
-
-def oracle_encoder(patches, variant, enc, mean=MEAN, std=STD, q=2):
-    return np.concatenate([O.encoder(patches[i:i + ORACLE_BATCH].astype(np.float32), variant, enc, mean, std, q)
-                           for i in range(0, len(patches), ORACLE_BATCH)])
-
-
-def oracle_decoder(symbols, variant, dec, mean=MEAN, std=STD, q=2):
-    return np.concatenate([O.decoder(symbols[i:i + ORACLE_BATCH], variant, dec, mean, std, q)
-                           for i in range(0, len(symbols), ORACLE_BATCH)])
-
-
-def logits64(patches, variant, enc, mean, std):
-    return np.concatenate([O.encoder_logits(patches[i:i + ORACLE_BATCH].astype(np.float32), variant, enc, mean, std,
-                                            dtype=torch.float64) for i in range(0, len(patches), ORACLE_BATCH)])
-
-
-def check_symbols(got, ref, patches, variant, enc, mean=MEAN, std=STD):
-    """q = 2: at most 1e-5 of the symbols (or one) differ from the oracle, and each difference sits where the fp64 logit
-    is within fp32 noise of 0 (test_gpu_parity.py's rule).  fp64 logits are evaluated for the patches with a mismatch only.
-    Returns (mismatches, largest |fp64 logit| at a mismatch)."""
-    got = np.asarray(got).reshape(ref.shape)
-    diff = got != ref
-    nm = int(diff.sum())
-    assert nm <= max(1, 1e-5 * ref.size), f"{nm}/{ref.size} symbol mismatches"
-    if not nm:
-        return 0, 0.0
-    bad = np.flatnonzero(diff.reshape(len(ref), -1).any(1))
-    l64 = logits64(patches[bad], variant, enc, mean, std)
-    at = np.abs(l64[diff[bad]])
-    bound = 1.5e-7 + 4e-6 * np.abs(l64).max()
-    assert at.max() < bound, f"mismatch at |fp64 logit| {at.max():.3e} outside the dead zone (< {bound:.3e})"
-    return nm, float(at.max())
-
-
-def check_recon(rec_f, rec_u8, want_f):
-    """float32 within 1e-3 max-abs of the oracle, uint8 within one grey level of np.around of it at a rate < 1e-4.
-    Returns (max-abs float error, fraction of u8 values that differ)."""
-    err = float(np.abs(np.asarray(rec_f) - want_f).max())
-    assert err <= 1e-3, f"reconstruction max-abs error {err:.3e}"
-    d = np.abs(np.asarray(rec_u8).astype(np.int32) - O.around_u8(want_f).astype(np.int32))
-    assert d.max() <= 1 and (d != 0).mean() < 1e-4, (int(d.max()), float((d != 0).mean()))
-    return err, float((d != 0).mean())
-
-
-def oracle_images(symbols, H, W, P, variant, dec, mean=MEAN, std=STD):
-    """The oracle decoder of [B, gh*gw, ...] symbols, stitched and cropped like utils.concat_patches: [B,H,W,3] f32."""
-    return np.stack([O.concat_patches(list(oracle_decoder(s, variant, dec, mean, std)), H, W, P) for s in symbols])
-
 
 # ---- A. the benchmark workload --------------------------------------------------------------------------------------
 def test_benchmark_workload_against_oracle():
@@ -120,11 +66,15 @@ def test_benchmark_workload_against_oracle():
                          [("model_0", 128, True, True),                 # fused pairs around the u16 trunk
                           ("base_model/ch_128", 128, False, False),     # output-channel slices
                           ("model_1", 256, False, False),               # 3 -> 16 first layer, eight tile columns
-                          ("base_model/input_256", 256, False, True)])  # fused decoder at eight tile columns
+                          ("base_model/input_256", 256, False, True),   # fused decoder at eight tile columns
+                          ("model_3", 128, False, False),               # stride-2 80-channel quantiser, SIMT decode_4
+                          ("model_2", 128, False, False)])              # stride-2 quantiser, decoder from symbols
 def test_wave_and_pair_boundaries(variant, P, enc_fused, dec_fused):
     """A CTA pair takes patches pair0, pair0 + npairs, ... : patch counts of one patch, one pair, one wave of pairs minus /
     plus one patch, and two waves plus an odd tail, through encode_patches and decode_patches against the oracle.  Each
-    count runs the prefix of one seeded batch, so one oracle pass covers them all."""
+    count runs the prefix of one seeded batch, so one oracle pass covers them all.  On 8x8 maps two patches share a
+    tile, so the largest counts also cross the first wave of the quantiser layer; the histogram the quantiser epilogue
+    accumulates must equal np.bincount of the symbols it wrote at every count."""
     t0 = time.perf_counter()
     npairs = torch.cuda.get_device_properties(0).multi_processor_count // 2
     ns = [1, 2, 2 * npairs - 1, 2 * npairs, 2 * npairs + 1, 4 * npairs + 1, 4 * npairs + 3]
@@ -134,7 +84,10 @@ def test_wave_and_pair_boundaries(variant, P, enc_fused, dec_fused):
     want = oracle_decoder(ref, variant, dec)
     nm, worst, err = 0, 0.0, 0.0
     for n in ns:
-        n_i, w_i = check_symbols(codec.encode_patches(patches[:n]), ref[:n], patches[:n], variant, enc)
+        codec.hist_reset()
+        got = codec.encode_patches(patches[:n])
+        assert np.array_equal(codec.hist_read(), np.bincount(got.reshape(-1), minlength=2).astype(np.uint64)), n
+        n_i, w_i = check_symbols(got, ref[:n], patches[:n], variant, enc)
         nm, worst = nm + n_i, max(worst, w_i)
         e = float(np.abs(codec.decode_patches(ref[:n]) - want[:n]).max())
         assert e <= 1e-3, (n, e)
@@ -312,31 +265,34 @@ def test_chunk_boundaries(chunk):
 
 
 # ---- E. quan_scale > 2 in tensor mode ---------------------------------------------------------------------------------
-@pytest.mark.parametrize("q", [3, 4, 16, 255, 256])
-def test_quan_scale_in_tensor_mode(q):
-    """The quantiser epilogue, the general (q != 2) histogram and the q-entry inverse-sigmoid table of the tensor path.
+@pytest.mark.parametrize("variant,q", [pytest.param("model_0", q, id=str(q)) for q in (3, 4, 16, 255, 256)] +
+                         [pytest.param("model_3", q, id=f"model_3-{q}") for q in (3, 16)])
+def test_quan_scale_in_tensor_mode(variant, q):
+    """The quantiser epilogue, the general (q != 2) histogram and the q-entry inverse-sigmoid table of the tensor path:
+    model_0's stride-1 64-channel quantiser, and model_3's stride-2 80-channel one (8 epilogue warps), whose decoder
+    reads the table on the CUDA cores.
     A symbol may differ from the oracle's by one where the fp64 value sigmoid(logit) * (q - 1) is within fp32 noise of a
     half-integer: the logit's accumulation error (4e-6 of the largest logit, as for q = 2) times the sigmoid's slope
     (at most (q - 1) / 4), plus a few fp32 ulps of sigmoid * (q - 1)."""
     t0 = time.perf_counter()
-    codec, enc, dec = make_codec("model_0", q=q, compute="tensor")
+    codec, enc, dec = make_codec(variant, q=q, compute="tensor")
     patches = seeded_u8((48, 128, 128, 3), 500 + q)
     codec.hist_reset()
     sym = codec.encode_patches(patches)
     assert np.array_equal(codec.hist_read(), np.bincount(sym.reshape(-1), minlength=q).astype(np.uint64))
-    ref = oracle_encoder(patches, "model_0", enc, q=q)
+    ref = oracle_encoder(patches, variant, enc, q=q)
     d = np.abs(sym.astype(np.int32) - ref.astype(np.int32))
     assert d.max() <= 1
     nm, dist, bound = int((d != 0).sum()), 0.0, 0.0
     if nm:
-        l64 = logits64(patches, "model_0", enc, MEAN, STD)
+        l64 = logits64(patches, variant, enc, MEAN, STD)
         o = (q - 1) / (1 + np.exp(-l64[d != 0]))
         dist = float(np.abs(o - np.floor(o) - 0.5).max())
         bound = (q - 1) * 1e-6 * float(np.abs(l64).max()) + 4 * np.spacing(np.float32(q - 1)).item()
         assert dist <= bound, f"a mismatch {dist:.3e} from a half-integer, bound {bound:.3e}"
     rec = codec.decode_patches(ref)
-    err = float(np.abs(rec - oracle_decoder(ref, "model_0", dec, q=q)).max())
+    err = float(np.abs(rec - oracle_decoder(ref, variant, dec, q=q)).max())
     assert err <= 1e-3
-    print(f"[E q={q}] {len(patches)} patches, {ref.size} symbols; mismatches {nm} (|d| <= 1, max distance from a "
+    print(f"[E {variant} q={q}] {len(patches)} patches, {ref.size} symbols; mismatches {nm} (|d| <= 1, max distance from a "
           f"half-integer {dist:.2e}, bound {bound:.2e}); recon max-abs {err:.2e}; {time.perf_counter() - t0:.1f} s")
     codec.close()
