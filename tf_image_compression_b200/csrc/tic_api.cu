@@ -67,10 +67,8 @@ struct tic_codec {
   int mode = TIC_COMPUTE_FP32;
   int chunk128 = 4096;
   // workspaces
-  float* act[3] = {nullptr, nullptr, nullptr};  // rotating (sub-)chunk activations
+  float* act[3] = {nullptr, nullptr, nullptr};  // rotating chunk activations
   size_t act_bytes = 0;
-  float* bnd[2] = {nullptr, nullptr};           // chunk-level tensors at layer-group boundaries
-  size_t bnd_bytes = 0;
   void* stage_in[2] = {nullptr, nullptr};
   void* stage_out[2] = {nullptr, nullptr};
   void* stage_sym[2] = {nullptr, nullptr};      // round trips: the symbols between the two graphs
@@ -262,26 +260,41 @@ struct Shape {
   int h, w, c;
 };
 
-int graph_out_shape(const Graph& g, Shape in, Shape* out, size_t* max_act_elems, int limit = -1) {
-  Shape s = in;
-  size_t mx = 0;
+struct LayerShape {
+  int hin, win, cin, hout, wout, cout, pad_t, pad_l;
+};
+
+// Shapes of the first `limit` layers of g (all of them for limit <= 0) on an `in` input; false when a layer's cin is not
+// the channel count it receives.
+bool layer_shapes(const Graph& g, Shape in, int limit, std::vector<LayerShape>* sh) {
   const size_t L = limit > 0 ? std::min<size_t>((size_t)limit, g.layers.size()) : g.layers.size();
+  sh->resize(L);
+  Shape s = in;
   for (size_t i = 0; i < L; ++i) {
     const tic_layer_desc& d = g.layers[i].d;
-    if (d.cin != s.c) return -1;
+    if (d.cin != s.c) return false;
+    LayerShape& t = (*sh)[i];
+    t.hin = s.h;
+    t.win = s.w;
+    t.cin = s.c;
+    t.pad_t = t.pad_l = 0;
     if (d.kind == TIC_CONV) {
-      int pb;
-      same_pad(s.h, d.stride, &s.h, &pb);
-      same_pad(s.w, d.stride, &s.w, &pb);
+      same_pad(s.h, d.stride, &t.hout, &t.pad_t);
+      same_pad(s.w, d.stride, &t.wout, &t.pad_l);
     } else {
-      s.h *= 2;
-      s.w *= 2;
+      t.hout = 2 * s.h;
+      t.wout = 2 * s.w;
     }
-    s.c = d.cout;
-    if (i + 1 < L) mx = std::max(mx, (size_t)s.h * s.w * s.c);
+    t.cout = d.cout;
+    s = Shape{t.hout, t.wout, t.cout};
   }
-  *out = s;
-  if (max_act_elems) *max_act_elems = mx;
+  return true;
+}
+
+int graph_out_shape(const Graph& g, Shape in, Shape* out, int limit = -1) {
+  std::vector<LayerShape> sh;
+  if (!layer_shapes(g, in, limit, &sh)) return -1;
+  *out = sh.empty() ? in : Shape{sh.back().hout, sh.back().wout, sh.back().cout};
   return 0;
 }
 
@@ -292,75 +305,6 @@ int check_graph_ready(tic_codec* h, int gi, bool need_norm) {
     if (!g.layers[i].loaded) return fail(h, TIC_ERR_STATE, "graph %d layer %zu has no weights (tic_load_weights)", gi, i);
   if (need_norm && !g.has_norm) return fail(h, TIC_ERR_STATE, "graph %d has no normalisation (tic_set_norm)", gi);
   return TIC_OK;
-}
-
-// Layer groups of one graph execution (fp16-pair mode).  With every layer at (or near) the HBM roofline the
-// remaining lever is to keep inter-layer tensors in the 126 MB L2: consecutive layers run over a SUB-chunk of
-// m patches so that the tensors between them (m x bytes per patch) fit the L2 budget, and only the tensor at a
-// group boundary is written out for the whole chunk.  A group is closed when the next layer would push m so
-// low that some layer of the group could not fill the 148 SMs twice (model_0: {encode_0, encode_1} at m = 111
-// and {encode_2 .. encode_4} at m = 888; decoder {decode_4 .. decode_2} and {decode_1, decode_0}).
-struct LayerShape {
-  int hin, win, cin, hout, wout, cout, pad_t, pad_l;
-};
-struct LayerGroup {
-  int first, last, m;
-};
-
-long long l2_budget_bytes_per_group() {
-  // 0 (default, and the only value outside -DTIC_ABLATE builds) disables grouping.  Measured on B200 (model_0, 12288
-  // patches): 56 MB -> 20.3 ms per encode+decode step against 14.0 ms ungrouped: each extra (20 us) launch costs ~8 us
-  // of prologue (weight tiles, TMEM, cluster sync) and tail.  The schedule pays off only once a group runs as one
-  // persistent kernel.
-  const long long v = tic_env_int("TIC_L2_BUDGET_MB", 0);
-  return (v < 0 ? 0 : std::min<long long>(v, 4096)) << 20;
-}
-
-std::vector<LayerGroup> plan_groups(const Graph& g, const std::vector<LayerShape>& sh, int L, int n, bool enable) {
-  std::vector<LayerGroup> groups;
-  const long long budget = l2_budget_bytes_per_group();
-  if (!enable || budget <= 0 || n < 64) {
-    groups.push_back({0, L - 1, n});
-    return groups;
-  }
-  auto tiles_pp = [&](int i) {
-    const bool dc = g.layers[i].d.kind == TIC_DECONV;
-    return (double)(dc ? sh[i].hin * sh[i].win : sh[i].hout * sh[i].wout) / 128.0;
-  };
-  auto out_bytes = [&](int i) { return (long long)sh[i].hout * sh[i].wout * sh[i].cout * 4; };
-  const double min_tiles = 296.0;  // two tiles per SM (one CTA pair per TPC, twice)
-  int first = 0;
-  while (first < L) {
-    int last = first;
-    long long tmax = 0;
-    bool in_res = g.layers[first].d.res_begin && !g.layers[first].d.res_end;
-    while (last + 1 < L) {
-      const long long tnew = std::max(tmax, out_bytes(last));
-      const long long mnew = std::min<long long>(n, std::max<long long>(1, budget / std::max<long long>(tnew, 1)));
-      bool ok = true;
-      if (mnew < n)
-        for (int j = first; j <= last + 1; ++j) ok = ok && tiles_pp(j) * (double)mnew >= min_tiles;
-      if (!ok && !in_res) break;
-      ++last;
-      tmax = tnew;
-      if (g.layers[last].d.res_begin) in_res = true;
-      if (g.layers[last].d.res_end) in_res = false;
-    }
-    long long m = tmax > 0 ? std::min<long long>(n, std::max<long long>(1, budget / tmax)) : n;
-    if (m < n) {
-      // a whole number of waves for the layer with the fewest tiles: m a multiple of q patches
-      double tp_min = 1e30;
-      for (int j = first; j <= last; ++j) tp_min = std::min(tp_min, tiles_pp(j));
-      const long long q = std::max<long long>(1, (long long)(296.0 / tp_min + 0.5));
-      long long mr = ((m + q / 2) / q) * q;
-      if (mr < q) mr = q;
-      if (mr * tmax > budget + budget / 4) mr = std::max<long long>(q, (m / q) * q);
-      m = std::min<long long>(n, mr);
-    }
-    groups.push_back({first, last, (int)m});
-    first = last + 1;
-  }
-  return groups;
 }
 
 int ensure_buffers(tic_codec* h, float** bufs, int count, size_t* have, size_t need) {
@@ -379,270 +323,193 @@ int ensure_buffers(tic_codec* h, float** bufs, int count, size_t* have, size_t n
   return TIC_OK;
 }
 
+// The fields of a layer's launch arguments that come from the layer itself: shapes, padding, activation, weights.
+void set_layer(LayerArgs& a, const Layer& ly, const LayerShape& t) {
+  a.hin = t.hin;
+  a.win = t.win;
+  a.cin = t.cin;
+  a.hout = t.hout;
+  a.wout = t.wout;
+  a.cout = t.cout;
+  a.pad_t = t.pad_t;
+  a.pad_l = t.pad_l;
+  a.act = ly.d.act;
+  a.wgt = ly.w;
+  a.bias = ly.b;
+}
+
 // Run graph gi over n patches whose first-layer input map is h0 x w0 x c0.
 int run_graph(tic_codec* h, int gi, const IoSpec& io_in, const IoSpec& io_out, int n, int h0, int w0, int limit = -1) {
   Graph& g = h->g[gi];
-  const int L = limit > 0 ? std::min(limit, (int)g.layers.size()) : (int)g.layers.size();
-  std::vector<LayerShape> sh(L);
-  {
-    Shape s{h0, w0, g.layers[0].d.cin};
-    for (int i = 0; i < L; ++i) {
-      const tic_layer_desc& d = g.layers[i].d;
-      if (d.cin != s.c) return fail(h, TIC_ERR_INVALID, "layer channel chain is inconsistent");
-      LayerShape& t = sh[i];
-      t.hin = s.h;
-      t.win = s.w;
-      t.cin = s.c;
-      t.pad_t = t.pad_l = 0;
-      if (d.kind == TIC_CONV) {
-        same_pad(s.h, d.stride, &t.hout, &t.pad_t);
-        same_pad(s.w, d.stride, &t.wout, &t.pad_l);
-      } else {
-        t.hout = 2 * s.h;
-        t.wout = 2 * s.w;
-      }
-      t.cout = d.cout;
-      s = Shape{t.hout, t.wout, t.cout};
-    }
-  }
+  std::vector<LayerShape> sh;
+  if (!layer_shapes(g, Shape{h0, w0, g.layers[0].d.cin}, limit, &sh))
+    return fail(h, TIC_ERR_INVALID, "layer channel chain is inconsistent");
+  if (n == 0) return TIC_OK;
+  const int L = (int)sh.size();
   const bool pair16 = h->mode == TIC_COMPUTE_TENSOR_F16X3;  // intermediate activations are fp16 pair planes
   // pair mode: f32 / symbol inputs of a tensor-capable first layer are split into a workspace buffer first
   bool split_input = false;
   if (pair16 && (io_in.mode == IO_ACT || io_in.mode == IO_U8_SYMLUT)) {
     LayerArgs t{};
-    const tic_layer_desc& d0 = g.layers[0].d;
     t.n = n;
-    t.hin = sh[0].hin;
-    t.win = sh[0].win;
-    t.cin = sh[0].cin;
-    t.hout = sh[0].hout;
-    t.wout = sh[0].wout;
-    t.cout = sh[0].cout;
+    set_layer(t, g.layers[0], sh[0]);
     t.in_mode = IO_ACT16;
     t.out_mode = L == 1 ? io_out.mode : IO_ACT16;
-    split_input = u16_supported(t, d0.kind, d0.stride);
+    split_input = u16_supported(t, g.layers[0].d.kind, g.layers[0].d.stride);
   }
-  const std::vector<LayerGroup> groups = plan_groups(g, sh, L, n, pair16);
-  // workspaces: three rotating sub-chunk buffers, two chunk-level group-boundary buffers
-  size_t intra = 0, bnd = 0;
-  for (size_t gx = 0; gx < groups.size(); ++gx) {
-    const LayerGroup& G = groups[gx];
-    for (int i = G.first; i < G.last; ++i) intra = std::max(intra, (size_t)G.m * sh[i].hout * sh[i].wout * sh[i].cout);
-    if (gx == 0 && split_input) intra = std::max(intra, (size_t)G.m * sh[0].hin * sh[0].win * sh[0].cin);
-    if (gx + 1 < groups.size()) bnd = std::max(bnd, (size_t)n * sh[G.last].hout * sh[G.last].wout * sh[G.last].cout);
-  }
-  int rc0 = ensure_buffers(h, h->act, 3, &h->act_bytes, intra * sizeof(float));
-  if (rc0 != TIC_OK) return rc0;
-  rc0 = ensure_buffers(h, h->bnd, 2, &h->bnd_bytes, bnd * sizeof(float));
+  // workspaces: three rotating activation buffers
+  size_t act_elems = 0;
+  for (int i = 0; i + 1 < L; ++i) act_elems = std::max(act_elems, (size_t)n * sh[i].hout * sh[i].wout * sh[i].cout);
+  if (split_input) act_elems = std::max(act_elems, (size_t)n * sh[0].hin * sh[0].win * sh[0].cin);
+  const int rc0 = ensure_buffers(h, h->act, 3, &h->act_bytes, act_elems * sizeof(float));
   if (rc0 != TIC_OK) return rc0;
 
-  for (size_t gx = 0; gx < groups.size(); ++gx) {
-    const LayerGroup& G = groups[gx];
-    const bool first_group = gx == 0, last_group = gx + 1 == groups.size();
-    for (int s0 = 0; s0 < n; s0 += G.m) {
-      const int ns = std::min(G.m, n - s0);
-      int cur = -1;        // act[] index holding the current activation (-1: the group's input)
-      int res_buf = -1;    // act[] index of the live residual source (-1: none, or not an act[] buffer)
-      const void* res_ptr = nullptr;
-      long long res_lo = 0;
-      if (first_group && split_input) {
-        const long long per = (long long)sh[0].hin * sh[0].win * sh[0].cin;
-        const long long count = (long long)ns * per;
-        __half* hi = reinterpret_cast<__half*>(h->act[0]);
-        const int blocks = (int)std::min<long long>((count + 255) / 256, (long long)h->num_sms * 8);
-        if (io_in.mode == IO_ACT)
-          u16_split_f32_kernel<<<blocks, 256, 0, h->stream>>>(reinterpret_cast<const float*>(io_in.in) + (long long)s0 * per, hi,
-                                                             hi + count, count, h->d_oflow);
-        else
-          u16_split_symlut_kernel<<<blocks, 256, 0, h->stream>>>(
-              reinterpret_cast<const uint8_t*>(io_in.in) + ((long long)io_in.geo.n0 + s0) * per, h->d_symlut, h->q, hi, hi + count, count,
-              h->d_oflow);
-        h->launches++;
-        TIC_CUDA(h, cudaGetLastError());
-        cur = 0;
-      }
-      for (int i = G.first; i <= G.last; ++i) {
-        Layer& ly = g.layers[i];
-        const tic_layer_desc& d = ly.d;
-        const LayerShape& t = sh[i];
-        LayerArgs a{};
-        a.n = ns;
-        a.hin = t.hin;
-        a.win = t.win;
-        a.cin = t.cin;
-        a.hout = t.hout;
-        a.wout = t.wout;
-        a.cout = t.cout;
-        a.pad_t = t.pad_t;
-        a.pad_l = t.pad_l;
-        a.act = d.act;
-        a.wgt = ly.w;
-        a.bias = ly.b;
-        a.q = h->q;
-        a.hist = h->d_hist;
-        a.oflow = h->d_oflow;
-        a.dbg = tic_env_int("TIC_DBG", 0);  // -DTIC_ABLATE builds only
-        for (int c = 0; c < 3; ++c) {
-          a.mean[c] = g.mean[c];
-          a.stdv[c] = g.stdv[c];
+  int cur = -1;        // act[] index holding the current activation (-1: the caller's input)
+  int res_buf = -1;    // act[] index of the live residual source (-1: none, or not an act[] buffer)
+  const void* res_ptr = nullptr;
+  long long res_lo = 0;
+  if (split_input) {
+    const long long per = (long long)sh[0].hin * sh[0].win * sh[0].cin;
+    const long long count = (long long)n * per;
+    __half* hi = reinterpret_cast<__half*>(h->act[0]);
+    const int blocks = (int)std::min<long long>((count + 255) / 256, (long long)h->num_sms * 8);
+    if (io_in.mode == IO_ACT)
+      u16_split_f32_kernel<<<blocks, 256, 0, h->stream>>>(reinterpret_cast<const float*>(io_in.in), hi, hi + count, count, h->d_oflow);
+    else
+      u16_split_symlut_kernel<<<blocks, 256, 0, h->stream>>>(reinterpret_cast<const uint8_t*>(io_in.in) + (long long)io_in.geo.n0 * per,
+                                                             h->d_symlut, h->q, hi, hi + count, count, h->d_oflow);
+    h->launches++;
+    TIC_CUDA(h, cudaGetLastError());
+    cur = 0;
+  }
+  for (int i = 0; i < L; ++i) {
+    Layer& ly = g.layers[i];
+    const tic_layer_desc& d = ly.d;
+    LayerArgs a{};
+    a.n = n;
+    set_layer(a, ly, sh[i]);
+    a.q = h->q;
+    a.hist = h->d_hist;
+    a.oflow = h->d_oflow;
+    a.dbg = tic_env_int("TIC_DBG", 0);  // -DTIC_ABLATE builds only
+    for (int c = 0; c < 3; ++c) {
+      a.mean[c] = g.mean[c];
+      a.stdv[c] = g.stdv[c];
+    }
+    const long long ein = (long long)a.hin * a.win * a.cin, eout = (long long)a.hout * a.wout * a.cout;
+    // ---- input
+    if (cur < 0) {
+      a.in_mode = io_in.mode;
+      a.geo = io_in.geo;
+      a.lut = (io_in.mode == IO_U8_NORM) ? g.d_normlut : (io_in.mode == IO_U8_SYMLUT ? h->d_symlut : nullptr);
+      a.in = io_in.in;
+    } else {
+      a.in = h->act[cur];
+      a.in_mode = pair16 ? IO_ACT16 : IO_ACT;
+      a.in_lo_off = (long long)n * ein;
+    }
+    if (d.res_begin) {
+      res_buf = cur;
+      res_ptr = a.in;
+      res_lo = a.in_lo_off;
+    }
+    // ---- output: a workspace buffer that is neither the input nor the live residual
+    int ob = -1;
+    if (i == L - 1) {
+      a.out_mode = io_out.mode;
+      a.out = io_out.out;
+      // a single-layer graph shares one geo between prologue and epilogue only if both need it
+      if (!(i == 0 && io_out.mode == IO_ACT)) a.geo = io_out.geo;
+    } else {
+      for (int b = 0; b < 3; ++b)
+        if (b != cur && b != res_buf) {
+          ob = b;
+          break;
         }
-        const long long ein = (long long)t.hin * t.win * t.cin, eout = (long long)t.hout * t.wout * t.cout;
-        // ---- input
-        if (i == G.first && cur < 0) {
-          if (first_group) {
-            a.in_mode = io_in.mode;
-            a.geo = io_in.geo;
-            a.geo.n0 += s0;
-            a.lut = (io_in.mode == IO_U8_NORM) ? g.d_normlut : (io_in.mode == IO_U8_SYMLUT ? h->d_symlut : nullptr);
-            a.in = io_in.mode == IO_ACT ? (const void*)(reinterpret_cast<const float*>(io_in.in) + (long long)s0 * ein) : io_in.in;
-          } else {
-            a.in = reinterpret_cast<const __half*>(h->bnd[(gx - 1) & 1]) + (long long)s0 * ein;
-            a.in_mode = IO_ACT16;
-            a.in_lo_off = (long long)n * ein;
-          }
-        } else {
-          a.in = h->act[cur];
-          a.in_mode = pair16 ? IO_ACT16 : IO_ACT;
-          a.in_lo_off = (long long)ns * ein;
-        }
-        if (d.res_begin) {
-          res_buf = cur;
-          res_ptr = a.in;
-          res_lo = a.in_lo_off;
-        }
-        // ---- output: a workspace buffer that is neither the input nor the live residual
-        int ob = -1;
-        if (i == G.last) {
-          if (last_group) {
-            a.out_mode = io_out.mode;
-            a.out = io_out.mode == IO_ACT ? (void*)(reinterpret_cast<float*>(io_out.out) + (long long)s0 * eout) : io_out.out;
-            // a single-layer graph shares one geo between prologue and epilogue only if both need it
-            if (!(first_group && i == G.first && io_out.mode == IO_ACT)) {
-              a.geo = io_out.geo;
-              a.geo.n0 += s0;
-            }
-          } else {
-            a.out = reinterpret_cast<__half*>(h->bnd[gx & 1]) + (long long)s0 * eout;
-            a.out_mode = IO_ACT16;
-            a.out_lo_off = (long long)n * eout;
-          }
-        } else {
-          for (int b = 0; b < 3; ++b)
-            if (b != cur && b != res_buf) {
-              ob = b;
-              break;
-            }
-          a.out = h->act[ob];
-          a.out_mode = pair16 ? IO_ACT16 : IO_ACT;
-          a.out_lo_off = (long long)ns * eout;
-        }
-        if (d.res_end) {
-          if (!res_ptr) return fail(h, TIC_ERR_INVALID, "res_end without res_begin at layer %d", i);
-          a.res = reinterpret_cast<const float*>(res_ptr);
-          a.res16 = pair16 ? 1 : 0;
-          a.res_lo_off = res_lo;
-        }
-        int rc;
-        tic_codec::ProfRec pr{gi, i, nullptr, nullptr};
-        if (h->profile) {
-          cudaEventCreate(&pr.e0);
-          cudaEventCreate(&pr.e1);
-          cudaEventRecord(pr.e0, h->stream);
-        }
-        // the last two transposed convs of a decoder (32 -> 32 -> 3 into the image) run as one back-to-back kernel: the
-        // tensor between them never leaves shared memory (tic_fused16.cuh)
-        bool fused = false;
-        if (pair16 && last_group && i + 1 == G.last && i + 1 == L - 1 && !d.res_begin && !d.res_end && !g.layers[i + 1].d.res_begin &&
-            !g.layers[i + 1].d.res_end && tic_env_int("TIC_FUSE_DEC", 1) != 0) {
-          Layer& ly2 = g.layers[i + 1];
-          const LayerShape& t2 = sh[i + 1];
-          LayerArgs a2 = a;
-          a2.hin = t2.hin;
-          a2.win = t2.win;
-          a2.cin = t2.cin;
-          a2.hout = t2.hout;
-          a2.wout = t2.wout;
-          a2.cout = t2.cout;
-          a2.pad_t = t2.pad_t;
-          a2.pad_l = t2.pad_l;
-          a2.act = ly2.d.act;
-          a2.wgt = ly2.w;
-          a2.bias = ly2.b;
-          a2.res = nullptr;
-          a2.in = nullptr;
-          a2.in_mode = IO_ACT16;
-          a2.out_mode = io_out.mode;
-          a2.out = io_out.mode == IO_ACT ? nullptr : io_out.out;
-          a2.geo = io_out.geo;
-          a2.geo.n0 += s0;
-          if (a2.out && fused_dec_supported(a, d.kind, a2, ly2.d.kind)) {
-            int nl = 0;
-            rc = launch_fused_dec(h->stream, a, a2, ly.w, ly2.w, ly.hb.data(), ly2.hb.data(), &ly.fdw, h->num_sms, &h->err, &nl);
-            h->launches += nl;
-            fused = true;
-          }
-        }
-        // ... and the first two layers of an encoder (u8 image -> 3 -> 32 -> 32, both stride 2): tic_fused_enc16.cuh
-        if (!fused && pair16 && first_group && i == 0 && cur < 0 && i + 1 < G.last && !g.layers[1].d.res_begin && !g.layers[1].d.res_end &&
-            tic_env_int("TIC_FUSE_ENC", 1) != 0) {
-          Layer& ly2 = g.layers[1];
-          const LayerShape& t2 = sh[1];
-          LayerArgs a2 = a;
-          a2.hin = t2.hin;
-          a2.win = t2.win;
-          a2.cin = t2.cin;
-          a2.hout = t2.hout;
-          a2.wout = t2.wout;
-          a2.cout = t2.cout;
-          a2.pad_t = t2.pad_t;
-          a2.pad_l = t2.pad_l;
-          a2.act = ly2.d.act;
-          a2.wgt = ly2.w;
-          a2.bias = ly2.b;
-          a2.res = nullptr;
-          a2.in = nullptr;
-          a2.in_mode = IO_ACT16;
-          a2.out_mode = IO_ACT16;
-          a2.out = h->act[0];
-          a2.out_lo_off = (long long)ns * t2.hout * t2.wout * t2.cout;
-          if (fused_enc_supported(a, d.kind, d.stride, a2, ly2.d.kind, ly2.d.stride)) {
-            int nl = 0;
-            rc = launch_fused_enc(h->stream, a, a2, ly.w, ly2.w, ly.hb.data(), &ly.few, h->num_sms, &h->err, &nl);
-            h->launches += nl;
-            fused = true;
-            ob = 0;  // the pair's output lives in act[0]
-          }
-        }
-        if (fused) {
-          ++i;  // the next layer ran inside this launch (its time is reported with this layer)
-        } else if (pair16 && f16_first_supported(a, d.kind, d.stride)) {
-          int nl = 0;
-          rc = launch_first16(h->stream, a, d.stride, ly.w, &ly.fw16, h->num_sms, &h->err, &nl);
-          h->launches += nl;
-        } else if (pair16 && u16_supported(a, d.kind, d.stride)) {
-          int nl = 0;
-          rc = launch_u16(h->stream, a, d.kind, d.stride, ly.w, &ly.uw16, h->num_sms, &h->err, &nl);
-          h->launches += nl;
-        } else if (h->mode != TIC_COMPUTE_FP32 && !pair16 && umma_supported(a, d.kind, d.stride)) {
-          int nl = 0;
-          rc = launch_umma(h->stream, a, d.kind, d.stride, ly.w, &ly.uw, h->mode == TIC_COMPUTE_TENSOR_3XTF32, h->num_sms,
-                           &h->err, &nl);
-          h->launches += nl;
-        } else {
-          rc = launch_simt(h, a, d.kind, d.stride);
-        }
-        if (h->profile) {
-          cudaEventRecord(pr.e1, h->stream);
-          h->prof_pending.push_back(pr);
-        }
-        if (rc != TIC_OK) return rc < 0 && rc >= TIC_ERR_UNSUPPORTED ? rc : TIC_ERR_CUDA;
-        if (d.res_end) {
-          res_buf = -1;
-          res_ptr = nullptr;
-        }
-        cur = ob;
+      a.out = h->act[ob];
+      a.out_mode = pair16 ? IO_ACT16 : IO_ACT;
+      a.out_lo_off = (long long)n * eout;
+    }
+    if (d.res_end) {
+      if (!res_ptr) return fail(h, TIC_ERR_INVALID, "res_end without res_begin at layer %d", i);
+      a.res = reinterpret_cast<const float*>(res_ptr);
+      a.res16 = pair16 ? 1 : 0;
+      a.res_lo_off = res_lo;
+    }
+    int rc;
+    tic_codec::ProfRec pr{gi, i, nullptr, nullptr};
+    if (h->profile) {
+      cudaEventCreate(&pr.e0);
+      cudaEventCreate(&pr.e1);
+      cudaEventRecord(pr.e0, h->stream);
+    }
+    // the last two transposed convs of a decoder (32 -> 32 -> 3 into the image) run as one back-to-back kernel: the
+    // tensor between them never leaves shared memory (tic_fused16.cuh)
+    bool fused = false;
+    if (pair16 && i + 2 == L && !d.res_begin && !d.res_end && !g.layers[i + 1].d.res_begin && !g.layers[i + 1].d.res_end) {
+      Layer& ly2 = g.layers[i + 1];
+      LayerArgs a2 = a;
+      set_layer(a2, ly2, sh[i + 1]);
+      a2.res = nullptr;
+      a2.in = nullptr;
+      a2.in_mode = IO_ACT16;
+      a2.out_mode = io_out.mode;
+      a2.out = io_out.mode == IO_ACT ? nullptr : io_out.out;
+      a2.geo = io_out.geo;
+      if (a2.out && fused_dec_supported(a, d.kind, a2, ly2.d.kind)) {
+        int nl = 0;
+        rc = launch_fused_dec(h->stream, a, a2, ly.w, ly2.w, ly.hb.data(), ly2.hb.data(), &ly.fdw, h->num_sms, &h->err, &nl);
+        h->launches += nl;
+        fused = true;
       }
     }
+    // ... and the first two layers of an encoder (u8 image -> 3 -> 32 -> 32, both stride 2): tic_fused_enc16.cuh
+    if (!fused && pair16 && i == 0 && cur < 0 && L >= 3 && !g.layers[1].d.res_begin && !g.layers[1].d.res_end) {
+      Layer& ly2 = g.layers[1];
+      LayerArgs a2 = a;
+      set_layer(a2, ly2, sh[1]);
+      a2.res = nullptr;
+      a2.in = nullptr;
+      a2.in_mode = IO_ACT16;
+      a2.out_mode = IO_ACT16;
+      a2.out = h->act[0];
+      a2.out_lo_off = (long long)n * a2.hout * a2.wout * a2.cout;
+      if (fused_enc_supported(a, d.kind, d.stride, a2, ly2.d.kind, ly2.d.stride)) {
+        int nl = 0;
+        rc = launch_fused_enc(h->stream, a, a2, ly.w, ly2.w, ly.hb.data(), &ly.few, h->num_sms, &h->err, &nl);
+        h->launches += nl;
+        fused = true;
+        ob = 0;  // the pair's output lives in act[0]
+      }
+    }
+    if (fused) {
+      ++i;  // the next layer ran inside this launch (its time is reported with this layer)
+    } else if (pair16 && f16_first_supported(a, d.kind, d.stride)) {
+      int nl = 0;
+      rc = launch_first16(h->stream, a, d.stride, ly.w, &ly.fw16, h->num_sms, &h->err, &nl);
+      h->launches += nl;
+    } else if (pair16 && u16_supported(a, d.kind, d.stride)) {
+      int nl = 0;
+      rc = launch_u16(h->stream, a, d.kind, d.stride, ly.w, &ly.uw16, h->num_sms, &h->err, &nl);
+      h->launches += nl;
+    } else if (h->mode != TIC_COMPUTE_FP32 && !pair16 && umma_supported(a, d.kind, d.stride)) {
+      int nl = 0;
+      rc = launch_umma(h->stream, a, d.kind, d.stride, ly.w, &ly.uw, h->mode == TIC_COMPUTE_TENSOR_3XTF32, h->num_sms,
+                       &h->err, &nl);
+      h->launches += nl;
+    } else {
+      rc = launch_simt(h, a, d.kind, d.stride);
+    }
+    if (h->profile) {
+      cudaEventRecord(pr.e1, h->stream);
+      h->prof_pending.push_back(pr);
+    }
+    if (rc != TIC_OK) return rc < 0 && rc >= TIC_ERR_UNSUPPORTED ? rc : TIC_ERR_CUDA;
+    if (d.res_end) {
+      res_buf = -1;
+      res_ptr = nullptr;
+    }
+    cur = ob;
   }
   return TIC_OK;
 }
@@ -660,38 +527,15 @@ int patches_per_chunk(const tic_codec* h, int P) {
 // 2, 4, 8, 18, 18, 8, 4, 2 images) was measured SLOWER (11.3 Gpixel/s): the round trip is bound by the D2H direction
 // running next to the H2D (654 MB at 50 GB/s under duplex load, tools/pcie_probe.py), and large chunks leave it idle
 // at both ends.
-// TIC_HOST_RAMP=1 selects the ramp, TIC_HOST_CHUNKS the equal-chunk count.
 std::vector<int64_t> host_chunk_schedule(int64_t units, int64_t cap, double patches128_per_unit) {
-  const bool ramp = tic_env_set("TIC_HOST_RAMP");                      // -DTIC_ABLATE builds only
-  const int want = std::max(1, tic_env_int("TIC_HOST_CHUNKS", 16));   // -DTIC_ABLATE builds only
   cap = std::max<int64_t>(1, std::min(cap, units));
+  int64_t chunks = (units + cap - 1) / cap;
+  const int64_t by_size = (int64_t)((double)units * patches128_per_unit / 768.0);
+  chunks = std::max<int64_t>(chunks, std::min<int64_t>(16, by_size));
+  chunks = std::max<int64_t>(1, std::min<int64_t>(chunks, units));
+  const int64_t upc = (units + chunks - 1) / chunks;
   std::vector<int64_t> out;
-  if (!ramp) {
-    int64_t chunks = (units + cap - 1) / cap;
-    const int64_t by_size = (int64_t)((double)units * patches128_per_unit / 768.0);
-    chunks = std::max<int64_t>(chunks, std::min<int64_t>(want, by_size));
-    chunks = std::max<int64_t>(1, std::min<int64_t>(chunks, units));
-    const int64_t upc = (units + chunks - 1) / chunks;
-    for (int64_t u0 = 0; u0 < units; u0 += upc) out.push_back(std::min<int64_t>(upc, units - u0));
-    return out;
-  }
-  std::vector<int64_t> up;
-  int64_t ramp_units = 0;
-  int64_t v = std::max<int64_t>(1, (int64_t)(384.0 / std::max(patches128_per_unit, 1e-9) + 0.999));
-  while (v < cap && 2 * (ramp_units + v) <= units / 2) {
-    up.push_back(v);
-    ramp_units += v;
-    v *= 2;
-  }
-  out = up;
-  const int64_t rem = units - 2 * ramp_units;
-  const int64_t nmid = (rem + cap - 1) / cap;
-  for (int64_t i = 0, left = rem; i < nmid; ++i) {
-    const int64_t c = (left + (nmid - i) - 1) / (nmid - i);
-    out.push_back(c);
-    left -= c;
-  }
-  for (auto it = up.rbegin(); it != up.rend(); ++it) out.push_back(*it);
+  for (int64_t u0 = 0; u0 < units; u0 += upc) out.push_back(std::min<int64_t>(upc, units - u0));
   return out;
 }
 
@@ -909,8 +753,6 @@ void tic_destroy(tic_codec* h) {
   }
   for (int i = 0; i < 3; ++i)
     if (h->act[i]) cudaFree(h->act[i]);
-  for (int i = 0; i < 2; ++i)
-    if (h->bnd[i]) cudaFree(h->bnd[i]);
   for (int b = 0; b < 2; ++b) {
     if (h->stage_in[b]) cudaFree(h->stage_in[b]);
     if (h->stage_out[b]) cudaFree(h->stage_out[b]);
@@ -1094,7 +936,7 @@ int tic_bottleneck_shape(tic_codec* h, int P, int* hb, int* wb, int* cb) {
   Graph& g = h->g[TIC_GRAPH_ENCODER];
   if (g.layers.empty()) return fail(h, TIC_ERR_STATE, "encoder graph not configured");
   Shape so;
-  if (graph_out_shape(g, Shape{P, P, g.layers[0].d.cin}, &so, nullptr) != 0) return fail(h, TIC_ERR_INVALID, "inconsistent graph");
+  if (graph_out_shape(g, Shape{P, P, g.layers[0].d.cin}, &so) != 0) return fail(h, TIC_ERR_INVALID, "inconsistent graph");
   if (hb) *hb = so.h;
   if (wb) *wb = so.w;
   if (cb) *cb = so.c;
@@ -1170,7 +1012,7 @@ int tic_decode_patches(tic_codec* h, const uint8_t* symbols, int64_t n, int hb, 
   Graph& g = h->g[TIC_GRAPH_DECODER];
   const int cb = g.layers[0].d.cin;
   Shape so;
-  if (graph_out_shape(g, Shape{hb, wb, cb}, &so, nullptr) != 0) return fail(h, TIC_ERR_INVALID, "inconsistent graph");
+  if (graph_out_shape(g, Shape{hb, wb, cb}, &so) != 0) return fail(h, TIC_ERR_INVALID, "inconsistent graph");
   if (so.c != 3 || so.h != so.w) return fail(h, TIC_ERR_INVALID, "decoder must produce square RGB patches (got %dx%dx%d)", so.h, so.w, so.c);
   const int P = so.h;
   return drive(h, mem, symbols, recon, n, patches_per_chunk(h, P), (size_t)hb * wb * cb, (size_t)P * P * 3 * 4, false,
@@ -1204,7 +1046,7 @@ int tic_decode_images(tic_codec* h, const uint8_t* symbols, int64_t n_images, in
   if (P % up != 0) return fail(h, TIC_ERR_INVALID, "patch size %d is not a multiple of the decoder upsampling %d", P, up);
   const int hb = P / up, wb = P / up;
   Shape so;
-  if (graph_out_shape(g, Shape{hb, wb, cb}, &so, nullptr) != 0 || so.c != 3 || so.h != P)
+  if (graph_out_shape(g, Shape{hb, wb, cb}, &so) != 0 || so.c != 3 || so.h != P)
     return fail(h, TIC_ERR_INVALID, "decoder graph does not map %dx%d symbols to %dx%d RGB", hb, wb, P, P);
   const Geo g0 = image_geo(H, W, P, 0);
   const int ppi = g0.gh * g0.gw;
@@ -1253,7 +1095,7 @@ int tic_roundtrip_images(tic_codec* h, const uint8_t* images, int64_t n_images, 
   if (rc != TIC_OK) return rc;
   Graph& gd = h->g[TIC_GRAPH_DECODER];
   Shape so;
-  if (gd.layers[0].d.cin != cb || graph_out_shape(gd, Shape{hb, wb, cb}, &so, nullptr) != 0 || so.c != 3 || so.h != P || so.w != P)
+  if (gd.layers[0].d.cin != cb || graph_out_shape(gd, Shape{hb, wb, cb}, &so) != 0 || so.c != 3 || so.h != P || so.w != P)
     return fail(h, TIC_ERR_INVALID, "decoder graph does not map the encoder's %dx%dx%d symbols back to %dx%d RGB", hb, wb, cb, P, P);
   if (n_images == 0) return TIC_OK;
   TIC_CUDA(h, cudaSetDevice(h->device));
@@ -1332,7 +1174,7 @@ int tic_postfilter_patches(tic_codec* h, const float* tiles, int64_t n, int P, f
   if (rc != TIC_OK) return rc;
   Graph& g = h->g[TIC_GRAPH_POSTFILTER];
   Shape so;
-  if (g.layers[0].d.cin != 3 || graph_out_shape(g, Shape{P, P, 3}, &so, nullptr) != 0 || so.c != 3 || so.h != P || so.w != P)
+  if (g.layers[0].d.cin != 3 || graph_out_shape(g, Shape{P, P, 3}, &so) != 0 || so.c != 3 || so.h != P || so.w != P)
     return fail(h, TIC_ERR_INVALID, "post-filter graph must map PxPx3 to PxPx3");
   const size_t unit = (size_t)P * P * 3 * 4;
   return drive(h, mem, tiles, out, n, patches_per_chunk(h, P), unit, unit, false,
@@ -1356,7 +1198,7 @@ int tic_postfilter_images(tic_codec* h, float* images, int64_t n_images, int H, 
   Graph& g = h->g[TIC_GRAPH_POSTFILTER];
   const int P = 128, off = 64;  // submit/2/rmbe/rmbe.py:12,16
   Shape so;
-  if (g.layers[0].d.cin != 3 || graph_out_shape(g, Shape{P, P, 3}, &so, nullptr) != 0 || so.c != 3 || so.h != P || so.w != P)
+  if (g.layers[0].d.cin != 3 || graph_out_shape(g, Shape{P, P, 3}, &so) != 0 || so.c != 3 || so.h != P || so.w != P)
     return fail(h, TIC_ERR_INVALID, "post-filter graph must map 128x128x3 to 128x128x3");
   const size_t unit = (size_t)H * W * 3 * 4;
   // tiles per image of the two passes; whole images per chunk so that pass 2 reads pass-1 output
@@ -1411,7 +1253,7 @@ int tic_run_layers(tic_codec* h, int graph, const float* in, int64_t n, int h0, 
   if (g.layers[n_layers - 1].d.res_begin) return fail(h, TIC_ERR_INVALID, "cannot stop inside a residual block");
   const int cin = g.layers[0].d.cin;
   Shape so;
-  if (graph_out_shape(g, Shape{h0, w0, cin}, &so, nullptr, n_layers) != 0) return fail(h, TIC_ERR_INVALID, "inconsistent graph");
+  if (graph_out_shape(g, Shape{h0, w0, cin}, &so, n_layers) != 0) return fail(h, TIC_ERR_INVALID, "inconsistent graph");
   const size_t in_unit = (size_t)h0 * w0 * cin * 4, out_unit = (size_t)so.h * so.w * so.c * 4;
   const int64_t upc = std::max<int64_t>(1, (int64_t)h->chunk128 * 128 * 128 / ((int64_t)std::max(h0 * w0, so.h * so.w)));
   return drive(h, mem, in, out, n, upc, in_unit, out_unit, false,
@@ -1735,7 +1577,7 @@ int tic_evaluate_images(tic_codec* h, const uint8_t* images, int64_t n_images, i
   if (rc != TIC_OK) return rc;
   Graph& gd = h->g[TIC_GRAPH_DECODER];
   Shape so;
-  if (gd.layers[0].d.cin != cb || graph_out_shape(gd, Shape{hb, wb, cb}, &so, nullptr) != 0 || so.c != 3 || so.h != P || so.w != P)
+  if (gd.layers[0].d.cin != cb || graph_out_shape(gd, Shape{hb, wb, cb}, &so) != 0 || so.c != 3 || so.h != P || so.w != P)
     return fail(h, TIC_ERR_INVALID, "decoder graph does not map the encoder's %dx%dx%d symbols back to %dx%d RGB", hb, wb, cb, P, P);
   if ((rc = entropy_table_check(h, cum_freq, n_cum)) != TIC_OK) return rc;
   if (n_images == 0) return TIC_OK;

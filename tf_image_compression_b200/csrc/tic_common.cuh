@@ -10,9 +10,9 @@
 
 namespace tic {
 
-// Measurement aids (stage ablations, alternative schedules) exist only in builds made with -DTIC_ABLATE
-// (tools/build_ablate.sh).  The shipped library ignores every TIC_* environment variable: a stray variable must
-// never change what a kernel computes.
+// Measurement aids (the TIC_DBG stage switches and the fused kernels' wait counters) exist only in builds made with
+// -DTIC_ABLATE (tools/build_ablate.sh).  The shipped library ignores every TIC_* environment variable: a stray variable
+// must never change what a kernel computes.
 #ifdef TIC_ABLATE
 // wait-time accounting of the fused kernels' roles (cluster 0 only): cycles spent inside each barrier wait, summed over the
 // kernel's steps, read back by tools/fused_waits.py through tic_debug_prof_read (not part of the shipped ABI)
@@ -32,7 +32,6 @@ inline int tic_env_int(const char* name, int dflt) {
   const char* e = getenv(name);
   return e ? atoi(e) : dflt;
 }
-inline bool tic_env_set(const char* name) { return getenv(name) != nullptr; }
 #define TIC_DBG_BITS(x) (x)
 #else
 #define TIC_PROF_WAIT(acc, ...) \
@@ -44,7 +43,6 @@ inline bool tic_env_set(const char* name) { return getenv(name) != nullptr; }
   do {                        \
   } while (0)
 inline int tic_env_int(const char*, int dflt) { return dflt; }
-inline bool tic_env_set(const char*) { return false; }
 #define TIC_DBG_BITS(x) 0
 #endif
 

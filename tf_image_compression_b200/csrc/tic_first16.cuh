@@ -1081,9 +1081,8 @@ inline int launch_first16(cudaStream_t stream, const LayerArgs& a, int stride, c
   CUtensorMap tm_img{};
   p.use_tma = 0;
   if (windowed && f16_first_tma_ok(a)) {
-    const bool off = tic_env_set("TIC_FIRST_NO_TMA");  // -DTIC_ABLATE builds only
     auto encode = umma_encode_fn();
-    if (!off && encode) {
+    if (encode) {
       const Geo& g = a.geo;
       const long long per_img = (long long)g.gh * g.gw;
       const cuuint64_t nimg = (cuuint64_t)((g.n0 + a.n + per_img - 1) / per_img);
@@ -1106,10 +1105,8 @@ inline int launch_first16(cudaStream_t stream, const LayerArgs& a, int stride, c
       cache_k2.ensure(reinterpret_cast<const void*>(f16_first_kernel<2>), smem) != cudaSuccess ||
       cache_w2.ensure(reinterpret_cast<const void*>(f16_first_s2_kernel), smem_w2) != cudaSuccess)
     return fail("cudaFuncSetAttribute(first-layer kernel) failed", -2);
-  // the TMA-fed, pair-plane-output kernel (16 epilogue warps) when the launch qualifies; TIC_FIRST_T2=0 keeps the general one
-  const bool t2_off = tic_env_int("TIC_FIRST_T2", 1) == 0;  // -DTIC_ABLATE builds only
-  const bool t2 = windowed && p.use_tma && !t2_off && a.out_mode == IO_ACT16 && (a.cout == 32 || a.cout == 16) &&
-                  p.nbuf == 4;
+  // the TMA-fed, pair-plane-output kernel (16 epilogue warps) when the launch qualifies
+  const bool t2 = windowed && p.use_tma && a.out_mode == IO_ACT16 && (a.cout == 32 || a.cout == 16) && p.nbuf == 4;
   // the general kernel's TMA builders take u8 windows of an un-shifted grid only
   if (!t2 && (a.in_mode != IO_U8_NORM || a.geo.oy != 0 || a.geo.ox != 0)) p.use_tma = 0;
   if (t2) {

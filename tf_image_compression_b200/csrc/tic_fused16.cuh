@@ -227,10 +227,10 @@ fused_dec_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constan
           const uint32_t ah = (ptx::smem_u32(s_in + (size_t)s * slot_bytes) >> 4) | (1u << 16);
           const uint32_t al = ah + (p1.slot_bytes >> 4);
           uint32_t sp = 0, fresh = 0;
-          u16_issue_plane_t<U16_DECONV_PH, true, 2>(p1, ah, w1A_d, tmem_base, 2u * NPAD1, idesc1_st, a1_hi32, w1_hi32, tap1A >> 4, 0u, sp,
-                                                    fresh, true);
-          u16_issue_plane_t<U16_DECONV_PH, true, 2>(p1, al, w1B_d, tmem_base + (uint32_t)NPAD1, 2u * NPAD1, idesc1_lo, a1_hi32, w1_hi32,
-                                                    tap1B >> 4, 0u, sp, fresh, false);
+          u16_issue_plane_t<U16_DECONV_PH, 2>(p1, ah, w1A_d, tmem_base, 2u * NPAD1, idesc1_st, a1_hi32, w1_hi32, tap1A >> 4, 0u, sp,
+                                              fresh, true);
+          u16_issue_plane_t<U16_DECONV_PH, 2>(p1, al, w1B_d, tmem_base + (uint32_t)NPAD1, 2u * NPAD1, idesc1_lo, a1_hi32, w1_hi32,
+                                              tap1B >> 4, 0u, sp, fresh, false);
         }
         __syncwarp();
         if (ptx::elect_one()) {
@@ -254,10 +254,10 @@ fused_dec_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constan
             const uint32_t ah = reg_d + (aoff >> 4), al = ah + (kFusedRegionLoOff >> 4);
             const uint32_t d = dbase + (uint32_t)sub * 32u;
             uint32_t sp = 0, fresh = 0;
-            u16_issue_plane_t<U16_DECONV_RGB, true, 2>(p2, ah, w2A_d, d, 2u * NPAD2, idesc2_st, a2_hi32, w2_hi32, tap2A >> 4, 0u, sp, fresh,
-                                                       true);
-            u16_issue_plane_t<U16_DECONV_RGB, true, 2>(p2, al, w2B_d, d + (uint32_t)NPAD2, 2u * NPAD2, idesc2_lo, a2_hi32, w2_hi32,
-                                                       tap2B >> 4, 0u, sp, fresh, false);
+            u16_issue_plane_t<U16_DECONV_RGB, 2>(p2, ah, w2A_d, d, 2u * NPAD2, idesc2_st, a2_hi32, w2_hi32, tap2A >> 4, 0u, sp, fresh,
+                                                 true);
+            u16_issue_plane_t<U16_DECONV_RGB, 2>(p2, al, w2B_d, d + (uint32_t)NPAD2, 2u * NPAD2, idesc2_lo, a2_hi32, w2_hi32,
+                                                 tap2B >> 4, 0u, sp, fresh, false);
           }
         }
         __syncwarp();
@@ -452,14 +452,13 @@ struct FusedDecWeights {
 
 inline int u16_ensure_pair_weights(cudaStream_t stream, const float* w_dev, const LayerArgs& a, const U16Params& p, U16WeightSlice* ws) {
   const size_t img_bytes = 2 * (size_t)p.w_bytes;
-  if (!ws->img || ws->bytes != img_bytes || ws->mode != p.mode || ws->npad != p.npad || ws->oc0 != 0 || ws->pair != 1) {
+  if (!ws->img || ws->bytes != img_bytes || ws->mode != p.mode || ws->npad != p.npad || ws->oc0 != 0) {
     ws->release();
     if (cudaMalloc(&ws->img, img_bytes) != cudaSuccess) return -4;
     ws->bytes = img_bytes;
     ws->mode = p.mode;
     ws->npad = p.npad;
     ws->oc0 = 0;
-    ws->pair = 1;
     u16_build_weights_pair_kernel<<<64, 256, 0, stream>>>(w_dev, a.cin, a.cout, 0, a.cout, p.npad, p.cpad, p.mode == U16_DECONV_PH, p.kc, p.KB,
                                                           (p.wA_bytes + 1023u) & ~1023u, (p.wB_bytes + 1023u) & ~1023u, ws->img);
     if (cudaGetLastError() != cudaSuccess) return -2;
@@ -478,7 +477,7 @@ inline int launch_fused_dec(cudaStream_t stream, const LayerArgs& a1, const Laye
   if (!encode) return fail("cuTensorMapEncodeTiled is unavailable (driver too old?)", -2);
   if (num_sms < 2) return fail("the fused decoder kernel needs CTA pairs", -5);
   U16Plan pl1{}, pl2{};
-  if (!u16_plan(a1, 1, 2, a1.cout, &pl1, true) || !u16_plan(a2, 1, 2, a2.cout, &pl2, true)) return fail("fused decoder plan failed", -5);
+  if (!u16_plan(a1, 1, 2, a1.cout, &pl1) || !u16_plan(a2, 1, 2, a2.cout, &pl2)) return fail("fused decoder plan failed", -5);
   U16Params p1 = pl1.p, p2 = pl2.p;
   if (p1.mode != U16_DECONV_PH || p1.cpad != 32 || p2.mode != U16_DECONV_PH || p2.cpad != 4 || p1.ksteps != 2 || p2.ksteps != 2)
     return fail("fused decoder: unexpected layer plan", -5);

@@ -259,10 +259,10 @@ fused_enc_kernel(const __grid_constant__ CUtensorMap tm_img, const __grid_consta
         if (!(TIC_DBG_BITS(p2.dbg) & 1) && ptx::elect_one()) {
           const uint32_t d = tmem_base + 256u + b * 64u;
           uint32_t sp = 0, fresh = 1;
-          u16_issue_plane_t<U16_S2, true, 2>(p2, reg_d, w2A_d, d, 2u * NPAD2, idesc2_st, a2_hi32, w2_hi32, tap2A >> 4, 0u, sp, fresh, true);
+          u16_issue_plane_t<U16_S2, 2>(p2, reg_d, w2A_d, d, 2u * NPAD2, idesc2_st, a2_hi32, w2_hi32, tap2A >> 4, 0u, sp, fresh, true);
           fresh = 0;
-          u16_issue_plane_t<U16_S2, true, 2>(p2, reg_d + (kFERegionPlane >> 4), w2B_d, d + (uint32_t)NPAD2, 2u * NPAD2, idesc2_lo, a2_hi32,
-                                             w2_hi32, tap2B >> 4, 0u, sp, fresh, false);
+          u16_issue_plane_t<U16_S2, 2>(p2, reg_d + (kFERegionPlane >> 4), w2B_d, d + (uint32_t)NPAD2, 2u * NPAD2, idesc2_lo, a2_hi32,
+                                       w2_hi32, tap2B >> 4, 0u, sp, fresh, false);
         }
         __syncwarp();
         if (ptx::elect_one()) {
@@ -601,7 +601,7 @@ inline int launch_fused_enc(cudaStream_t stream, const LayerArgs& a1, const Laye
   if (!encode) return fail("cuTensorMapEncodeTiled is unavailable (driver too old?)", -2);
   if (num_sms < 2) return fail("the fused encoder kernel needs CTA pairs", -5);
   U16Plan pl2{};
-  if (!u16_plan(a2, 0, 2, a2.cout, &pl2, true)) return fail("fused encoder plan failed", -5);
+  if (!u16_plan(a2, 0, 2, a2.cout, &pl2)) return fail("fused encoder plan failed", -5);
   U16Params p2 = pl2.p;
   if (p2.mode != U16_S2 || p2.nbox != 1 || p2.ksteps != 2 || p2.KB != 1 || p2.bn != 1 || p2.npad != 32 || p2.nsplit != 1)
     return fail("fused encoder: unexpected layer plan", -5);

@@ -53,7 +53,6 @@ namespace tic {
 enum U16Mode : int { U16_S1 = 0, U16_S2 = 1, U16_DECONV = 2, U16_DECONV_PH = 3, U16_DECONV_RGB = 4 };
 __host__ __device__ constexpr bool u16_is_ph(int mode) { return mode == U16_DECONV_PH || mode == U16_DECONV_RGB; }
 
-constexpr int kU16Threads = 384;
 constexpr int kU16MaxSlots = 8;
 
 struct U16Params {
@@ -98,7 +97,7 @@ struct U16Params {
 struct U16WeightSlice {
   uint8_t* img = nullptr;
   size_t bytes = 0;
-  int mode = -1, npad = 0, oc0 = -1, pair = -1;
+  int mode = -1, npad = 0, oc0 = -1;
   void release() {
     if (img) cudaFree(img);
     img = nullptr;
@@ -118,54 +117,6 @@ __host__ __device__ inline uint32_t u16_swz(uint32_t off, uint32_t rowbytes) {
   return off ^ (((off >> 7) & mask) << 4);
 }
 __host__ __device__ inline uint32_t u16_layout_code(uint32_t rowbytes) { return rowbytes >= 128 ? 2u : rowbytes == 64 ? 4u : 6u; }
-
-// device [9][cin][cout] fp32 -> [kb][tap][hi rows npad | lo' rows npad][kc] fp16, swizzled rows of kc * 2 bytes
-__global__ void u16_build_weights_kernel(const float* __restrict__ w, int cin, int cout, int oc0, int cs, int npad, int kc,
-                                         int KB, uint8_t* __restrict__ img) {
-  const uint32_t wrow = (uint32_t)kc * 2u;
-  const uint32_t tap_bytes = 2u * npad * wrow;
-  const long long total = (long long)KB * 9 * npad * kc;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const int k = (int)(i % kc);
-    const int oc = (int)((i / kc) % npad);
-    const int t = (int)(i / ((long long)kc * npad));
-    const int kb = t / 9, tap = t % 9;
-    const int ic = kb * kc + k;
-    const float v = (oc < cs && ic < cin) ? w[((size_t)tap * cin + ic) * cout + oc0 + oc] : 0.f;
-    __half hi, lo;
-    split16(v, hi, lo);
-    uint8_t* base = img + (size_t)t * tap_bytes;
-    *reinterpret_cast<__half*>(base + u16_swz((uint32_t)oc * wrow + k * 2, wrow)) = hi;
-    *reinterpret_cast<__half*>(base + u16_swz((uint32_t)(npad + oc) * wrow + k * 2, wrow)) = lo;
-  }
-}
-
-// phase-stacked transposed conv: [kb][view dy*2+dx][hi rows neff | lo' rows neff][kc], row = phase * cpad + oc
-__global__ void u16_build_weights_ph_kernel(const float* __restrict__ w, int cin, int cout, int oc0, int cs, int neff, int cpad,
-                                            int kc, int KB, uint8_t* __restrict__ img) {
-  const uint32_t wrow = (uint32_t)kc * 2u;
-  const uint32_t view_bytes = 2u * neff * wrow;
-  const long long total = (long long)KB * 4 * neff * kc;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const int k = (int)(i % kc);
-    const int row = (int)((i / kc) % neff);
-    const int t = (int)(i / ((long long)kc * neff));
-    const int kb = t / 4, view = t % 4;
-    const int dy = view >> 1, dx = view & 1;
-    const int ph = row / cpad, oc = row % cpad;
-    const int py = ph >> 1, px = ph & 1;
-    const int kh = py ? (dy ? 1 : -1) : (dy ? 0 : 2);
-    const int kw = px ? (dx ? 1 : -1) : (dx ? 0 : 2);
-    const int ic = kb * kc + k;
-    float v = 0.f;
-    if (ph < 4 && kh >= 0 && kw >= 0 && oc < cs && ic < cin) v = w[((size_t)(kh * 3 + kw) * cin + ic) * cout + oc0 + oc];
-    __half hi, lo;
-    split16(v, hi, lo);
-    uint8_t* base = img + (size_t)t * view_bytes;
-    *reinterpret_cast<__half*>(base + u16_swz((uint32_t)row * wrow + k * 2, wrow)) = hi;
-    *reinterpret_cast<__half*>(base + u16_swz((uint32_t)(neff + row) * wrow + k * 2, wrow)) = lo;
-  }
-}
 
 // CTA-pair weight image = the exact per-CTA shared-memory layout, per rank r of the pair:
 //   region A [kb][tap][rows nn]   : r = 0 -> W_hi rows, r = 1 -> W_lo' rows      (stacked product, N = 2 nn over the pair)
@@ -763,7 +714,7 @@ __device__ __forceinline__ void u16_epilogue_tile_staged(const LayerArgs& a, con
 // KS = MMAs (K = 16) per tap and K-block, compile-time: with a run-time bound the unrolled body carries four
 // predicated instruction groups per tap, and the issuing warp's instruction stream — not the tensor pipe — is what
 // bounds the layers with small N (TIC_DBG=6: 105 cycles per MMA in decode_0 against 58 in the rate probe).
-template <int MODE, bool PAIR, int KS>
+template <int MODE, int KS>
 __device__ __forceinline__ void u16_issue_plane_t(const U16Params& p, uint32_t abase, uint32_t wbase, uint32_t dplane,
                                                   uint32_t pairw, uint32_t idesc, uint32_t a_hi32, uint32_t w_hi32,
                                                   uint32_t tapw, uint32_t smask, uint32_t& sp, uint32_t& fresh_left,
@@ -790,200 +741,22 @@ __device__ __forceinline__ void u16_issue_plane_t(const U16Params& p, uint32_t a
         accumulate = fresh_left ? 0u : 1u;
         fresh_left = fresh_left ? fresh_left - 1u : 0u;
       }
-      if (PAIR)
-        ptx::mma2_f16_ss(d, u16_desc(ad + 2u * ks, a_hi32), u16_desc(bd + 2u * ks, w_hi32), idesc, accumulate);
-      else
-        ptx::mma_f16_ss(d, u16_desc(ad + 2u * ks, a_hi32), u16_desc(bd + 2u * ks, w_hi32), idesc, accumulate);
+      ptx::mma2_f16_ss(d, u16_desc(ad + 2u * ks, a_hi32), u16_desc(bd + 2u * ks, w_hi32), idesc, accumulate);
     }
   }
 }
 
-template <int MODE, bool PAIR = false>
+template <int MODE>
 __device__ __forceinline__ void u16_issue_plane(const U16Params& p, uint32_t abase, uint32_t wbase, uint32_t dplane,
                                                 uint32_t pairw, uint32_t idesc, uint32_t a_hi32, uint32_t w_hi32,
                                                 uint32_t tapw, int ksteps, uint32_t smask, uint32_t& sp, uint32_t& fresh_left,
                                                 bool fresh_kb) {
   if (ksteps == 2)  // 32-channel K-blocks
-    u16_issue_plane_t<MODE, PAIR, 2>(p, abase, wbase, dplane, pairw, idesc, a_hi32, w_hi32, tapw, smask, sp, fresh_left, fresh_kb);
+    u16_issue_plane_t<MODE, 2>(p, abase, wbase, dplane, pairw, idesc, a_hi32, w_hi32, tapw, smask, sp, fresh_left, fresh_kb);
   else if (ksteps == 4)  // 64-channel K-blocks
-    u16_issue_plane_t<MODE, PAIR, 4>(p, abase, wbase, dplane, pairw, idesc, a_hi32, w_hi32, tapw, smask, sp, fresh_left, fresh_kb);
+    u16_issue_plane_t<MODE, 4>(p, abase, wbase, dplane, pairw, idesc, a_hi32, w_hi32, tapw, smask, sp, fresh_left, fresh_kb);
   else
-    u16_issue_plane_t<MODE, PAIR, 1>(p, abase, wbase, dplane, pairw, idesc, a_hi32, w_hi32, tapw, smask, sp, fresh_left, fresh_kb);
-}
-
-template <int MODE>
-__global__ void __launch_bounds__(kU16Threads, 1)
-u16_conv_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant__ CUtensorMap tm_lo, const U16Params p,
-                const LayerArgs a) {
-  const int NPAD = p.npad;
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint8_t* s_w = smem;                                             // resident weights
-  uint8_t* s_a = smem + ((p.w_bytes + 1023u) & ~1023u);            // S plane slots
-  uint8_t* s_stage = s_a + (size_t)p.S * p.slot_bytes;             // 8 x 4 KB epilogue stages (if p.staged)
-  U16SmemBars* bars = reinterpret_cast<U16SmemBars*>(s_stage + (p.staged ? kU16StageBytes : 0u));
-  __shared__ unsigned s_hist[256];
-  __shared__ __align__(16) float s_bias[128];
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-
-  if (tid < 128) s_bias[tid] = (tid < NPAD && p.oc0 + tid < a.cout) ? a.bias[p.oc0 + tid] : 0.f;
-  if (tid == 0) {
-    ptx::mbar_init(&bars->w_full, 1);
-    for (int i = 0; i < p.S; ++i) {
-      ptx::mbar_init(&bars->full[i], 1);
-      ptx::mbar_init(&bars->empty[i], 1);
-    }
-    for (int i = 0; i < 4; ++i) {
-      ptx::mbar_init(&bars->acc_full[i], 1);
-      ptx::mbar_init(&bars->acc_empty[i], p.staged ? 4 : 8);
-    }
-    ptx::fence_barrier_init();
-  }
-  if (warp == 2) {
-    ptx::tmem_alloc(&bars->tmem_base, 512);
-    ptx::tmem_relinquish();
-  }
-  for (int i = tid; i < 256; i += kU16Threads) s_hist[i] = 0;
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = bars->tmem_base;
-
-  if (warp == 0) {
-    // ===== TMA producer: resident weights once, then per tile and K-block the hi plane and the lo' plane =====
-    if (ptx::elect_one()) {
-      ptx::prefetch_tmap(&tm_hi);
-      ptx::prefetch_tmap(&tm_lo);
-      ptx::mbar_expect_tx(&bars->w_full, p.w_bytes);
-      for (uint32_t off = 0; off < p.w_bytes; off += p.tap_bytes)
-        ptx::bulk_load(s_w + off, p.wimg + off, p.tap_bytes, &bars->w_full);
-    }
-    __syncwarp();
-    uint32_t it = 0;
-    for (long long tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
-      long long tt = tile;
-      uint32_t tq, tx, ty, tn;
-      fast_divmod((uint32_t)tt, p.tx_d, tq, tx);
-      fast_divmod(tq, p.ty_d, tn, ty);
-      const int n0 = (int)tn * p.bn;
-      const int x0 = (int)tx * 8, y0 = (int)ty * p.bh;
-      for (int kb = 0; kb < p.KB; ++kb) {
-        for (int plane = 0; plane < 2; ++plane, ++it) {
-          const int s = it % p.S;
-          ptx::mbar_wait(&bars->empty[s], ((it / p.S) & 1) ^ 1);
-          if (ptx::elect_one()) {
-            const CUtensorMap* tm = plane ? &tm_lo : &tm_hi;
-            uint8_t* dst = s_a + (size_t)s * p.slot_bytes;
-            ptx::mbar_expect_tx(&bars->full[s], p.box_bytes * (uint32_t)p.nbox);
-            if (MODE == U16_S2) {
-              if (p.nbox == 1) {
-                ptx::tma_load_5d(dst, tm, &bars->full[s], kb * p.kc, x0, 0, n0, y0);  // row = both w parities (kc == cin)
-              } else {
-                ptx::tma_load_5d(dst, tm, &bars->full[s], kb * p.kc, x0, 0, n0, y0);
-                ptx::tma_load_5d(dst + p.box_stride, tm, &bars->full[s], a.cin + kb * p.kc, x0, 0, n0, y0);
-              }
-            } else {
-              ptx::tma_load_4d(dst, tm, &bars->full[s], kb * p.kc, x0 - 1, n0, y0 - 1);
-            }
-          }
-          __syncwarp();
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===== MMA issuer: the whole warp walks the loop, one elected lane issues =====
-    const uint32_t idesc_st = ptx::make_idesc_f16(128, 2 * NPAD);  // A_hi x [W_hi ; W_lo'] -> (D_main | D_lo)
-    const uint32_t idesc_lo = ptx::make_idesc_f16(128, NPAD);      // A_lo' x W_hi -> D_lo
-    const uint32_t a_hi32 = (p.sbo >> 4) | (1u << 14) | (p.a_layout << 29);
-    const uint32_t w_hi32 = (p.w_sbo >> 4) | (1u << 14) | (p.w_layout << 29);
-    const uint32_t tapw = p.tap_bytes >> 4, pairw = 2u * (uint32_t)NPAD, smask = (uint32_t)p.nsplit - 1u;
-    const int ksteps = p.ksteps;
-    ptx::mbar_wait(&bars->w_full, 0);
-    uint32_t it = 0, ti = 0;
-    for (long long tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++ti) {
-      const uint32_t b = ti & ((uint32_t)p.nbuf - 1u);
-      const uint32_t use = ti >> p.nbshift;
-      ptx::mbar_wait(&bars->acc_empty[b], (use & 1) ^ 1);
-      ptx::tc_fence_after();
-      const uint32_t dbase = tmem_base + b * p.acc_cols;
-      for (int kb = 0; kb < p.KB; ++kb) {
-        for (int plane = 0; plane < 2; ++plane, ++it) {
-          const int s = it % p.S;
-          ptx::mbar_wait(&bars->full[s], (it / p.S) & 1);
-          ptx::tc_fence_after();
-          if (ptx::elect_one()) {
-            const uint32_t abase = (ptx::smem_u32(s_a + (size_t)s * p.slot_bytes) >> 4) | (1u << 16);
-            const uint32_t wbase = (ptx::smem_u32(s_w + (size_t)kb * (u16_is_ph(MODE) ? 4 : 9) * p.tap_bytes) >> 4) | (1u << 16);
-            uint32_t sp = 0, fresh_left = (plane == 0 && kb == 0) ? (uint32_t)p.nsplit : 0u;
-            u16_issue_plane<MODE>(p, abase, wbase, dbase + (plane ? (uint32_t)NPAD : 0u), pairw, plane ? idesc_lo : idesc_st,
-                                  a_hi32, w_hi32, tapw, ksteps, smask, sp, fresh_left, plane == 0 && kb == 0);
-          }
-          __syncwarp();
-          if (ptx::elect_one()) ptx::tc_commit(&bars->empty[s]);
-          __syncwarp();
-        }
-      }
-      if (ptx::elect_one()) ptx::tc_commit(&bars->acc_full[b]);
-      __syncwarp();
-    }
-  } else if (warp >= 4) {
-    // ===== epilogue: TMEM -> registers -> sum splits / bias / act / residual -> pair planes | f32 | symbols =====
-    const int q4 = warp & 3;            // TMEM lane quadrant this warp may access
-    const int half = (warp - 4) >> 2;   // which 16-column chunks this warp takes
-    const int m = q4 * 32 + lane;       // tile row = pixel
-    const int grp = m >> 3, xx = m & 7;
-    const int hh = grp / p.bn, nb = grp % p.bn;
-    int h_ones = 0, h_valid = 0;
-    __half2 omax = __floats2half2_rn(0.f, 0.f);
-    uint32_t ti = 0;
-    for (long long tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++ti) {
-      if (p.staged && (int)(ti & 1u) != half) continue;  // staged: a warp group owns every other tile (= one TMEM buffer)
-      const uint32_t b = ti & ((uint32_t)p.nbuf - 1u);
-      const uint32_t use = ti >> p.nbshift;
-      ptx::mbar_wait(&bars->acc_full[b], use & 1);
-      ptx::tc_fence_after();
-      long long tt = tile;
-      uint32_t tq, tx, ty, tn;
-      fast_divmod((uint32_t)tt, p.tx_d, tq, tx);
-      fast_divmod(tq, p.ty_d, tn, ty);
-      const int n = (int)tn * p.bn + nb;
-      const int yt = (int)ty * p.bh + hh, xt = (int)tx * 8 + xx;
-      const bool valid = n < p.n;
-      const uint32_t tbuf = tmem_base + ((uint32_t)(q4 * 32) << 16) + b * p.acc_cols;
-      if (p.staged) {
-        u16_epilogue_tile_staged<MODE>(a, NPAD, p.oc0, p.nsplit, tbuf, n, yt, xt, valid, s_bias,
-                                       s_stage + (size_t)(warp - 4) * kU16StagePerWarp, lane, p.cpad, &bars->acc_empty[b], 1, omax);
-        continue;  // the staged epilogue released the buffer itself
-      }
-      u16_epilogue_tile<MODE>(a, NPAD, p.oc0, p.nsplit, tbuf, n, yt, xt, valid, half, s_bias, s_hist, h_ones, h_valid, omax, p.cpad);
-      ptx::tc_fence_before();
-      __syncwarp();
-      if (lane == 0) ptx::mbar_arrive(&bars->acc_empty[b]);
-    }
-    if (ovf_hit(omax)) ovf_raise(a.oflow);
-    // symbol histogram (quantising layers): reduce the epilogue warps through shared memory
-    if (a.out_mode == IO_QUANT_U8 || a.out_mode == IO_QUANT_F32) {
-      if (a.q == 2) {
-        h_ones = __reduce_add_sync(0xffffffffu, h_ones);
-        h_valid = __reduce_add_sync(0xffffffffu, h_valid);
-        if (lane == 0) {
-          if (h_ones) atomicAdd(&s_hist[1], (unsigned)h_ones);
-          if (h_valid - h_ones) atomicAdd(&s_hist[0], (unsigned)(h_valid - h_ones));
-        }
-      }
-      asm volatile("bar.sync 1, 256;" ::: "memory");  // the eight epilogue warps only
-      for (int i = tid - 128; i < a.q; i += 256)
-        if (s_hist[i]) atomicAdd(&a.hist[i], (unsigned long long)s_hist[i]);
-    }
-  }
-
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    ptx::tc_fence_after();
-    ptx::tmem_dealloc(tmem_base, 512);
-  }
+    u16_issue_plane_t<MODE, 1>(p, abase, wbase, dplane, pairw, idesc, a_hi32, w_hi32, tapw, smask, sp, fresh_left, fresh_kb);
 }
 
 // ---- CTA-pair variant (cta_group::2) ------------------------------------------------------------------
@@ -1138,9 +911,9 @@ u16_pair_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant
                 const uint32_t wbase = plane ? (ptx::smem_u32(s_wB + (size_t)kb * T * tapB) >> 4) | (1u << 16)
                                              : (ptx::smem_u32(s_wA + (size_t)kb * T * tapA) >> 4) | (1u << 16);
                 uint32_t sp = 0, fresh_left = (plane == 0 && kb == 0) ? (uint32_t)p.nsplit : 0u;
-                u16_issue_plane<MODE, true>(p, abase, wbase, dbase + (plane ? (uint32_t)NPAD : 0u), pairw,
-                                            plane ? idesc_lo : idesc_st, a_hi32, w_hi32, (plane ? tapB : tapA) >> 4, ksteps, smask,
-                                            sp, fresh_left, plane == 0 && kb == 0);
+                u16_issue_plane<MODE>(p, abase, wbase, dbase + (plane ? (uint32_t)NPAD : 0u), pairw, plane ? idesc_lo : idesc_st,
+                                      a_hi32, w_hi32, (plane ? tapB : tapA) >> 4, ksteps, smask, sp, fresh_left,
+                                      plane == 0 && kb == 0);
               }
             }
             __syncwarp();
@@ -1237,19 +1010,6 @@ inline bool u16_supported(const LayerArgs& a, int kind, int stride) {
   return true;
 }
 
-template <int MODE>
-inline cudaError_t u16_launch_t(cudaStream_t stream, const CUtensorMap& th, const CUtensorMap& tl, const U16Params& p,
-                                const LayerArgs& a, int grid, size_t smem) {
-  auto k = u16_conv_kernel<MODE>;
-  static SmemAttrCache cache;
-  {
-    cudaError_t e = cache.ensure(reinterpret_cast<const void*>(k), smem);
-    if (e != cudaSuccess) return e;
-  }
-  k<<<grid, kU16Threads, smem, stream>>>(th, tl, p, a);
-  return cudaGetLastError();
-}
-
 template <int MODE, int PPS, int EW>
 inline cudaError_t u16_launch_pair_ew(cudaStream_t stream, const CUtensorMap& th, const CUtensorMap& tl, const U16Params& p,
                                       const LayerArgs& a, int grid, size_t smem) {
@@ -1289,10 +1049,9 @@ struct U16Plan {
 
 // Geometry + shared-memory plan for one slice width; returns false if it does not fit.
 // variant: bit 0 = 32-channel K-blocks (half-size operand slots), bit 1 = no staged epilogue (its 32 KB go to the ring)
-inline bool u16_plan(const LayerArgs& a, int kind, int stride, int cs, U16Plan* out, bool pair = false, bool allow_ph = true,
-                     int variant = 0) {
+inline bool u16_plan(const LayerArgs& a, int kind, int stride, int cs, U16Plan* out, int variant = 0) {
   U16Params p{};
-  p.pair = pair ? 1 : 0;
+  p.pair = 1;
   p.mode = u16_mode_of(kind, stride);
   p.n = a.n;
   p.Ht = p.mode == U16_DECONV ? a.hin : a.hout;
@@ -1309,7 +1068,7 @@ inline bool u16_plan(const LayerArgs& a, int kind, int stride, int cs, U16Plan* 
   p.KB = a.cin / p.kc;
   p.ksteps = p.kc / 16;
   p.npad = (cs + 15) / 16 * 16;
-  if (p.mode == U16_DECONV && cs <= 32 && (allow_ph || a.cout <= 32)) {
+  if (p.mode == U16_DECONV && cs <= 32) {
     p.mode = U16_DECONV_PH;
     p.cpad = cs <= 4 ? 4 : (cs + 15) / 16 * 16;
     p.npad = (4 * p.cpad + 15) / 16 * 16;  // N = (phase, channel)
@@ -1368,12 +1127,10 @@ inline bool u16_plan(const LayerArgs& a, int kind, int stride, int cs, U16Plan* 
   p.slot_bytes = p.box_stride * (uint32_t)p.nbox;
   p.tap_bytes = 2u * (uint32_t)p.npad * wrow;
   p.w_bytes = (uint32_t)p.KB * (p.mode == U16_DECONV_PH ? 4u : 9u) * p.tap_bytes;
-  if (pair) {
-    // each CTA of the pair keeps half of every stacked tile plus half of W_hi
-    p.wA_bytes = p.w_bytes / 2;
-    p.wB_bytes = p.w_bytes / 4;
-    p.w_bytes = ((p.wA_bytes + 1023u) & ~1023u) + ((p.wB_bytes + 1023u) & ~1023u);
-  }
+  // each CTA of the pair keeps half of every stacked tile plus half of W_hi
+  p.wA_bytes = p.w_bytes / 2;
+  p.wB_bytes = p.w_bytes / 4;
+  p.w_bytes = ((p.wA_bytes + 1023u) & ~1023u) + ((p.wB_bytes + 1023u) & ~1023u);
   // TMEM: conv nsplit pairs x 2 buffers; deconv 4 phase pairs
   const int accw = 2 * p.npad;  // one (D_main | D_lo) accumulator pair
   if (p.mode == U16_DECONV_PH) {
@@ -1397,24 +1154,20 @@ inline bool u16_plan(const LayerArgs& a, int kind, int stride, int cs, U16Plan* 
     p.acc_cols = (uint32_t)(p.nsplit * accw);
     if (p.acc_cols * 4 <= 512) p.nbuf = 4;
   }
-  // The accumulator hand-over (tcgen05.commit -> epilogue wake-up -> cross-CTA arrive -> issuer wake-up) is ~1400
-  // cycles; with two buffers that alone is ~700 cycles per tile (TIC_DBG=7 skeleton: 0.96 of decode_0's 1.95 ms).
-  {
-    const int maxbuf = tic_env_int("TIC_MAX_NBUF", 4);  // -DTIC_ABLATE builds only
-    while (p.nbuf > maxbuf && p.nbuf > 1) p.nbuf /= 2;
-  }
+  // Four tile buffers wherever TMEM holds them: the accumulator hand-over (tcgen05.commit -> epilogue wake-up -> cross-CTA
+  // arrive -> issuer wake-up) is ~1400 cycles; with two buffers that alone is ~700 cycles per tile (TIC_DBG=7 skeleton:
+  // 0.96 of decode_0's 1.95 ms).
   p.nbshift = p.nbuf == 4 ? 2 : (p.nbuf == 2 ? 1 : 0);
   p.dbg = tic_env_int("TIC_DBG", 0);  // -DTIC_ABLATE builds only
   if (2 * p.npad > 256) return false;  // MMA N limit for the stacked product
   // (phase-stacked output-channel slices keep the staged epilogue: a slice owns 64 contiguous bytes of every pixel row)
-  p.staged = u16_staged_ok(a, p.mode, p.nbuf, p.mode == U16_DECONV_PH ? p.cpad : p.npad, p.mode == U16_DECONV_PH,
-                           tic_env_int("TIC_STAGED64", 1) != 0) ? 1 : 0;   // knob: -DTIC_ABLATE builds only
+  p.staged = u16_staged_ok(a, p.mode, p.nbuf, p.mode == U16_DECONV_PH ? p.cpad : p.npad, p.mode == U16_DECONV_PH, true) ? 1 : 0;
   if (variant & 2) p.staged = 0;
   const size_t budget = 227 * 1024 - 2048 /* static histogram + bias */ - 1024 /* alignment slack */ - sizeof(U16SmemBars) - 256;
   const size_t wres = ((p.w_bytes + 1023u) & ~1023u) + (p.staged ? kU16StageBytes : 0u);
   if (wres + 2 * (size_t)p.slot_bytes > budget) return false;
   p.S = (int)std::min<size_t>(kU16MaxSlots, (budget - wres) / p.slot_bytes);
-  if (pair && p.S >= 4) p.S &= ~1;  // the pair kernel's ring slots hold both planes when four plane buffers fit
+  if (p.S >= 4) p.S &= ~1;  // the pair kernel's ring slots hold both planes when four plane buffers fit
   out->cs = cs;
   out->variant = variant;
   out->p = p;
@@ -1430,32 +1183,24 @@ inline int launch_u16(cudaStream_t stream, const LayerArgs& a, int kind, int str
   };
   auto encode = umma_encode_fn();
   if (!encode) return fail("cuTensorMapEncodeTiled is unavailable (driver too old?)", -2);
+  if (num_sms < 2) return fail("the fp16-pair tensor kernels need CTA pairs", -5);
   // widest output-channel slice whose weights stay resident
-  const bool pair_enabled = tic_env_int("TIC_U16_PAIR", 1) != 0;  // -DTIC_ABLATE builds only
-  const bool pair = pair_enabled && num_sms >= 2;
   U16Plan plan{};
   int cs = std::min(a.cout, 128);
   // Transposed convs with 64 or more output channels run as phase-stacked 32-channel slices WITH the staged epilogue:
   // decode_3 (64 -> 64 on 8 x 8 maps) 0.42 ms tap-based (one TMEM buffer, epilogue-bound on 16-byte strided stores), 0.37 ms
   // as slices with the direct epilogue, 0.28 ms as slices with the staged one; the input (small) is read once per slice.
-  if (kind == 1 && a.cout >= 64 && a.cout % 32 == 0 && tic_env_int("TIC_DECONV_TAP", 0) == 0) cs = std::min(cs, 32);
-  // (ablation builds) tap-based slices of 32 output channels: two TMEM buffers instead of one (the unsliced 64-channel
-  // tile needs all 512 columns, so its MMAs and its epilogue alternate).  Measured on decode_3: 2 x 0.205 ms against
-  // 0.414 ms unsliced, identical output — the layer is bound by its epilogue's 16-byte strided stores, not by the
-  // missing overlap, so the default stays one launch.
-  const bool tap_slices = kind == 1 && a.cout == 64 && tic_env_int("TIC_DECONV_TAP_SLICES", 0) != 0;
-  if (tap_slices) cs = std::min(cs, 32);
-  cs = (cs + 15) / 16 * 16;
+  if (kind == 1 && a.cout >= 64 && a.cout % 32 == 0) cs = std::min(cs, 32);
+  cs =  (cs + 15) / 16 * 16;
   bool ok = false;
   // A stride-2 conv with 64 input channels whose full-width plan does not fit (two 83 KB parity boxes per plane next to
   // 110 KB of weights) is tried with 32-channel K-blocks before its output channels are sliced: the slices each re-read
   // the input (encode_3: 2 x 0.145 ms at 6.2 TB/s).
-  const int small_kc_knob = tic_env_int("TIC_SMALL_KC", 1);  // knob: -DTIC_ABLATE builds only (2: any conv with >= 64 input channels)
-  const bool small_kc = (kind == 0 && stride == 2 && a.cin == 64 && small_kc_knob != 0) || (kind == 0 && a.cin >= 64 && small_kc_knob == 2);
+  const bool small_kc = kind == 0 && stride == 2 && a.cin == 64;
   for (; cs >= 16; cs -= 16) {
     const int csl = std::min(cs, a.cout);
-    ok = u16_plan(a, kind, stride, csl, &plan, pair, !tap_slices);
-    if (!ok && small_kc) ok = u16_plan(a, kind, stride, csl, &plan, pair, !tap_slices, 1) || u16_plan(a, kind, stride, csl, &plan, pair, !tap_slices, 3);
+    ok = u16_plan(a, kind, stride, csl, &plan);
+    if (!ok && small_kc) ok = u16_plan(a, kind, stride, csl, &plan, 1) || u16_plan(a, kind, stride, csl, &plan, 3);
     if (ok) break;
   }
   if (!ok) return fail("layer does not fit the fp16-pair tensor path", -5);
@@ -1494,56 +1239,36 @@ inline int launch_u16(cudaStream_t stream, const LayerArgs& a, int kind, int str
     if (si >= 16) return fail("too many output-channel slices", -5);
     const int csl = std::min(cs, a.cout - oc0);
     U16Plan pl{};
-    if (!u16_plan(a, kind, stride, csl, &pl, pair, !tap_slices, plan.variant)) return fail("slice plan failed", -5);
+    if (!u16_plan(a, kind, stride, csl, &pl, plan.variant)) return fail("slice plan failed", -5);
     U16Params p = pl.p;
     p.oc0 = oc0;
     U16WeightSlice* ws = &uw->slice[si];
-    const size_t img_bytes = pair ? 2 * (size_t)p.w_bytes : (size_t)p.w_bytes;
-    if (!ws->img || ws->bytes != img_bytes || ws->mode != p.mode || ws->npad != p.npad || ws->oc0 != oc0 || ws->pair != p.pair) {
+    const size_t img_bytes = 2 * (size_t)p.w_bytes;
+    if (!ws->img || ws->bytes != img_bytes || ws->mode != p.mode || ws->npad != p.npad || ws->oc0 != oc0) {
       ws->release();
       if (cudaMalloc(&ws->img, img_bytes) != cudaSuccess) return fail("cudaMalloc for weight images failed", -4);
       ws->bytes = img_bytes;
       ws->mode = p.mode;
       ws->npad = p.npad;
       ws->oc0 = oc0;
-      ws->pair = p.pair;
-      if (pair)
-        u16_build_weights_pair_kernel<<<64, 256, 0, stream>>>(w_dev, a.cin, a.cout, oc0, csl, p.npad, p.cpad, p.mode == U16_DECONV_PH,
-                                                              p.kc, p.KB, (p.wA_bytes + 1023u) & ~1023u,
-                                                              (p.wB_bytes + 1023u) & ~1023u, ws->img);
-      else if (p.mode == U16_DECONV_PH)
-        u16_build_weights_ph_kernel<<<64, 256, 0, stream>>>(w_dev, a.cin, a.cout, oc0, csl, p.npad, p.cpad, p.kc, p.KB, ws->img);
-      else
-        u16_build_weights_kernel<<<64, 256, 0, stream>>>(w_dev, a.cin, a.cout, oc0, csl, p.npad, p.kc, p.KB, ws->img);
+      u16_build_weights_pair_kernel<<<64, 256, 0, stream>>>(w_dev, a.cin, a.cout, oc0, csl, p.npad, p.cpad, p.mode == U16_DECONV_PH,
+                                                            p.kc, p.KB, (p.wA_bytes + 1023u) & ~1023u,
+                                                            (p.wB_bytes + 1023u) & ~1023u, ws->img);
       if (cudaGetLastError() != cudaSuccess) return fail("weight image kernel failed", -2);
     }
     p.wimg = ws->img;
+    const int grid = 2 * (int)std::min<long long>((p.num_tiles + 1) / 2, num_sms / 2);
     cudaError_t e;
-    if (pair) {
-      const int grid = 2 * (int)std::min<long long>((p.num_tiles + 1) / 2, num_sms / 2);
-      if (p.mode == U16_S1)
-        e = u16_launch_pair_t<U16_S1>(stream, tm[0], tm[1], p, a, grid, pl.smem);
-      else if (p.mode == U16_S2)
-        e = u16_launch_pair_t<U16_S2>(stream, tm[0], tm[1], p, a, grid, pl.smem);
-      else if (p.mode == U16_DECONV_PH && p.cpad == 4)
-        e = u16_launch_pair_t<U16_DECONV_RGB>(stream, tm[0], tm[1], p, a, grid, pl.smem);
-      else if (p.mode == U16_DECONV_PH)
-        e = u16_launch_pair_t<U16_DECONV_PH>(stream, tm[0], tm[1], p, a, grid, pl.smem);
-      else
-        e = u16_launch_pair_t<U16_DECONV>(stream, tm[0], tm[1], p, a, grid, pl.smem);
-    } else {
-      const int grid = (int)std::min<long long>(p.num_tiles, num_sms);
-      if (p.mode == U16_S1)
-        e = u16_launch_t<U16_S1>(stream, tm[0], tm[1], p, a, grid, pl.smem);
-      else if (p.mode == U16_S2)
-        e = u16_launch_t<U16_S2>(stream, tm[0], tm[1], p, a, grid, pl.smem);
-      else if (p.mode == U16_DECONV_PH && p.cpad == 4)
-        e = u16_launch_t<U16_DECONV_RGB>(stream, tm[0], tm[1], p, a, grid, pl.smem);
-      else if (p.mode == U16_DECONV_PH)
-        e = u16_launch_t<U16_DECONV_PH>(stream, tm[0], tm[1], p, a, grid, pl.smem);
-      else
-        e = u16_launch_t<U16_DECONV>(stream, tm[0], tm[1], p, a, grid, pl.smem);
-    }
+    if (p.mode == U16_S1)
+      e = u16_launch_pair_t<U16_S1>(stream, tm[0], tm[1], p, a, grid, pl.smem);
+    else if (p.mode == U16_S2)
+      e = u16_launch_pair_t<U16_S2>(stream, tm[0], tm[1], p, a, grid, pl.smem);
+    else if (p.mode == U16_DECONV_PH && p.cpad == 4)
+      e = u16_launch_pair_t<U16_DECONV_RGB>(stream, tm[0], tm[1], p, a, grid, pl.smem);
+    else if (p.mode == U16_DECONV_PH)
+      e = u16_launch_pair_t<U16_DECONV_PH>(stream, tm[0], tm[1], p, a, grid, pl.smem);
+    else
+      e = u16_launch_pair_t<U16_DECONV>(stream, tm[0], tm[1], p, a, grid, pl.smem);
     if (e != cudaSuccess) return fail(std::string("fp16-pair tensor launch failed: ") + cudaGetErrorString(e), -2);
     if (launches) ++*launches;
   }
