@@ -409,7 +409,8 @@ def test_cfg5_model1_decode_and_rmbe(mode):
 @pytest.mark.parametrize("mode", MODES)
 def test_roundtrip_equals_encode_then_decode(mode):
     """tic_roundtrip_images (test.py:95-146, encoder and decoder in one graph) == tic_encode_images followed by
-    tic_decode_images, bit for bit: host buffers (streamed, several chunks, pinned and pageable), device buffers,
+    tic_decode_images, bit for bit: host buffers (streamed, several chunks, pinned and pageable), device buffers (one
+    launch sequence and two),
     images that need reflect padding, float output, no symbol read-back; the histogram counts every symbol once."""
     codec, enc, dec = make_codec("model_0", "fanin", compute=mode)
     rs = np.random.RandomState(77)
@@ -436,6 +437,10 @@ def test_roundtrip_equals_encode_then_decode(mode):
     from tf_image_compression_b200 import entry
     outs = entry.compress_and_uncompress(codec, [imgs[0], imgs[1][:200, :256].copy(), imgs[2]], {"patch_size": 128})
     assert np.array_equal(outs[0], rec[0]) and np.array_equal(outs[2], rec[2]) and outs[1].shape == (200, 256, 3)
+    # device buffers over two launch sequences (one image per chunk: 3 + 2 images), encoder then decoder per sequence
+    codec.set_chunk_patches(12)
+    rd, sd = codec.roundtrip_images(torch.from_numpy(imgs).cuda(), 128)
+    assert np.array_equal(sd.cpu().numpy(), sym) and np.array_equal(rd.cpu().numpy(), rec)
     codec.close()
 
 

@@ -6,6 +6,8 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <functional>
+#include <initializer_list>
 #include <string>
 #include <vector>
 
@@ -36,6 +38,13 @@ struct Layer {
   FusedDecWeights fdw;    // operand images of this layer and the next one for the fused transposed-conv pair
   FusedEncWeights few;    // ... for the fused first two layers of an encoder
   bool loaded = false;
+  void release() {  // the operand images (rebuilt from w on the next launch)
+    uw.release();
+    uw16.release();
+    fw16.release();
+    fdw.release();
+    few.release();
+  }
 };
 
 struct Graph {
@@ -52,6 +61,18 @@ struct IoSpec {
   Geo geo{};
 };
 
+// A device buffer that only grows (grow()).  Its destructor frees the memory.
+struct DevBuf {
+  void* p = nullptr;
+  size_t bytes = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { cudaFree(p); }
+  template <typename T>
+  T* as() const { return static_cast<T*>(p); }
+};
+
 }  // namespace
 
 struct tic_codec {
@@ -59,7 +80,7 @@ struct tic_codec {
   cudaStream_t stream = nullptr;
   bool own_stream = false;
   cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
-  cudaEvent_t ev_in[2]{}, ev_comp[2]{}, ev_out[2]{}, ev_enc[2]{}, ev_t0 = nullptr, ev_t1 = nullptr, ev_rt = nullptr;
+  cudaEvent_t ev_in[2]{}, ev_comp[2]{}, ev_out[2]{}, ev_enc[2]{}, ev_t0 = nullptr, ev_t1 = nullptr;
   Graph g[3];
   int q = 0;
   float* d_symlut = nullptr;  // [256]
@@ -67,12 +88,10 @@ struct tic_codec {
   int mode = TIC_COMPUTE_FP32;
   int chunk128 = 4096;
   // workspaces
-  float* act[3] = {nullptr, nullptr, nullptr};  // rotating chunk activations
-  size_t act_bytes = 0;
-  void* stage_in[2] = {nullptr, nullptr};
-  void* stage_out[2] = {nullptr, nullptr};
-  void* stage_sym[2] = {nullptr, nullptr};      // round trips: the symbols between the two graphs
-  size_t stage_in_bytes = 0, stage_out_bytes = 0, stage_sym_bytes = 0;
+  DevBuf act[3];        // rotating chunk activations
+  DevBuf stage_in[2];   // host-buffer staging sets
+  DevBuf stage_out[2];
+  DevBuf stage_sym[2];  // round trips: the symbols between the two graphs
   int64_t launches = 0;
   float last_ms = 0.f;
   bool profile = false;
@@ -88,11 +107,9 @@ struct tic_codec {
                                     // [1] entropy stage (1: symbol outside the table / of zero width, 2: slot too small)
   unsigned int* d_oflow = nullptr;  // their device address
   uint32_t* d_cum = nullptr;        // entropy stage: the call's cumulative-frequency table [257]
-  uint8_t* d_seg = nullptr;         // entropy stage: worst-case slots of a segmented call's pieces (grow-only)
-  long long* d_seg_bytes = nullptr; //   and their stored lengths
-  int64_t seg_cap = 0;              //   pieces both hold
-  long long* d_eval = nullptr;      // tic_evaluate_images with host buffers: per-image stored lengths, then squared errors
-  int64_t eval_cap = 0;             //   images it holds (grow-only)
+  DevBuf d_seg;                     // entropy stage: worst-case slots of a segmented call's pieces
+  DevBuf d_seg_bytes;               //   and their stored lengths (long long)
+  DevBuf d_eval;                    // tic_evaluate_images with host buffers: per-image stored lengths, then squared errors
   cudaEvent_t ev_switch = nullptr;  // orders the old stream before the new one in tic_set_stream
   std::string err;
 };
@@ -116,13 +133,35 @@ int fail(tic_codec* h, int code, const char* fmt, ...) {
       return fail((h), TIC_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__); \
   } while (0)
 
-// Error paths of the staged (host-buffer) drivers: nothing may still be copying into / out of the caller's buffers
-// or the staging sets when the call returns.
-void quiesce(tic_codec* h) {
-  cudaStreamSynchronize(h->s_h2d);
-  cudaStreamSynchronize(h->stream);
-  cudaStreamSynchronize(h->s_d2h);
+// The set bufs[0, count) grows together: each buffer holds at least `need` bytes.  Work queued earlier on any stream
+// may still use the memory a grown set frees, so the device is drained first.  A failed allocation returns `nomem`.
+int grow(tic_codec* h, DevBuf* bufs, int count, size_t need, int nomem = TIC_ERR_CUDA) {
+  if (bufs[0].bytes >= need) return TIC_OK;
+  bool held = false;
+  for (int i = 0; i < count; ++i) held = held || bufs[i].p;
+  if (held) TIC_CUDA(h, cudaDeviceSynchronize());
+  for (int i = 0; i < count; ++i) {
+    cudaFree(bufs[i].p);
+    bufs[i].p = nullptr;
+    bufs[i].bytes = 0;
+  }
+  for (int i = 0; i < count; ++i) {
+    const cudaError_t e = cudaMalloc(&bufs[i].p, need);
+    if (e != cudaSuccess) return fail(h, nomem, "cudaMalloc(%zu) failed: %s", need, cudaGetErrorString(e));
+  }
+  for (int i = 0; i < count; ++i) bufs[i].bytes = need;
+  return TIC_OK;
 }
+
+// Device temporaries of one host-buffer call.  They are freed on every return path, after the handle's stream, where
+// their copies and kernels are queued, has drained.
+struct CallTemps {
+  tic_codec* h;
+  DevBuf buf[3];
+  ~CallTemps() {
+    if (buf[0].p || buf[1].p || buf[2].p) cudaStreamSynchronize(h->stream);
+  }
+};
 
 const char* kOverflowMsg =
     "fp16-pair tensor mode: an activation reached the fp16 range limit (|x| >= 65504); results are invalid. "
@@ -307,22 +346,6 @@ int check_graph_ready(tic_codec* h, int gi, bool need_norm) {
   return TIC_OK;
 }
 
-int ensure_buffers(tic_codec* h, float** bufs, int count, size_t* have, size_t need) {
-  if (need <= *have) return TIC_OK;
-  TIC_CUDA(h, cudaStreamSynchronize(h->stream));
-  for (int i = 0; i < count; ++i) {
-    if (bufs[i]) cudaFree(bufs[i]);
-    bufs[i] = nullptr;
-  }
-  *have = 0;
-  for (int i = 0; i < count; ++i) {
-    cudaError_t e = cudaMalloc((void**)&bufs[i], need);
-    if (e != cudaSuccess) return fail(h, TIC_ERR_NOMEM, "cudaMalloc(%zu) for activations failed: %s", need, cudaGetErrorString(e));
-  }
-  *have = need;
-  return TIC_OK;
-}
-
 // The fields of a layer's launch arguments that come from the layer itself: shapes, padding, activation, weights.
 void set_layer(LayerArgs& a, const Layer& ly, const LayerShape& t) {
   a.hin = t.hin;
@@ -361,7 +384,7 @@ int run_graph(tic_codec* h, int gi, const IoSpec& io_in, const IoSpec& io_out, i
   size_t act_elems = 0;
   for (int i = 0; i + 1 < L; ++i) act_elems = std::max(act_elems, (size_t)n * sh[i].hout * sh[i].wout * sh[i].cout);
   if (split_input) act_elems = std::max(act_elems, (size_t)n * sh[0].hin * sh[0].win * sh[0].cin);
-  const int rc0 = ensure_buffers(h, h->act, 3, &h->act_bytes, act_elems * sizeof(float));
+  const int rc0 = grow(h, h->act, 3, act_elems * sizeof(float), TIC_ERR_NOMEM);
   if (rc0 != TIC_OK) return rc0;
 
   int cur = -1;        // act[] index holding the current activation (-1: the caller's input)
@@ -371,7 +394,7 @@ int run_graph(tic_codec* h, int gi, const IoSpec& io_in, const IoSpec& io_out, i
   if (split_input) {
     const long long per = (long long)sh[0].hin * sh[0].win * sh[0].cin;
     const long long count = (long long)n * per;
-    __half* hi = reinterpret_cast<__half*>(h->act[0]);
+    __half* hi = h->act[0].as<__half>();
     const int blocks = (int)std::min<long long>((count + 255) / 256, (long long)h->num_sms * 8);
     if (io_in.mode == IO_ACT)
       u16_split_f32_kernel<<<blocks, 256, 0, h->stream>>>(reinterpret_cast<const float*>(io_in.in), hi, hi + count, count, h->d_oflow);
@@ -404,7 +427,7 @@ int run_graph(tic_codec* h, int gi, const IoSpec& io_in, const IoSpec& io_out, i
       a.lut = (io_in.mode == IO_U8_NORM) ? g.d_normlut : (io_in.mode == IO_U8_SYMLUT ? h->d_symlut : nullptr);
       a.in = io_in.in;
     } else {
-      a.in = h->act[cur];
+      a.in = h->act[cur].p;
       a.in_mode = pair16 ? IO_ACT16 : IO_ACT;
       a.in_lo_off = (long long)n * ein;
     }
@@ -426,7 +449,7 @@ int run_graph(tic_codec* h, int gi, const IoSpec& io_in, const IoSpec& io_out, i
           ob = b;
           break;
         }
-      a.out = h->act[ob];
+      a.out = h->act[ob].p;
       a.out_mode = pair16 ? IO_ACT16 : IO_ACT;
       a.out_lo_off = (long long)n * eout;
     }
@@ -472,7 +495,7 @@ int run_graph(tic_codec* h, int gi, const IoSpec& io_in, const IoSpec& io_out, i
       a2.in = nullptr;
       a2.in_mode = IO_ACT16;
       a2.out_mode = IO_ACT16;
-      a2.out = h->act[0];
+      a2.out = h->act[0].p;
       a2.out_lo_off = (long long)n * a2.hout * a2.wout * a2.cout;
       if (fused_enc_supported(a, d.kind, d.stride, a2, ly2.d.kind, ly2.d.stride)) {
         int nl = 0;
@@ -549,94 +572,120 @@ std::vector<int64_t> device_chunk_schedule(int64_t units, int64_t cap) {
   return out;
 }
 
-// Both buffers of a staging set hold at least `need` bytes (grow-only; the device is drained before a buffer is freed).
-int grow_pair(tic_codec* h, void** bufs, size_t* have, size_t need) {
-  if (*have >= need) return TIC_OK;
-  TIC_CUDA(h, cudaDeviceSynchronize());
-  for (int b = 0; b < 2; ++b) {
-    if (bufs[b]) cudaFree(bufs[b]);
-    bufs[b] = nullptr;
-  }
-  *have = 0;
-  for (int b = 0; b < 2; ++b) TIC_CUDA(h, cudaMalloc(&bufs[b], need));
-  *have = need;
-  return TIC_OK;
+std::vector<int64_t> chunk_schedule(int mem, int64_t units, int64_t cap, double patches128_per_unit) {
+  return mem == TIC_MEM_DEVICE ? device_chunk_schedule(units, cap) : host_chunk_schedule(units, cap, patches128_per_unit);
 }
 
-// Generic chunked driver.  `units` are processed `upc` (units per chunk) at a time; a unit is a
-// patch or a whole image.  in_unit_bytes / out_unit_bytes describe the caller's buffers; run()
-// executes one chunk given device pointers (chunk-local when staged from host) and the unit offset.
+// One output of a driven call: the caller's buffer `dst`, `unit` bytes per unit.  With host buffers it is staged in the
+// pair `stage` and copied back chunk by chunk; dst == nullptr: the run still writes the staging buffer, nothing is
+// copied.  An `early` output is copied once the run has marked its input consumed, the others at the end of the run.
+// stage == h->stage_in: the run works in place on the input's staging buffer.
+struct Output {
+  void* dst;
+  size_t unit;
+  DevBuf* stage;
+  bool early;
+};
+
+// One chunk of a driven call, as its run callback sees it.
+struct Chunk {
+  const void* in;        // the chunk's staging buffer, or the caller's device buffer
+  void* out[2];          // the outputs, likewise (device buffers: the caller's pointers, possibly nullptr)
+  int64_t off;           // index of the chunk's first unit in `in` / `out`: 0 when staged
+  int64_t u0, nu;        // the chunk's first unit in the call, and its unit count
+  bool last;             // the call's last chunk
+  // Host buffers: marks the point on the handle's stream after which the input staging buffer may be refilled, and
+  // queues the early outputs' copies from there.  Without a mark that point is the end of the run.
+  std::function<int()> mark;
+};
+
+int mark_consumed(Chunk& c) { return c.mark ? c.mark() : (int)TIC_OK; }
+
+// The chunked driver of every call that takes host or device buffers.  `units` (patches, whole images, elements) of
+// `in_unit` bytes run in chunks of at most `upc`; run(Chunk&) queues one chunk's work on the handle's stream.  Device
+// buffers: device_chunk_schedule over the caller's pointers.  Host buffers: host_chunk_schedule over two staging sets
+// and three streams, so that the H2D of chunk i+1 (s_h2d) runs under the kernels of chunk i and the D2H of chunk i-1
+// (s_d2h).
 template <typename RunFn>
-int drive(tic_codec* h, int mem, const void* in, void* out, int64_t units, int64_t upc, size_t in_unit_bytes,
-          size_t out_unit_bytes, bool inout_same, RunFn run, double patches128_per_unit = 1.0) {
+int drive(tic_codec* h, int mem, const void* in, size_t in_unit, std::initializer_list<Output> outs, int64_t units,
+          int64_t upc, RunFn run, double patches128_per_unit = 1.0) {
   if (units <= 0) return TIC_OK;
   TIC_CUDA(h, cudaSetDevice(h->device));
+  const std::vector<int64_t> sched = chunk_schedule(mem, units, upc, patches128_per_unit);
+  Output o[2] = {};
+  std::copy(outs.begin(), outs.end(), o);
+  if (mem != TIC_MEM_DEVICE) {
+    const size_t most = (size_t)*std::max_element(sched.begin(), sched.end());
+    int rc = grow(h, h->stage_in, 2, most * in_unit);
+    for (const Output& x : outs)
+      if (rc == TIC_OK) rc = grow(h, x.stage, 2, most * x.unit);
+    if (rc != TIC_OK) return rc;
+  }
   if (int st = overflow_status(h)) return st;
   TIC_CUDA(h, cudaEventRecord(h->ev_t0, h->stream));
   if (mem == TIC_MEM_DEVICE) {
     int64_t u0 = 0;
-    for (const int64_t nu : device_chunk_schedule(units, upc)) {
-      int rc = run(in, out, u0, nu, /*local=*/false);
-      if (rc != TIC_OK) return rc;
-      u0 += nu;
+    for (size_t idx = 0; idx < sched.size(); u0 += sched[idx++]) {
+      Chunk c{in, {o[0].dst, o[1].dst}, u0, u0, sched[idx], idx + 1 == sched.size(), nullptr};
+      if (int rc = run(c)) return rc;
     }
     TIC_CUDA(h, cudaEventRecord(h->ev_t1, h->stream));
     return TIC_OK;
   }
-  // host buffers: double-buffered staging, copies on side streams
-  const std::vector<int64_t> sched = host_chunk_schedule(units, upc, patches128_per_unit);
-  upc = *std::max_element(sched.begin(), sched.end());
-  const size_t in_need = (size_t)upc * in_unit_bytes, out_need = (size_t)upc * out_unit_bytes;
-  if (h->stage_in_bytes < in_need) {
-    for (int b = 0; b < 2; ++b) {
-      if (h->stage_in[b]) cudaFree(h->stage_in[b]);
-      h->stage_in[b] = nullptr;
-    }
-    h->stage_in_bytes = 0;
-    for (int b = 0; b < 2; ++b) TIC_CUDA(h, cudaMalloc(&h->stage_in[b], in_need));
-    h->stage_in_bytes = in_need;
-  }
-  if (!inout_same && h->stage_out_bytes < out_need) {
-    for (int b = 0; b < 2; ++b) {
-      if (h->stage_out[b]) cudaFree(h->stage_out[b]);
-      h->stage_out[b] = nullptr;
-    }
-    h->stage_out_bytes = 0;
-    for (int b = 0; b < 2; ++b) TIC_CUDA(h, cudaMalloc(&h->stage_out[b], out_need));
-    h->stage_out_bytes = out_need;
+  bool in_place = false, copies = false;
+  for (const Output& x : outs) {
+    in_place = in_place || x.stage == h->stage_in;
+    copies = copies || x.dst;
   }
   // the pipeline proper runs inside a lambda: ANY failure (a CUDA call, a layer launch) drains the three streams before
   // the error is returned, so no copy is still in flight into or out of the caller's buffers
   const int rc_pipe = [&]() -> int {
-  int64_t u0 = 0;
-  for (int64_t idx = 0; idx < (int64_t)sched.size(); u0 += sched[idx], ++idx) {
-    const int b = (int)(idx & 1);
-    const int64_t nu = sched[idx];
-    // staging buffer b is free once the D2H (or compute) of chunk idx-2 finished
-    if (idx >= 2) {
-      TIC_CUDA(h, cudaStreamWaitEvent(h->s_h2d, inout_same ? h->ev_out[b] : h->ev_comp[b], 0));
+    cudaEvent_t consumed[2] = {};  // where chunk idx-2 was done with stage_in[b]
+    int64_t u0 = 0;
+    for (size_t idx = 0; idx < sched.size(); u0 += sched[idx++]) {
+      const int b = (int)(idx & 1);
+      const int64_t nu = sched[idx];
+      if (idx >= 2) TIC_CUDA(h, cudaStreamWaitEvent(h->s_h2d, in_place ? h->ev_out[b] : consumed[b], 0));
+      TIC_CUDA(h, cudaMemcpyAsync(h->stage_in[b].p, (const char*)in + (size_t)u0 * in_unit, (size_t)nu * in_unit,
+                                  cudaMemcpyHostToDevice, h->s_h2d));
+      TIC_CUDA(h, cudaEventRecord(h->ev_in[b], h->s_h2d));
+      TIC_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_in[b], 0));
+      if (idx >= 2 && copies && !in_place) TIC_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_out[b], 0));  // outputs copied
+      // copies the early outputs, or the others, back once the stream has passed `ready`
+      auto copy_back = [&](bool early, cudaEvent_t ready) -> int {
+        for (const Output& x : outs) {
+          if (!x.dst || x.early != early) continue;
+          TIC_CUDA(h, cudaStreamWaitEvent(h->s_d2h, ready, 0));
+          TIC_CUDA(h, cudaMemcpyAsync((char*)x.dst + (size_t)u0 * x.unit, x.stage[b].p, (size_t)nu * x.unit,
+                                      cudaMemcpyDeviceToHost, h->s_d2h));
+        }
+        return TIC_OK;
+      };
+      consumed[b] = nullptr;
+      Chunk c{h->stage_in[b].p, {o[0].stage ? o[0].stage[b].p : nullptr, o[1].stage ? o[1].stage[b].p : nullptr}, 0, u0, nu,
+              idx + 1 == sched.size(), [&]() -> int {
+                TIC_CUDA(h, cudaEventRecord(h->ev_enc[b], h->stream));
+                consumed[b] = h->ev_enc[b];
+                return copy_back(true, h->ev_enc[b]);
+              }};
+      if (int rc = run(c)) return rc;
+      TIC_CUDA(h, cudaEventRecord(h->ev_comp[b], h->stream));
+      if (!consumed[b]) {
+        consumed[b] = h->ev_comp[b];
+        if (int rc = copy_back(true, h->ev_comp[b])) return rc;
+      }
+      if (int rc = copy_back(false, h->ev_comp[b])) return rc;
+      if (copies) TIC_CUDA(h, cudaEventRecord(h->ev_out[b], h->s_d2h));
     }
-    TIC_CUDA(h, cudaMemcpyAsync(h->stage_in[b], (const char*)in + (size_t)u0 * in_unit_bytes, (size_t)nu * in_unit_bytes,
-                                cudaMemcpyHostToDevice, h->s_h2d));
-    TIC_CUDA(h, cudaEventRecord(h->ev_in[b], h->s_h2d));
-    TIC_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_in[b], 0));
-    if (idx >= 2 && !inout_same) TIC_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_out[b], 0));
-    void* dout = inout_same ? h->stage_in[b] : h->stage_out[b];
-    int rc = run(h->stage_in[b], dout, 0, nu, /*local=*/true);
-    if (rc != TIC_OK) return rc;
-    TIC_CUDA(h, cudaEventRecord(h->ev_comp[b], h->stream));
-    TIC_CUDA(h, cudaStreamWaitEvent(h->s_d2h, h->ev_comp[b], 0));
-    TIC_CUDA(h, cudaMemcpyAsync((char*)out + (size_t)u0 * out_unit_bytes, dout, (size_t)nu * out_unit_bytes,
-                                cudaMemcpyDeviceToHost, h->s_d2h));
-    TIC_CUDA(h, cudaEventRecord(h->ev_out[b], h->s_d2h));
-  }
-  TIC_CUDA(h, cudaEventRecord(h->ev_t1, h->stream));
-  TIC_CUDA(h, cudaStreamSynchronize(h->s_d2h));
-  TIC_CUDA(h, cudaStreamSynchronize(h->stream));
-  return TIC_OK;
+    TIC_CUDA(h, cudaEventRecord(h->ev_t1, h->stream));
+    TIC_CUDA(h, cudaStreamSynchronize(h->s_d2h));
+    TIC_CUDA(h, cudaStreamSynchronize(h->stream));
+    return TIC_OK;
   }();
   if (rc_pipe != TIC_OK) {
-    quiesce(h);
+    cudaStreamSynchronize(h->s_h2d);
+    cudaStreamSynchronize(h->stream);
+    cudaStreamSynchronize(h->s_d2h);
     return rc_pipe;
   }
   return overflow_status(h);
@@ -668,6 +717,56 @@ Geo image_geo(int H, int W, int P, long long n0) {
   g.n0 = n0;
   geo_finish(g);
   return g;
+}
+
+// What an image call needs to know about its graphs: the symbol map of one P x P patch (hb x wb x cb) and the patches
+// per H x W image.
+struct ImageShapes {
+  int hb, wb, cb, ppi;
+};
+
+// The checks every image call makes.  `enc` / `dec`: the call runs the encoder / the decoder graph.
+int image_shapes(tic_codec* h, int H, int W, int P, bool enc, bool dec, ImageShapes* s) {
+  if (enc && ((H % P != 0 && H < 2) || (W % P != 0 && W < 2)))
+    return fail(h, TIC_ERR_INVALID, "reflect padding needs at least 2 pixels");
+  if (enc)
+    if (int rc = check_graph_ready(h, TIC_GRAPH_ENCODER, true)) return rc;
+  if (dec)
+    if (int rc = check_graph_ready(h, TIC_GRAPH_DECODER, true)) return rc;
+  if (h->q < 2) return fail(h, TIC_ERR_STATE, "quantiser not configured (tic_set_quantizer)");
+  const Graph& gd = h->g[TIC_GRAPH_DECODER];
+  Shape so;
+  if (enc) {
+    if (h->g[TIC_GRAPH_ENCODER].layers[0].d.cin != 3) return fail(h, TIC_ERR_INVALID, "encoder must take 3 channels");
+    if (int rc = tic_bottleneck_shape(h, P, &s->hb, &s->wb, &s->cb)) return rc;
+    if (dec && (gd.layers[0].d.cin != s->cb || graph_out_shape(gd, Shape{s->hb, s->wb, s->cb}, &so) != 0 || so.c != 3 ||
+                so.h != P || so.w != P))
+      return fail(h, TIC_ERR_INVALID, "decoder graph does not map the encoder's %dx%dx%d symbols back to %dx%d RGB", s->hb, s->wb,
+                  s->cb, P, P);
+  } else {
+    // bottleneck map size for patch size P: invert the decoder's upsampling
+    int up = 1;
+    for (auto& l : gd.layers)
+      if (l.d.kind == TIC_DECONV) up *= 2;
+    if (P % up != 0) return fail(h, TIC_ERR_INVALID, "patch size %d is not a multiple of the decoder upsampling %d", P, up);
+    s->hb = s->wb = P / up;
+    s->cb = gd.layers[0].d.cin;
+    if (graph_out_shape(gd, Shape{s->hb, s->wb, s->cb}, &so) != 0 || so.c != 3 || so.h != P)
+      return fail(h, TIC_ERR_INVALID, "decoder graph does not map %dx%d symbols to %dx%d RGB", s->hb, s->wb, P, P);
+  }
+  const Geo g0 = image_geo(H, W, P, 0);
+  s->ppi = g0.gh * g0.gw;
+  return TIC_OK;
+}
+
+// Frees a graph's weights and operand images.
+void free_layers(Graph& g) {
+  for (auto& l : g.layers) {
+    cudaFree(l.w);
+    cudaFree(l.b);
+    l.release();
+  }
+  g.layers.clear();
 }
 
 }  // namespace
@@ -718,7 +817,6 @@ int tic_create(tic_codec** out, int device) {
     cudaEventCreateWithFlags(&h->ev_out[b], cudaEventDisableTiming);
     cudaEventCreateWithFlags(&h->ev_enc[b], cudaEventDisableTiming);
   }
-  cudaEventCreate(&h->ev_rt);
   cudaEventCreate(&h->ev_t0);
   cudaEventCreate(&h->ev_t1);
   if ((e = cudaMalloc(&h->d_hist, 256 * sizeof(unsigned long long))) != cudaSuccess) return bail("cudaMalloc", e);
@@ -739,39 +837,22 @@ void tic_destroy(tic_codec* h) {
   if (!h) return;
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();
-  for (int gi = 0; gi < 3; ++gi) {
-    for (auto& l : h->g[gi].layers) {
-      if (l.w) cudaFree(l.w);
-      if (l.b) cudaFree(l.b);
-      l.uw.release();
-      l.uw16.release();
-      l.fw16.release();
-      l.fdw.release();
-      l.few.release();
-    }
-    if (h->g[gi].d_normlut) cudaFree(h->g[gi].d_normlut);
+  for (Graph& g : h->g) {
+    free_layers(g);
+    if (g.d_normlut) cudaFree(g.d_normlut);
   }
-  for (int i = 0; i < 3; ++i)
-    if (h->act[i]) cudaFree(h->act[i]);
   for (int b = 0; b < 2; ++b) {
-    if (h->stage_in[b]) cudaFree(h->stage_in[b]);
-    if (h->stage_out[b]) cudaFree(h->stage_out[b]);
-    if (h->stage_sym[b]) cudaFree(h->stage_sym[b]);
     cudaEventDestroy(h->ev_enc[b]);
     cudaEventDestroy(h->ev_in[b]);
     cudaEventDestroy(h->ev_comp[b]);
     cudaEventDestroy(h->ev_out[b]);
   }
-  cudaEventDestroy(h->ev_rt);
   cudaEventDestroy(h->ev_t0);
   cudaEventDestroy(h->ev_t1);
   if (h->d_hist) cudaFree(h->d_hist);
   if (h->d_symlut) cudaFree(h->d_symlut);
   if (h->h_oflow) cudaFreeHost(h->h_oflow);
   if (h->d_cum) cudaFree(h->d_cum);
-  if (h->d_seg) cudaFree(h->d_seg);
-  if (h->d_seg_bytes) cudaFree(h->d_seg_bytes);
-  if (h->d_eval) cudaFree(h->d_eval);
   if (h->ev_switch) cudaEventDestroy(h->ev_switch);
   if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
   if (h->s_h2d) cudaStreamDestroy(h->s_h2d);
@@ -847,16 +928,8 @@ int tic_set_graph(tic_codec* h, int graph, const tic_layer_desc* layers, int n_l
     prev = d.cout;
   }
   Graph& g = h->g[graph];
-  for (auto& l : g.layers) {
-    if (l.w) cudaFree(l.w);
-    if (l.b) cudaFree(l.b);
-    l.uw.release();
-    l.uw16.release();
-    l.fw16.release();
-    l.fdw.release();
-    l.few.release();
-  }
-  g.layers.assign(n_layers, Layer());
+  free_layers(g);
+  g.layers.resize(n_layers);
   for (int i = 0; i < n_layers; ++i) {
     Layer& l = g.layers[i];
     l.d = layers[i];
@@ -888,11 +961,7 @@ int tic_load_weights(tic_codec* h, int graph, int layer, const float* kernel, co
   TIC_CUDA(h, cudaMemcpy(l.w, w.data(), w.size() * sizeof(float), cudaMemcpyHostToDevice));
   TIC_CUDA(h, cudaMemcpy(l.b, bias, (size_t)cout * sizeof(float), cudaMemcpyHostToDevice));
   l.hb.assign(bias, bias + cout);
-  l.uw.release();
-  l.uw16.release();
-  l.fw16.release();
-  l.fdw.release();
-  l.few.release();
+  l.release();
   if (layer > 0) {  // the fused pair kernels keep this layer's operand image with the previous layer
     g.layers[layer - 1].fdw.release();
     g.layers[layer - 1].few.release();
@@ -950,25 +1019,20 @@ int tic_encode_patches(tic_codec* h, const void* patches, int in_dtype, int64_t 
   if (n < 0 || P <= 0 || (n > 0 && (!patches || !symbols))) return fail(h, TIC_ERR_INVALID, "bad arguments");
   if (in_dtype != TIC_U8 && in_dtype != TIC_F32) return fail(h, TIC_ERR_INVALID, "bad in_dtype");
   if (out_dtype != TIC_U8 && out_dtype != TIC_F32) return fail(h, TIC_ERR_INVALID, "bad out_dtype");
-  int rc = check_graph_ready(h, TIC_GRAPH_ENCODER, true);
-  if (rc != TIC_OK) return rc;
-  if (h->q < 2) return fail(h, TIC_ERR_STATE, "quantiser not configured (tic_set_quantizer)");
-  if (h->g[TIC_GRAPH_ENCODER].layers[0].d.cin != 3) return fail(h, TIC_ERR_INVALID, "encoder must take 3 channels");
-  int hb, wb, cb;
-  rc = tic_bottleneck_shape(h, P, &hb, &wb, &cb);
-  if (rc != TIC_OK) return rc;
+  ImageShapes s;
+  if (int rc = image_shapes(h, P, P, P, true, false, &s)) return rc;  // a patch is a P x P image
   const size_t in_unit = (size_t)P * P * 3 * (in_dtype == TIC_U8 ? 1 : 4);
-  const size_t out_unit = (size_t)hb * wb * cb * (out_dtype == TIC_U8 ? 1 : 4);
-  return drive(h, mem, patches, symbols, n, patches_per_chunk(h, P), in_unit, out_unit, false,
-               [&](const void* din, void* dout, int64_t u0, int64_t nu, bool) {
+  const size_t out_unit = (size_t)s.hb * s.wb * s.cb * (out_dtype == TIC_U8 ? 1 : 4);
+  return drive(h, mem, patches, in_unit, {{symbols, out_unit, h->stage_out, false}}, n, patches_per_chunk(h, P),
+               [&](Chunk& c) {
                  IoSpec i, o;
                  i.mode = in_dtype == TIC_U8 ? IO_U8_NORM : IO_F32_NORM;
-                 i.in = din;
-                 i.geo = patch_geo(P, u0);
+                 i.in = c.in;
+                 i.geo = patch_geo(P, c.off);
                  o.mode = out_dtype == TIC_U8 ? IO_QUANT_U8 : IO_QUANT_F32;
-                 o.out = dout;
-                 o.geo = patch_geo(P, u0);
-                 return run_graph(h, TIC_GRAPH_ENCODER, i, o, (int)nu, P, P);
+                 o.out = c.out[0];
+                 o.geo = patch_geo(P, c.off);
+                 return run_graph(h, TIC_GRAPH_ENCODER, i, o, (int)c.nu, P, P);
                }, (double)P * P / 16384.0);
 }
 
@@ -977,29 +1041,22 @@ int tic_encode_images(tic_codec* h, const uint8_t* images, int64_t n_images, int
   if (!h) return TIC_ERR_INVALID;
   if (n_images < 0 || H <= 0 || W <= 0 || P <= 0 || (n_images > 0 && (!images || !symbols)))
     return fail(h, TIC_ERR_INVALID, "bad arguments");
-  if ((H % P != 0 && H < 2) || (W % P != 0 && W < 2)) return fail(h, TIC_ERR_INVALID, "reflect padding needs at least 2 pixels");
-  int rc = check_graph_ready(h, TIC_GRAPH_ENCODER, true);
-  if (rc != TIC_OK) return rc;
-  if (h->q < 2) return fail(h, TIC_ERR_STATE, "quantiser not configured (tic_set_quantizer)");
-  if (h->g[TIC_GRAPH_ENCODER].layers[0].d.cin != 3) return fail(h, TIC_ERR_INVALID, "encoder must take 3 channels");
-  int hb, wb, cb;
-  rc = tic_bottleneck_shape(h, P, &hb, &wb, &cb);
-  if (rc != TIC_OK) return rc;
-  const Geo g0 = image_geo(H, W, P, 0);
-  const int ppi = g0.gh * g0.gw;
+  ImageShapes s;
+  if (int rc = image_shapes(h, H, W, P, true, false, &s)) return rc;
+  const int ppi = s.ppi;
   const int64_t ipc = std::max<int64_t>(1, patches_per_chunk(h, P) / ppi);
   const size_t in_unit = (size_t)H * W * 3;
-  const size_t out_unit = (size_t)ppi * hb * wb * cb;
-  return drive(h, mem, images, symbols, n_images, ipc, in_unit, out_unit, false,
-               [&](const void* din, void* dout, int64_t u0, int64_t nu, bool) {
+  const size_t out_unit = (size_t)ppi * s.hb * s.wb * s.cb;
+  return drive(h, mem, images, in_unit, {{symbols, out_unit, h->stage_out, false}}, n_images, ipc,
+               [&](Chunk& c) {
                  IoSpec i, o;
                  i.mode = IO_U8_NORM;
-                 i.in = din;
-                 i.geo = image_geo(H, W, P, u0 * ppi);
+                 i.in = c.in;
+                 i.geo = image_geo(H, W, P, c.off * ppi);
                  o.mode = IO_QUANT_U8;
-                 o.out = dout;
+                 o.out = c.out[0];
                  o.geo = i.geo;
-                 return run_graph(h, TIC_GRAPH_ENCODER, i, o, (int)(nu * ppi), P, P);
+                 return run_graph(h, TIC_GRAPH_ENCODER, i, o, (int)(c.nu * ppi), P, P);
                }, (double)ppi * P * P / 16384.0);
 }
 
@@ -1015,16 +1072,17 @@ int tic_decode_patches(tic_codec* h, const uint8_t* symbols, int64_t n, int hb, 
   if (graph_out_shape(g, Shape{hb, wb, cb}, &so) != 0) return fail(h, TIC_ERR_INVALID, "inconsistent graph");
   if (so.c != 3 || so.h != so.w) return fail(h, TIC_ERR_INVALID, "decoder must produce square RGB patches (got %dx%dx%d)", so.h, so.w, so.c);
   const int P = so.h;
-  return drive(h, mem, symbols, recon, n, patches_per_chunk(h, P), (size_t)hb * wb * cb, (size_t)P * P * 3 * 4, false,
-               [&](const void* din, void* dout, int64_t u0, int64_t nu, bool) {
+  return drive(h, mem, symbols, (size_t)hb * wb * cb, {{recon, (size_t)P * P * 3 * 4, h->stage_out, false}}, n,
+               patches_per_chunk(h, P),
+               [&](Chunk& c) {
                  IoSpec i, o;
                  i.mode = IO_U8_SYMLUT;
-                 i.in = din;
-                 i.geo = patch_geo(P, u0);
+                 i.in = c.in;
+                 i.geo = patch_geo(P, c.off);
                  o.mode = IO_DENORM_F32;
-                 o.out = dout;
-                 o.geo = patch_geo(P, u0);
-                 return run_graph(h, TIC_GRAPH_DECODER, i, o, (int)nu, hb, wb);
+                 o.out = c.out[0];
+                 o.geo = patch_geo(P, c.off);
+                 return run_graph(h, TIC_GRAPH_DECODER, i, o, (int)c.nu, hb, wb);
                }, (double)P * P / 16384.0);
 }
 
@@ -1034,35 +1092,22 @@ int tic_decode_images(tic_codec* h, const uint8_t* symbols, int64_t n_images, in
   if (n_images < 0 || H <= 0 || W <= 0 || P <= 0 || (n_images > 0 && (!symbols || !images)))
     return fail(h, TIC_ERR_INVALID, "bad arguments");
   if (out_dtype != TIC_U8 && out_dtype != TIC_F32) return fail(h, TIC_ERR_INVALID, "bad out_dtype");
-  int rc = check_graph_ready(h, TIC_GRAPH_DECODER, true);
-  if (rc != TIC_OK) return rc;
-  if (h->q < 2) return fail(h, TIC_ERR_STATE, "quantiser not configured (tic_set_quantizer)");
-  Graph& g = h->g[TIC_GRAPH_DECODER];
-  const int cb = g.layers[0].d.cin;
-  // bottleneck map size for patch size P: invert the decoder's upsampling
-  int up = 1;
-  for (auto& l : g.layers)
-    if (l.d.kind == TIC_DECONV) up *= 2;
-  if (P % up != 0) return fail(h, TIC_ERR_INVALID, "patch size %d is not a multiple of the decoder upsampling %d", P, up);
-  const int hb = P / up, wb = P / up;
-  Shape so;
-  if (graph_out_shape(g, Shape{hb, wb, cb}, &so) != 0 || so.c != 3 || so.h != P)
-    return fail(h, TIC_ERR_INVALID, "decoder graph does not map %dx%d symbols to %dx%d RGB", hb, wb, P, P);
-  const Geo g0 = image_geo(H, W, P, 0);
-  const int ppi = g0.gh * g0.gw;
+  ImageShapes s;
+  if (int rc = image_shapes(h, H, W, P, false, true, &s)) return rc;
+  const int ppi = s.ppi;
   const int64_t ipc = std::max<int64_t>(1, patches_per_chunk(h, P) / ppi);
-  const size_t in_unit = (size_t)ppi * hb * wb * cb;
+  const size_t in_unit = (size_t)ppi * s.hb * s.wb * s.cb;
   const size_t out_unit = (size_t)H * W * 3 * (out_dtype == TIC_U8 ? 1 : 4);
-  return drive(h, mem, symbols, images, n_images, ipc, in_unit, out_unit, false,
-               [&](const void* din, void* dout, int64_t u0, int64_t nu, bool) {
+  return drive(h, mem, symbols, in_unit, {{images, out_unit, h->stage_out, false}}, n_images, ipc,
+               [&](Chunk& c) {
                  IoSpec i, o;
                  i.mode = IO_U8_SYMLUT;
-                 i.in = din;
-                 i.geo = image_geo(H, W, P, u0 * ppi);
+                 i.in = c.in;
+                 i.geo = image_geo(H, W, P, c.off * ppi);
                  o.mode = out_dtype == TIC_U8 ? IO_DENORM_U8 : IO_DENORM_F32;
-                 o.out = dout;
+                 o.out = c.out[0];
                  o.geo = i.geo;
-                 return run_graph(h, TIC_GRAPH_DECODER, i, o, (int)(nu * ppi), hb, wb);
+                 return run_graph(h, TIC_GRAPH_DECODER, i, o, (int)(c.nu * ppi), s.hb, s.wb);
                }, (double)ppi * P * P / 16384.0);
 }
 
@@ -1072,99 +1117,37 @@ int tic_roundtrip_images(tic_codec* h, const uint8_t* images, int64_t n_images, 
   if (n_images < 0 || H <= 0 || W <= 0 || P <= 0 || (n_images > 0 && (!images || !recon)))
     return fail(h, TIC_ERR_INVALID, "bad arguments");
   if (out_dtype != TIC_U8 && out_dtype != TIC_F32) return fail(h, TIC_ERR_INVALID, "bad out_dtype");
-  if (mem == TIC_MEM_DEVICE) {
-    if (!symbols && n_images > 0) return fail(h, TIC_ERR_INVALID, "device-resident round trips need a symbol buffer");
-    int rc = tic_encode_images(h, images, n_images, H, W, P, symbols, mem);
-    if (rc != TIC_OK) return rc;
-    cudaEvent_t t0 = h->ev_t0;  // keep the encoder's start event: last_kernel_ms covers both graphs
-    h->ev_t0 = h->ev_rt;
-    rc = tic_decode_images(h, symbols, n_images, H, W, P, recon, out_dtype, mem);
-    h->ev_rt = h->ev_t0;
-    h->ev_t0 = t0;
-    return rc;
-  }
-  if ((H % P != 0 && H < 2) || (W % P != 0 && W < 2)) return fail(h, TIC_ERR_INVALID, "reflect padding needs at least 2 pixels");
-  int rc = check_graph_ready(h, TIC_GRAPH_ENCODER, true);
-  if (rc != TIC_OK) return rc;
-  rc = check_graph_ready(h, TIC_GRAPH_DECODER, true);
-  if (rc != TIC_OK) return rc;
-  if (h->q < 2) return fail(h, TIC_ERR_STATE, "quantiser not configured (tic_set_quantizer)");
-  if (h->g[TIC_GRAPH_ENCODER].layers[0].d.cin != 3) return fail(h, TIC_ERR_INVALID, "encoder must take 3 channels");
-  int hb, wb, cb;
-  rc = tic_bottleneck_shape(h, P, &hb, &wb, &cb);
-  if (rc != TIC_OK) return rc;
-  Graph& gd = h->g[TIC_GRAPH_DECODER];
-  Shape so;
-  if (gd.layers[0].d.cin != cb || graph_out_shape(gd, Shape{hb, wb, cb}, &so) != 0 || so.c != 3 || so.h != P || so.w != P)
-    return fail(h, TIC_ERR_INVALID, "decoder graph does not map the encoder's %dx%dx%d symbols back to %dx%d RGB", hb, wb, cb, P, P);
-  if (n_images == 0) return TIC_OK;
-  TIC_CUDA(h, cudaSetDevice(h->device));
-  const Geo g0 = image_geo(H, W, P, 0);
-  const int ppi = g0.gh * g0.gw;
-  const std::vector<int64_t> sched =
-      host_chunk_schedule(n_images, std::max<int64_t>(1, patches_per_chunk(h, P) / ppi), (double)ppi * P * P / 16384.0);
-  const int64_t ipc = *std::max_element(sched.begin(), sched.end());
-  const size_t img_unit = (size_t)H * W * 3;
-  const size_t sym_unit = (size_t)ppi * hb * wb * cb;
-  const size_t rec_unit = img_unit * (out_dtype == TIC_U8 ? 1 : 4);
-  if ((rc = grow_pair(h, h->stage_in, &h->stage_in_bytes, (size_t)ipc * img_unit)) != TIC_OK) return rc;
-  if ((rc = grow_pair(h, h->stage_sym, &h->stage_sym_bytes, (size_t)ipc * sym_unit)) != TIC_OK) return rc;
-  if ((rc = grow_pair(h, h->stage_out, &h->stage_out_bytes, (size_t)ipc * rec_unit)) != TIC_OK) return rc;
-  // Three streams, two staging sets: H2D of chunk i+1 (one PCIe direction) runs under the kernels of chunk i and
-  // the D2H of chunk i-1 (the other direction).
-  if (int st = overflow_status(h)) return st;
-  const int rc_pipe = [&]() -> int {  // any failure drains the three streams before returning (see drive())
-  TIC_CUDA(h, cudaEventRecord(h->ev_t0, h->stream));
-  int64_t u0 = 0;
-  for (int64_t idx = 0; idx < (int64_t)sched.size(); u0 += sched[idx], ++idx) {
-    const int b = (int)(idx & 1);
-    const int64_t nu = sched[idx];
-    if (idx >= 2) TIC_CUDA(h, cudaStreamWaitEvent(h->s_h2d, h->ev_enc[b], 0));  // encoder of chunk idx-2 consumed stage_in[b]
-    TIC_CUDA(h, cudaMemcpyAsync(h->stage_in[b], images + (size_t)u0 * img_unit, (size_t)nu * img_unit, cudaMemcpyHostToDevice,
-                                h->s_h2d));
-    TIC_CUDA(h, cudaEventRecord(h->ev_in[b], h->s_h2d));
-    TIC_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_in[b], 0));
-    if (idx >= 2) TIC_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_out[b], 0));  // stage_sym / stage_out[b] drained
-    IoSpec i, o;
-    i.mode = IO_U8_NORM;
-    i.in = h->stage_in[b];
-    i.geo = image_geo(H, W, P, 0);
-    o.mode = IO_QUANT_U8;
-    o.out = h->stage_sym[b];
-    o.geo = i.geo;
-    rc = run_graph(h, TIC_GRAPH_ENCODER, i, o, (int)(nu * ppi), P, P);
-    if (rc != TIC_OK) return rc;
-    TIC_CUDA(h, cudaEventRecord(h->ev_enc[b], h->stream));
-    IoSpec di, dout;
-    di.mode = IO_U8_SYMLUT;
-    di.in = h->stage_sym[b];
-    di.geo = i.geo;
-    dout.mode = out_dtype == TIC_U8 ? IO_DENORM_U8 : IO_DENORM_F32;
-    dout.out = h->stage_out[b];
-    dout.geo = i.geo;
-    rc = run_graph(h, TIC_GRAPH_DECODER, di, dout, (int)(nu * ppi), hb, wb);
-    if (rc != TIC_OK) return rc;
-    TIC_CUDA(h, cudaEventRecord(h->ev_comp[b], h->stream));
-    if (symbols) {
-      TIC_CUDA(h, cudaStreamWaitEvent(h->s_d2h, h->ev_enc[b], 0));
-      TIC_CUDA(h, cudaMemcpyAsync(symbols + (size_t)u0 * sym_unit, h->stage_sym[b], (size_t)nu * sym_unit, cudaMemcpyDeviceToHost,
-                                  h->s_d2h));
-    }
-    TIC_CUDA(h, cudaStreamWaitEvent(h->s_d2h, h->ev_comp[b], 0));
-    TIC_CUDA(h, cudaMemcpyAsync((char*)recon + (size_t)u0 * rec_unit, h->stage_out[b], (size_t)nu * rec_unit, cudaMemcpyDeviceToHost,
-                                h->s_d2h));
-    TIC_CUDA(h, cudaEventRecord(h->ev_out[b], h->s_d2h));
-  }
-  TIC_CUDA(h, cudaEventRecord(h->ev_t1, h->stream));
-  TIC_CUDA(h, cudaStreamSynchronize(h->s_d2h));
-  TIC_CUDA(h, cudaStreamSynchronize(h->stream));
-  return TIC_OK;
-  }();
-  if (rc_pipe != TIC_OK) {
-    quiesce(h);
-    return rc_pipe;
-  }
-  return overflow_status(h);
+  if (mem == TIC_MEM_DEVICE && !symbols && n_images > 0)
+    return fail(h, TIC_ERR_INVALID, "device-resident round trips need a symbol buffer");
+  ImageShapes s;
+  if (int rc = image_shapes(h, H, W, P, true, true, &s)) return rc;
+  const int ppi = s.ppi;
+  const int64_t ipc = std::max<int64_t>(1, patches_per_chunk(h, P) / ppi);
+  const size_t sym_unit = (size_t)ppi * s.hb * s.wb * s.cb;
+  const size_t rec_unit = (size_t)H * W * 3 * (out_dtype == TIC_U8 ? 1 : 4);
+  // Per chunk: encoder -> symbols -> decoder.  With host buffers the next chunk's images may overwrite this one's once
+  // the encoder has read them, and the symbols go back while the decoder runs.
+  return drive(h, mem, images, (size_t)H * W * 3, {{symbols, sym_unit, h->stage_sym, true}, {recon, rec_unit, h->stage_out, false}},
+               n_images, ipc,
+               [&](Chunk& c) {
+                 IoSpec i, o;
+                 i.mode = IO_U8_NORM;
+                 i.in = c.in;
+                 i.geo = image_geo(H, W, P, c.off * ppi);
+                 o.mode = IO_QUANT_U8;
+                 o.out = c.out[0];
+                 o.geo = i.geo;
+                 if (int rc = run_graph(h, TIC_GRAPH_ENCODER, i, o, (int)(c.nu * ppi), P, P)) return rc;
+                 if (int rc = mark_consumed(c)) return rc;
+                 IoSpec di, dout;
+                 di.mode = IO_U8_SYMLUT;
+                 di.in = c.out[0];
+                 di.geo = i.geo;
+                 dout.mode = out_dtype == TIC_U8 ? IO_DENORM_U8 : IO_DENORM_F32;
+                 dout.out = c.out[1];
+                 dout.geo = i.geo;
+                 return run_graph(h, TIC_GRAPH_DECODER, di, dout, (int)(c.nu * ppi), s.hb, s.wb);
+               }, (double)ppi * P * P / 16384.0);
 }
 
 int tic_postfilter_patches(tic_codec* h, const float* tiles, int64_t n, int P, float* out, int mem) {
@@ -1177,16 +1160,16 @@ int tic_postfilter_patches(tic_codec* h, const float* tiles, int64_t n, int P, f
   if (g.layers[0].d.cin != 3 || graph_out_shape(g, Shape{P, P, 3}, &so) != 0 || so.c != 3 || so.h != P || so.w != P)
     return fail(h, TIC_ERR_INVALID, "post-filter graph must map PxPx3 to PxPx3");
   const size_t unit = (size_t)P * P * 3 * 4;
-  return drive(h, mem, tiles, out, n, patches_per_chunk(h, P), unit, unit, false,
-               [&](const void* din, void* dout, int64_t u0, int64_t nu, bool) {
+  return drive(h, mem, tiles, unit, {{out, unit, h->stage_out, false}}, n, patches_per_chunk(h, P),
+               [&](Chunk& c) {
                  IoSpec i, o;
                  i.mode = IO_F32_NORM;
-                 i.in = din;
-                 i.geo = patch_geo(P, u0);
+                 i.in = c.in;
+                 i.geo = patch_geo(P, c.off);
                  o.mode = IO_DENORM_F32;
-                 o.out = dout;
-                 o.geo = patch_geo(P, u0);
-                 return run_graph(h, TIC_GRAPH_POSTFILTER, i, o, (int)nu, P, P);
+                 o.out = c.out[0];
+                 o.geo = patch_geo(P, c.off);
+                 return run_graph(h, TIC_GRAPH_POSTFILTER, i, o, (int)c.nu, P, P);
                });
 }
 
@@ -1204,9 +1187,8 @@ int tic_postfilter_images(tic_codec* h, float* images, int64_t n_images, int H, 
   // tiles per image of the two passes; whole images per chunk so that pass 2 reads pass-1 output
   const int t1 = (H / P) * ((W - off) / P), t2 = ((H - off) / P) * (W / P);
   const int64_t ipc = std::max<int64_t>(1, patches_per_chunk(h, P) / std::max(1, std::max(t1, t2)));
-  return drive(h, mem, images, images, n_images, ipc, unit, unit, true,
-               [&](const void* din, void* dout, int64_t u0, int64_t nu, bool) {
-                 (void)din;
+  return drive(h, mem, images, unit, {{images, unit, h->stage_in, false}}, n_images, ipc,
+               [&](Chunk& c) {
                  for (int pass = 0; pass < 2; ++pass) {
                    Geo gg{};
                    gg.H = H;
@@ -1225,16 +1207,16 @@ int tic_postfilter_images(tic_codec* h, float* images, int64_t n_images, int H, 
                    }
                    const int tiles = gg.gh * gg.gw;
                    if (tiles <= 0) continue;
-                   gg.n0 = u0 * tiles;
+                   gg.n0 = c.off * tiles;
                    geo_finish(gg);
                    IoSpec i, o;
                    i.mode = IO_F32_NORM;
-                   i.in = dout;  // in place: pass 2 reads what pass 1 wrote
+                   i.in = c.out[0];  // in place: pass 2 reads what pass 1 wrote
                    i.geo = gg;
                    o.mode = IO_DENORM_F32;
-                   o.out = dout;
+                   o.out = c.out[0];
                    o.geo = gg;
-                   int r2 = run_graph(h, TIC_GRAPH_POSTFILTER, i, o, (int)(nu * tiles), P, P);
+                   int r2 = run_graph(h, TIC_GRAPH_POSTFILTER, i, o, (int)(c.nu * tiles), P, P);
                    if (r2 != TIC_OK) return r2;
                  }
                  return (int)TIC_OK;
@@ -1256,26 +1238,25 @@ int tic_run_layers(tic_codec* h, int graph, const float* in, int64_t n, int h0, 
   if (graph_out_shape(g, Shape{h0, w0, cin}, &so, n_layers) != 0) return fail(h, TIC_ERR_INVALID, "inconsistent graph");
   const size_t in_unit = (size_t)h0 * w0 * cin * 4, out_unit = (size_t)so.h * so.w * so.c * 4;
   const int64_t upc = std::max<int64_t>(1, (int64_t)h->chunk128 * 128 * 128 / ((int64_t)std::max(h0 * w0, so.h * so.w)));
-  return drive(h, mem, in, out, n, upc, in_unit, out_unit, false,
-               [&](const void* din, void* dout, int64_t u0, int64_t nu, bool) {
-                 IoSpec i, o;
-                 i.mode = IO_ACT;
-                 i.in = (const char*)din + (size_t)u0 * in_unit;
-                 o.mode = IO_ACT;
-                 o.out = (char*)dout + (size_t)u0 * out_unit;
-                 return run_graph(h, graph, i, o, (int)nu, h0, w0, n_layers);
-               });
+  return drive(h, mem, in, in_unit, {{out, out_unit, h->stage_out, false}}, n, upc, [&](Chunk& c) {
+    IoSpec i, o;
+    i.mode = IO_ACT;
+    i.in = (const char*)c.in + (size_t)c.off * in_unit;
+    o.mode = IO_ACT;
+    o.out = (char*)c.out[0] + (size_t)c.off * out_unit;
+    return run_graph(h, graph, i, o, (int)c.nu, h0, w0, n_layers);
+  });
 }
 
 int tic_round_u8(tic_codec* h, const float* src, uint8_t* dst, int64_t count, int mem) {
   if (!h) return TIC_ERR_INVALID;
   if (count < 0 || (count > 0 && (!src || !dst))) return fail(h, TIC_ERR_INVALID, "bad arguments");
   const int64_t upc = 1 << 26;
-  return drive(h, mem, src, dst, count, upc, 4, 1, false, [&](const void* din, void* dout, int64_t u0, int64_t nu, bool) {
-    const float* s = (const float*)din + u0;
-    uint8_t* d = (uint8_t*)dout + u0;
-    int blocks = (int)std::min<int64_t>((nu + 255) / 256, (int64_t)h->num_sms * 16);
-    round_u8_kernel<<<blocks, 256, 0, h->stream>>>(s, d, nu);
+  return drive(h, mem, src, 4, {{dst, 1, h->stage_out, false}}, count, upc, [&](Chunk& c) {
+    const float* s = (const float*)c.in + c.off;
+    uint8_t* d = (uint8_t*)c.out[0] + c.off;
+    int blocks = (int)std::min<int64_t>((c.nu + 255) / 256, (int64_t)h->num_sms * 16);
+    round_u8_kernel<<<blocks, 256, 0, h->stream>>>(s, d, c.nu);
     h->launches++;
     TIC_CUDA(h, cudaGetLastError());
     return (int)TIC_OK;
@@ -1311,23 +1292,22 @@ int tic_position_sums(tic_codec* h, const uint8_t* symbols, int64_t n, int64_t n
   TIC_CUDA(h, cudaSetDevice(h->device));
   const uint8_t* dsym = symbols;
   unsigned long long* dsum = (unsigned long long*)sums;
-  void *tmp_sym = nullptr, *tmp_sum = nullptr;
+  CallTemps t{h};
   if (mem == TIC_MEM_HOST) {
-    TIC_CUDA(h, cudaMalloc(&tmp_sym, (size_t)std::max<int64_t>(1, n * npos)));
-    TIC_CUDA(h, cudaMalloc(&tmp_sum, (size_t)npos * 8));
-    TIC_CUDA(h, cudaMemcpyAsync(tmp_sym, symbols, (size_t)(n * npos), cudaMemcpyHostToDevice, h->stream));
-    TIC_CUDA(h, cudaMemcpyAsync(tmp_sum, sums, (size_t)npos * 8, cudaMemcpyHostToDevice, h->stream));
-    dsym = (const uint8_t*)tmp_sym;
-    dsum = (unsigned long long*)tmp_sum;
+    int rc = grow(h, &t.buf[0], 1, (size_t)std::max<int64_t>(1, n * npos));
+    if (rc == TIC_OK) rc = grow(h, &t.buf[1], 1, (size_t)npos * 8);
+    if (rc != TIC_OK) return rc;
+    dsym = t.buf[0].as<uint8_t>();
+    dsum = t.buf[1].as<unsigned long long>();
+    TIC_CUDA(h, cudaMemcpyAsync(t.buf[0].p, symbols, (size_t)(n * npos), cudaMemcpyHostToDevice, h->stream));
+    TIC_CUDA(h, cudaMemcpyAsync(dsum, sums, (size_t)npos * 8, cudaMemcpyHostToDevice, h->stream));
   }
   position_sums_kernel<<<(unsigned)((npos + 255) / 256), 256, 0, h->stream>>>(dsym, n, npos, dsum);
   h->launches++;
   TIC_CUDA(h, cudaGetLastError());
   if (mem == TIC_MEM_HOST) {
-    TIC_CUDA(h, cudaMemcpyAsync(sums, tmp_sum, (size_t)npos * 8, cudaMemcpyDeviceToHost, h->stream));
+    TIC_CUDA(h, cudaMemcpyAsync(sums, dsum, (size_t)npos * 8, cudaMemcpyDeviceToHost, h->stream));
     TIC_CUDA(h, cudaStreamSynchronize(h->stream));
-    cudaFree(tmp_sym);
-    cudaFree(tmp_sum);
   }
   return TIC_OK;
 }
@@ -1342,24 +1322,21 @@ int tic_position_sums_batched(tic_codec* h, const uint8_t* symbols, int64_t n, i
   TIC_CUDA(h, cudaSetDevice(h->device));
   const uint8_t* dsym = symbols;
   unsigned long long* dsum = (unsigned long long*)sums;
-  void *tmp_sym = nullptr, *tmp_sum = nullptr;
+  CallTemps t{h};
   if (mem == TIC_MEM_HOST) {
-    TIC_CUDA(h, cudaMalloc(&tmp_sym, (size_t)(n * npos)));
-    TIC_CUDA(h, cudaMalloc(&tmp_sum, (size_t)(nb * npos) * 8));
-    TIC_CUDA(h, cudaMemcpyAsync(tmp_sym, symbols, (size_t)(n * npos), cudaMemcpyHostToDevice, h->stream));
-    dsym = (const uint8_t*)tmp_sym;
-    dsum = (unsigned long long*)tmp_sum;
+    int rc = grow(h, &t.buf[0], 1, (size_t)(n * npos));
+    if (rc == TIC_OK) rc = grow(h, &t.buf[1], 1, (size_t)(nb * npos) * 8);
+    if (rc != TIC_OK) return rc;
+    dsym = t.buf[0].as<uint8_t>();
+    dsum = t.buf[1].as<unsigned long long>();
+    TIC_CUDA(h, cudaMemcpyAsync(t.buf[0].p, symbols, (size_t)(n * npos), cudaMemcpyHostToDevice, h->stream));
   }
   position_sums_batched_kernel<<<dim3((unsigned)((npos + 255) / 256), (unsigned)nb), 256, 0, h->stream>>>(dsym, n, npos, batch, dsum);
   h->launches++;
   cudaError_t e = cudaGetLastError();
   if (e == cudaSuccess && mem == TIC_MEM_HOST)
-    e = cudaMemcpyAsync(sums, tmp_sum, (size_t)(nb * npos) * 8, cudaMemcpyDeviceToHost, h->stream);
-  if (mem == TIC_MEM_HOST) {
-    cudaStreamSynchronize(h->stream);
-    cudaFree(tmp_sym);
-    cudaFree(tmp_sum);
-  }
+    e = cudaMemcpyAsync(sums, dsum, (size_t)(nb * npos) * 8, cudaMemcpyDeviceToHost, h->stream);
+  if (mem == TIC_MEM_HOST) cudaStreamSynchronize(h->stream);
   if (e != cudaSuccess) return fail(h, TIC_ERR_CUDA, "position sums failed: %s", cudaGetErrorString(e));
   return TIC_OK;
 }
@@ -1430,20 +1407,10 @@ static int entropy_table(tic_codec* h, const uint32_t* cum, int n_cum) {
   return TIC_OK;
 }
 
-// Grow-only scratch of `pieces` worst-case segment slots and their stored lengths.  The stream is drained first: earlier
-// calls may still be reading the old buffer.
+// Scratch of `pieces` worst-case segment slots and their stored lengths.
 static int ensure_seg_scratch(tic_codec* h, int64_t pieces) {
-  if (pieces <= h->seg_cap) return TIC_OK;
-  TIC_CUDA(h, cudaStreamSynchronize(h->stream));
-  if (h->d_seg) cudaFree(h->d_seg);
-  if (h->d_seg_bytes) cudaFree(h->d_seg_bytes);
-  h->d_seg = nullptr;
-  h->d_seg_bytes = nullptr;
-  h->seg_cap = 0;
-  TIC_CUDA(h, cudaMalloc(&h->d_seg, (size_t)(pieces * kEntropySegSlot)));
-  TIC_CUDA(h, cudaMalloc(&h->d_seg_bytes, (size_t)pieces * sizeof(long long)));
-  h->seg_cap = pieces;
-  return TIC_OK;
+  const int rc = grow(h, &h->d_seg, 1, (size_t)(pieces * kEntropySegSlot));
+  return rc != TIC_OK ? rc : grow(h, &h->d_seg_bytes, 1, (size_t)pieces * sizeof(long long));
 }
 
 int tic_entropy_encode(tic_codec* h, const uint8_t* symbols, int64_t n_streams, int64_t stream_len, const uint32_t* cum_freq,
@@ -1460,15 +1427,16 @@ int tic_entropy_encode(tic_codec* h, const uint8_t* symbols, int64_t n_streams, 
   const uint8_t* dsym = symbols;
   uint8_t* dout = out;
   long long* dbytes = reinterpret_cast<long long*>(out_bytes);
-  void *t_sym = nullptr, *t_out = nullptr, *t_bytes = nullptr;
+  CallTemps t{h};
   if (mem == TIC_MEM_HOST) {
-    TIC_CUDA(h, cudaMalloc(&t_sym, (size_t)std::max<int64_t>(16, n_streams * stream_len)));
-    TIC_CUDA(h, cudaMalloc(&t_out, (size_t)std::max<int64_t>(16, n_streams * out_stride)));
-    TIC_CUDA(h, cudaMalloc(&t_bytes, (size_t)n_streams * 8));
-    TIC_CUDA(h, cudaMemcpyAsync(t_sym, symbols, (size_t)(n_streams * stream_len), cudaMemcpyHostToDevice, h->stream));
-    dsym = (const uint8_t*)t_sym;
-    dout = (uint8_t*)t_out;
-    dbytes = (long long*)t_bytes;
+    rc = grow(h, &t.buf[0], 1, (size_t)std::max<int64_t>(16, n_streams * stream_len));
+    if (rc == TIC_OK) rc = grow(h, &t.buf[1], 1, (size_t)std::max<int64_t>(16, n_streams * out_stride));
+    if (rc == TIC_OK) rc = grow(h, &t.buf[2], 1, (size_t)n_streams * 8);
+    if (rc != TIC_OK) return rc;
+    TIC_CUDA(h, cudaMemcpyAsync(t.buf[0].p, symbols, (size_t)(n_streams * stream_len), cudaMemcpyHostToDevice, h->stream));
+    dsym = t.buf[0].as<uint8_t>();
+    dout = t.buf[1].as<uint8_t>();
+    dbytes = t.buf[2].as<long long>();
   }
   const int64_t nseg = tic_rc_segments(stream_len);
   if (nseg > 0x7fffffffLL / std::max<int64_t>(1, n_streams)) return fail(h, TIC_ERR_INVALID, "too many segments");
@@ -1480,24 +1448,22 @@ int tic_entropy_encode(tic_codec* h, const uint8_t* symbols, int64_t n_streams, 
     h->launches++;
   } else {
     rc_encode_kernel<<<(unsigned)(n_streams * nseg), 32, 0, h->stream>>>(dsym, stream_len, TIC_RC_SEGMENT_SYMBOLS, (int)nseg, h->d_cum, n_cum,
-                                                                           h->d_seg, kEntropySegSlot, h->d_seg_bytes, h->d_oflow + 1);
-    rc_pack_kernel<<<(unsigned)(n_streams * nseg), 256, 0, h->stream>>>(h->d_seg, h->d_seg_bytes, (int)nseg, dout, out_stride, dbytes,
-                                                                                      h->d_oflow + 1);
+                                                                           h->d_seg.as<uint8_t>(), kEntropySegSlot,
+                                                                           h->d_seg_bytes.as<long long>(), h->d_oflow + 1);
+    rc_pack_kernel<<<(unsigned)(n_streams * nseg), 256, 0, h->stream>>>(h->d_seg.as<uint8_t>(), h->d_seg_bytes.as<long long>(), (int)nseg,
+                                                                        dout, out_stride, dbytes, h->d_oflow + 1);
     h->launches += 2;
   }
   cudaError_t e = cudaGetLastError();
   cudaEventRecord(h->ev_t1, h->stream);
   if (mem == TIC_MEM_HOST) {
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out_bytes, t_bytes, (size_t)n_streams * 8, cudaMemcpyDeviceToHost, h->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out_bytes, dbytes, (size_t)n_streams * 8, cudaMemcpyDeviceToHost, h->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
     // only the stored bytes of every stream come back
     for (int64_t i = 0; e == cudaSuccess && i < n_streams; ++i)
       if (out_bytes[i] > 0)
-        e = cudaMemcpyAsync(out + i * out_stride, (uint8_t*)t_out + i * out_stride, (size_t)out_bytes[i], cudaMemcpyDeviceToHost, h->stream);
+        e = cudaMemcpyAsync(out + i * out_stride, dout + i * out_stride, (size_t)out_bytes[i], cudaMemcpyDeviceToHost, h->stream);
     cudaStreamSynchronize(h->stream);
-    cudaFree(t_sym);
-    cudaFree(t_out);
-    cudaFree(t_bytes);
     if (e != cudaSuccess) return fail(h, TIC_ERR_CUDA, "entropy encode failed: %s", cudaGetErrorString(e));
     return overflow_status(h);
   }
@@ -1520,23 +1486,24 @@ int tic_entropy_decode(tic_codec* h, const uint8_t* in, int64_t n_streams, int64
   const uint8_t* din = in;
   const long long* dbytes = reinterpret_cast<const long long*>(in_bytes);
   uint8_t* dsym = symbols;
-  void *t_in = nullptr, *t_bytes = nullptr, *t_sym = nullptr;
+  CallTemps t{h};
   if (mem == TIC_MEM_HOST) {
     for (int64_t i = 0; i < n_streams; ++i)
       if (in_bytes[i] < 0 || in_bytes[i] > in_stride)
         return fail(h, TIC_ERR_INVALID, "entropy decode: stream %lld has %lld bytes in a %lld-byte slot", (long long)i,
                     (long long)in_bytes[i], (long long)in_stride);
-    TIC_CUDA(h, cudaMalloc(&t_in, (size_t)std::max<int64_t>(16, n_streams * in_stride)));
-    TIC_CUDA(h, cudaMalloc(&t_bytes, (size_t)n_streams * 8));
-    TIC_CUDA(h, cudaMalloc(&t_sym, (size_t)std::max<int64_t>(16, n_streams * stream_len)));
+    rc = grow(h, &t.buf[0], 1, (size_t)std::max<int64_t>(16, n_streams * in_stride));
+    if (rc == TIC_OK) rc = grow(h, &t.buf[1], 1, (size_t)n_streams * 8);
+    if (rc == TIC_OK) rc = grow(h, &t.buf[2], 1, (size_t)std::max<int64_t>(16, n_streams * stream_len));
+    if (rc != TIC_OK) return rc;
     for (int64_t i = 0; i < n_streams; ++i) {
       if (in_bytes[i] > 0)
-        TIC_CUDA(h, cudaMemcpyAsync((uint8_t*)t_in + i * in_stride, in + i * in_stride, (size_t)in_bytes[i], cudaMemcpyHostToDevice, h->stream));
+        TIC_CUDA(h, cudaMemcpyAsync(t.buf[0].as<uint8_t>() + i * in_stride, in + i * in_stride, (size_t)in_bytes[i], cudaMemcpyHostToDevice, h->stream));
     }
-    TIC_CUDA(h, cudaMemcpyAsync(t_bytes, in_bytes, (size_t)n_streams * 8, cudaMemcpyHostToDevice, h->stream));
-    din = (const uint8_t*)t_in;
-    dbytes = (const long long*)t_bytes;
-    dsym = (uint8_t*)t_sym;
+    TIC_CUDA(h, cudaMemcpyAsync(t.buf[1].p, in_bytes, (size_t)n_streams * 8, cudaMemcpyHostToDevice, h->stream));
+    din = t.buf[0].as<uint8_t>();
+    dbytes = t.buf[1].as<long long>();
+    dsym = t.buf[2].as<uint8_t>();
   } else if ((reinterpret_cast<uintptr_t>(in) & 15) != 0) {
     return fail(h, TIC_ERR_INVALID, "entropy decode: the stream buffer must be 16-byte aligned");
   }
@@ -1549,11 +1516,8 @@ int tic_entropy_decode(tic_codec* h, const uint8_t* in, int64_t n_streams, int64
   cudaError_t e = cudaGetLastError();
   cudaEventRecord(h->ev_t1, h->stream);
   if (mem == TIC_MEM_HOST) {
-    if (e == cudaSuccess) e = cudaMemcpyAsync(symbols, t_sym, (size_t)(n_streams * stream_len), cudaMemcpyDeviceToHost, h->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(symbols, dsym, (size_t)(n_streams * stream_len), cudaMemcpyDeviceToHost, h->stream);
     cudaStreamSynchronize(h->stream);
-    cudaFree(t_in);
-    cudaFree(t_bytes);
-    cudaFree(t_sym);
   }
   if (e != cudaSuccess) return fail(h, TIC_ERR_CUDA, "entropy decode failed: %s", cudaGetErrorString(e));
   return TIC_OK;
@@ -1565,32 +1529,19 @@ int tic_evaluate_images(tic_codec* h, const uint8_t* images, int64_t n_images, i
   if (!h) return TIC_ERR_INVALID;
   if (n_images < 0 || H <= 0 || W <= 0 || P <= 0 || (n_images > 0 && (!images || !code_bytes || !sq_err)))
     return fail(h, TIC_ERR_INVALID, "bad arguments");
-  if ((H % P != 0 && H < 2) || (W % P != 0 && W < 2)) return fail(h, TIC_ERR_INVALID, "reflect padding needs at least 2 pixels");
-  int rc = check_graph_ready(h, TIC_GRAPH_ENCODER, true);
-  if (rc != TIC_OK) return rc;
-  rc = check_graph_ready(h, TIC_GRAPH_DECODER, true);
-  if (rc != TIC_OK) return rc;
-  if (h->q < 2) return fail(h, TIC_ERR_STATE, "quantiser not configured (tic_set_quantizer)");
-  if (h->g[TIC_GRAPH_ENCODER].layers[0].d.cin != 3) return fail(h, TIC_ERR_INVALID, "encoder must take 3 channels");
-  int hb, wb, cb;
-  rc = tic_bottleneck_shape(h, P, &hb, &wb, &cb);
-  if (rc != TIC_OK) return rc;
-  Graph& gd = h->g[TIC_GRAPH_DECODER];
-  Shape so;
-  if (gd.layers[0].d.cin != cb || graph_out_shape(gd, Shape{hb, wb, cb}, &so) != 0 || so.c != 3 || so.h != P || so.w != P)
-    return fail(h, TIC_ERR_INVALID, "decoder graph does not map the encoder's %dx%dx%d symbols back to %dx%d RGB", hb, wb, cb, P, P);
-  if ((rc = entropy_table_check(h, cum_freq, n_cum)) != TIC_OK) return rc;
+  ImageShapes s;
+  if (int rc = image_shapes(h, H, W, P, true, true, &s)) return rc;
+  if (int rc = entropy_table_check(h, cum_freq, n_cum)) return rc;
   if (n_images == 0) return TIC_OK;
   TIC_CUDA(h, cudaSetDevice(h->device));
-  const bool host = mem == TIC_MEM_HOST;
-  const Geo g0 = image_geo(H, W, P, 0);
-  const int ppi = g0.gh * g0.gw;
+  const bool host = mem != TIC_MEM_DEVICE;
+  const int ppi = s.ppi;
   const int64_t cap = std::max<int64_t>(1, patches_per_chunk(h, P) / ppi);
-  const std::vector<int64_t> sched =
-      host ? host_chunk_schedule(n_images, cap, (double)ppi * P * P / 16384.0) : device_chunk_schedule(n_images, cap);
+  const double p128 = (double)ppi * P * P / 16384.0;
+  const std::vector<int64_t> sched = chunk_schedule(mem, n_images, cap, p128);
   const int64_t ipc = *std::max_element(sched.begin(), sched.end());
   const size_t img_unit = (size_t)H * W * 3;
-  const int64_t stream_len = (int64_t)ppi * hb * wb * cb;  // one image's symbols: one range-coded stream
+  const int64_t stream_len = (int64_t)ppi * s.hb * s.wb * s.cb;  // one image's symbols: one range-coded stream
   const int64_t nseg = tic_rc_segments(stream_len);
   const int64_t npiece = std::max<int64_t>(1, nseg);
   // A piece (one segment, or one plain stream) is a serial chain: a coder launch takes about as long as one piece, however
@@ -1601,64 +1552,39 @@ int tic_evaluate_images(tic_codec* h, const uint8_t* images, int64_t n_images, i
   const int64_t coder_imgs = (kCoderPieces + npiece - 1) / npiece;
   const int64_t sym_cap = std::min<int64_t>(n_images, coder_imgs - 1 + ipc);
   if (sym_cap * npiece > 0x7fffffffLL) return fail(h, TIC_ERR_INVALID, "too many segments");
-  if ((rc = grow_pair(h, h->stage_sym, &h->stage_sym_bytes, (size_t)sym_cap * stream_len)) != TIC_OK) return rc;
-  if (host || !recon)
-    if ((rc = grow_pair(h, h->stage_out, &h->stage_out_bytes, (size_t)ipc * img_unit)) != TIC_OK) return rc;
-  if (host) {
-    if ((rc = grow_pair(h, h->stage_in, &h->stage_in_bytes, (size_t)ipc * img_unit)) != TIC_OK) return rc;
-    if (n_images > h->eval_cap) {
-      TIC_CUDA(h, cudaStreamSynchronize(h->stream));
-      if (h->d_eval) cudaFree(h->d_eval);
-      h->d_eval = nullptr;
-      h->eval_cap = 0;
-      TIC_CUDA(h, cudaMalloc(&h->d_eval, (size_t)n_images * 2 * sizeof(long long)));
-      h->eval_cap = n_images;
-    }
-  }
-  if ((rc = ensure_seg_scratch(h, sym_cap * npiece)) != TIC_OK) return rc;
-  if (int st = overflow_status(h)) return st;
-  long long* d_bytes = host ? h->d_eval : reinterpret_cast<long long*>(code_bytes);
-  unsigned long long* d_sse = host ? reinterpret_cast<unsigned long long*>(h->d_eval + n_images) : reinterpret_cast<unsigned long long*>(sq_err);
+  int rc = grow(h, h->stage_sym, 2, (size_t)sym_cap * stream_len);
+  if (rc == TIC_OK && !host && !recon) rc = grow(h, h->stage_out, 2, (size_t)ipc * img_unit);  // the reconstruction's workspace
+  if (rc == TIC_OK && host) rc = grow(h, &h->d_eval, 1, (size_t)n_images * 2 * sizeof(long long));
+  if (rc == TIC_OK) rc = ensure_seg_scratch(h, sym_cap * npiece);
+  if (rc != TIC_OK) return rc;
+  long long* d_bytes = host ? h->d_eval.as<long long>() : reinterpret_cast<long long*>(code_bytes);
+  unsigned long long* d_sse = host ? reinterpret_cast<unsigned long long*>(d_bytes + n_images) : reinterpret_cast<unsigned long long*>(sq_err);
   // Per chunk, all on the handle's stream: encoder -> symbols -> decoder -> u8 reconstruction -> squared error against
   // the input still in place, then (see kCoderPieces) the range coder, stored lengths only, over the pending symbols.
-  // With host buffers the staging follows tic_roundtrip_images: H2D of chunk i+1 under the kernels of chunk i, the
-  // reconstruction's D2H (when asked for) on the other side stream.  Only n_images * 16 bytes of results come back.
-  const int rc_pipe = [&]() -> int {
-  TIC_CUDA(h, cudaEventRecord(h->ev_t0, h->stream));
+  // With host buffers the next chunk's images may overwrite this one's after the squared error, and the reconstruction
+  // (when asked for) goes back from then on.  Only n_images * 16 bytes of results come back.
+  // The table and the zeroed squared errors go first on the stream: they overlap the first chunk's H2D.  Nothing is
+  // queued for a handle that is already in error.
+  if (int st = overflow_status(h)) return st;
   if ((rc = entropy_table(h, cum_freq, n_cum)) != TIC_OK) return rc;
   TIC_CUDA(h, cudaMemsetAsync(d_sse, 0, (size_t)n_images * sizeof(unsigned long long), h->stream));
-  int64_t u0 = 0, p0 = 0;  // images [p0, u0) are encoded and wait for the range coder
-  for (int64_t idx = 0; idx < (int64_t)sched.size(); u0 += sched[idx], ++idx) {
-    const int b = host ? (int)(idx & 1) : 0;
-    const int64_t nu = sched[idx];
-    // chunk-local staging buffers are indexed from patch 0, the caller's device buffers from the chunk's first patch
-    const uint8_t* img = images;
-    int64_t img0 = u0;
-    uint8_t* rec = recon;
-    int64_t rec0 = u0;
-    if (host) {
-      if (idx >= 2) TIC_CUDA(h, cudaStreamWaitEvent(h->s_h2d, h->ev_enc[b], 0));  // chunk idx-2 is done with stage_in[b]
-      TIC_CUDA(h, cudaMemcpyAsync(h->stage_in[b], images + (size_t)u0 * img_unit, (size_t)nu * img_unit, cudaMemcpyHostToDevice,
-                                  h->s_h2d));
-      TIC_CUDA(h, cudaEventRecord(h->ev_in[b], h->s_h2d));
-      TIC_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_in[b], 0));
-      if (idx >= 2 && recon) TIC_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_out[b], 0));  // stage_out[b] drained
-      img = (const uint8_t*)h->stage_in[b];
-      img0 = 0;
-    }
-    if (host || !recon) {
-      rec = (uint8_t*)h->stage_out[b];
+  int64_t p0 = 0;  // images [p0, c.u0) are encoded and wait for the range coder
+  return drive(h, mem, images, img_unit, {{recon, img_unit, h->stage_out, true}}, n_images, cap, [&](Chunk& c) {
+    uint8_t* rec = (uint8_t*)c.out[0];
+    int64_t rec0 = c.off;
+    if (!rec) {  // device buffers, no reconstruction asked for
+      rec = h->stage_out[0].as<uint8_t>();
       rec0 = 0;
     }
-    uint8_t* sym = (uint8_t*)h->stage_sym[0] + (size_t)(u0 - p0) * stream_len;
+    uint8_t* sym = h->stage_sym[0].as<uint8_t>() + (size_t)(c.u0 - p0) * stream_len;
     IoSpec i, o;
     i.mode = IO_U8_NORM;
-    i.in = img;
-    i.geo = image_geo(H, W, P, img0 * ppi);
+    i.in = c.in;
+    i.geo = image_geo(H, W, P, c.off * ppi);
     o.mode = IO_QUANT_U8;
     o.out = sym;
     o.geo = image_geo(H, W, P, 0);
-    if ((rc = run_graph(h, TIC_GRAPH_ENCODER, i, o, (int)(nu * ppi), P, P)) != TIC_OK) return rc;
+    if (int rc2 = run_graph(h, TIC_GRAPH_ENCODER, i, o, (int)(c.nu * ppi), P, P)) return rc2;
     IoSpec di, dout;
     di.mode = IO_U8_SYMLUT;
     di.in = sym;
@@ -1666,58 +1592,42 @@ int tic_evaluate_images(tic_codec* h, const uint8_t* images, int64_t n_images, i
     dout.mode = IO_DENORM_U8;
     dout.out = rec;
     dout.geo = image_geo(H, W, P, rec0 * ppi);
-    if ((rc = run_graph(h, TIC_GRAPH_DECODER, di, dout, (int)(nu * ppi), hb, wb)) != TIC_OK) return rc;
+    if (int rc2 = run_graph(h, TIC_GRAPH_DECODER, di, dout, (int)(c.nu * ppi), s.hb, s.wb)) return rc2;
     // enough blocks to keep every SM streaming (8 per SM over the chunk), at least 2048 16-byte loads each
     const int64_t nvec = (int64_t)(img_unit + 15) / 16;
-    const int parts = (int)std::max<int64_t>(1, std::min<int64_t>((nvec + 2047) / 2048, (8LL * h->num_sms + nu - 1) / nu));
-    sse_u8_kernel<<<(unsigned)(nu * parts), kSseThreads, 0, h->stream>>>(img + (size_t)img0 * img_unit, rec + (size_t)rec0 * img_unit,
-                                                                         (long long)img_unit, parts, d_sse + u0);
+    const int parts = (int)std::max<int64_t>(1, std::min<int64_t>((nvec + 2047) / 2048, (8LL * h->num_sms + c.nu - 1) / c.nu));
+    sse_u8_kernel<<<(unsigned)(c.nu * parts), kSseThreads, 0, h->stream>>>((const uint8_t*)c.in + (size_t)c.off * img_unit,
+                                                                           rec + (size_t)rec0 * img_unit, (long long)img_unit, parts,
+                                                                           d_sse + c.u0);
     h->launches++;
     TIC_CUDA(h, cudaGetLastError());
-    if (host) {
-      TIC_CUDA(h, cudaEventRecord(h->ev_enc[b], h->stream));
-      if (recon) {
-        TIC_CUDA(h, cudaStreamWaitEvent(h->s_d2h, h->ev_enc[b], 0));
-        TIC_CUDA(h, cudaMemcpyAsync(recon + (size_t)u0 * img_unit, h->stage_out[b], (size_t)nu * img_unit, cudaMemcpyDeviceToHost,
-                                    h->s_d2h));
-        TIC_CUDA(h, cudaEventRecord(h->ev_out[b], h->s_d2h));
-      }
-    }
-    const int64_t pend = u0 + nu - p0;
-    if (pend >= coder_imgs || idx + 1 == (int64_t)sched.size()) {
+    if (int rc2 = mark_consumed(c)) return rc2;
+    const int64_t pend = c.u0 + c.nu - p0;
+    if (pend >= coder_imgs || c.last) {
       // the stored length of each image's stream, exactly tic_entropy_encode's out_bytes: plain streams report it
       // directly, segmented ones through their segment lengths.  The next chunk's encoder overwrites the symbols
       // after these kernels in stream order.
-      const uint8_t* s0 = (const uint8_t*)h->stage_sym[0];
+      const uint8_t* s0 = h->stage_sym[0].as<uint8_t>();
       if (nseg == 0) {
-        rc_encode_kernel<<<(unsigned)pend, 32, 0, h->stream>>>(s0, stream_len, stream_len, 1, h->d_cum, n_cum, h->d_seg, kEntropySegSlot,
-                                                               d_bytes + p0, h->d_oflow + 1);
+        rc_encode_kernel<<<(unsigned)pend, 32, 0, h->stream>>>(s0, stream_len, stream_len, 1, h->d_cum, n_cum, h->d_seg.as<uint8_t>(),
+                                                               kEntropySegSlot, d_bytes + p0, h->d_oflow + 1);
         h->launches++;
       } else {
         rc_encode_kernel<<<(unsigned)(pend * nseg), 32, 0, h->stream>>>(s0, stream_len, TIC_RC_SEGMENT_SYMBOLS, (int)nseg, h->d_cum, n_cum,
-                                                                        h->d_seg, kEntropySegSlot, h->d_seg_bytes, h->d_oflow + 1);
-        rc_stored_length_kernel<<<(unsigned)pend, 256, 0, h->stream>>>(h->d_seg_bytes, (int)nseg, d_bytes + p0);
+                                                                        h->d_seg.as<uint8_t>(), kEntropySegSlot,
+                                                                        h->d_seg_bytes.as<long long>(), h->d_oflow + 1);
+        rc_stored_length_kernel<<<(unsigned)pend, 256, 0, h->stream>>>(h->d_seg_bytes.as<long long>(), (int)nseg, d_bytes + p0);
         h->launches += 2;
       }
       TIC_CUDA(h, cudaGetLastError());
-      p0 = u0 + nu;
+      p0 = c.u0 + c.nu;
     }
-  }
-  TIC_CUDA(h, cudaEventRecord(h->ev_t1, h->stream));
-  if (host) {
-    TIC_CUDA(h, cudaMemcpyAsync(code_bytes, h->d_eval, (size_t)n_images * sizeof(int64_t), cudaMemcpyDeviceToHost, h->stream));
-    TIC_CUDA(h, cudaMemcpyAsync(sq_err, h->d_eval + n_images, (size_t)n_images * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
-    TIC_CUDA(h, cudaStreamSynchronize(h->s_d2h));
-    TIC_CUDA(h, cudaStreamSynchronize(h->stream));
-  }
-  return TIC_OK;
-  }();
-  if (!host) return rc_pipe;
-  if (rc_pipe != TIC_OK) {
-    quiesce(h);
-    return rc_pipe;
-  }
-  return overflow_status(h);
+    if (c.last && host) {
+      TIC_CUDA(h, cudaMemcpyAsync(code_bytes, d_bytes, (size_t)n_images * sizeof(int64_t), cudaMemcpyDeviceToHost, h->stream));
+      TIC_CUDA(h, cudaMemcpyAsync(sq_err, d_sse, (size_t)n_images * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
+    }
+    return (int)TIC_OK;
+  }, p128);
 }
 
 #ifdef TIC_ABLATE
