@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "../../include/tic.h"
+#include "tic_launch.cuh"
 #include "tic_simt.cuh"
 #include "tic_umma.cuh"
 #include "tic_umma16.cuh"
@@ -32,18 +33,16 @@ struct Layer {
   float* w = nullptr;     // device [9][cin][cout]
   float* b = nullptr;     // device [cout]
   std::vector<float> hb;  // host copy of the bias (the fused kernels take it as launch constants)
-  UmmaWeights uw;         // tensor-path operand images (built lazily from w)
-  U16Weights uw16;        // fp16-pair operand images
-  F16Weights fw16;        // fp16-pair first-layer (cin = 3) operand image
-  FusedDecWeights fdw;    // operand images of this layer and the next one for the fused transposed-conv pair
-  FusedEncWeights few;    // ... for the fused first two layers of an encoder
+  // operand images, built lazily from w: TF32 slices of 64 output channels, fp16-pair output-channel slices, the fp16-pair
+  // first layer (cin = 3), and this layer's and the next one's for a fused pair kernel (decoder tail or encoder head)
+  OperandImage img[4 + 16 + 1 + 2];
+  OperandImage* tf32() { return img; }
+  OperandImage* pair16() { return img + 4; }
+  OperandImage& first16() { return img[20]; }
+  OperandImage* fused() { return img + 21; }
   bool loaded = false;
   void release() {  // the operand images (rebuilt from w on the next launch)
-    uw.release();
-    uw16.release();
-    fw16.release();
-    fdw.release();
-    few.release();
+    for (OperandImage& i : img) i.release();
   }
 };
 
@@ -59,18 +58,6 @@ struct IoSpec {
   const void* in = nullptr;
   void* out = nullptr;
   Geo geo{};
-};
-
-// A device buffer that only grows (grow()).  Its destructor frees the memory.
-struct DevBuf {
-  void* p = nullptr;
-  size_t bytes = 0;
-  DevBuf() = default;
-  DevBuf(const DevBuf&) = delete;
-  DevBuf& operator=(const DevBuf&) = delete;
-  ~DevBuf() { cudaFree(p); }
-  template <typename T>
-  T* as() const { return static_cast<T*>(p); }
 };
 
 }  // namespace
@@ -140,11 +127,7 @@ int grow(tic_codec* h, DevBuf* bufs, int count, size_t need, int nomem = TIC_ERR
   bool held = false;
   for (int i = 0; i < count; ++i) held = held || bufs[i].p;
   if (held) TIC_CUDA(h, cudaDeviceSynchronize());
-  for (int i = 0; i < count; ++i) {
-    cudaFree(bufs[i].p);
-    bufs[i].p = nullptr;
-    bufs[i].bytes = 0;
-  }
+  for (int i = 0; i < count; ++i) bufs[i].reset();
   for (int i = 0; i < count; ++i) {
     const cudaError_t e = cudaMalloc(&bufs[i].p, need);
     if (e != cudaSuccess) return fail(h, nomem, "cudaMalloc(%zu) failed: %s", need, cudaGetErrorString(e));
@@ -195,23 +178,6 @@ void same_pad(int in, int s, int* out, int* before) {
 }
 
 // ---- SIMT launch planning -------------------------------------------------------------------
-template <int OCB, int S>
-int launch_conv_t(tic_codec* h, const LayerArgs& a, const SmemPlan& sp, dim3 grid, size_t smem) {
-  auto k = conv3x3_simt_kernel<OCB, S>;
-  static SmemAttrCache cache;
-  TIC_CUDA(h, cache.ensure(reinterpret_cast<const void*>(k), smem, 48 * 1024));
-  k<<<grid, kThreads, smem, h->stream>>>(a, sp);
-  return TIC_OK;
-}
-template <int OCB>
-int launch_deconv_t(tic_codec* h, const LayerArgs& a, const SmemPlan& sp, dim3 grid, size_t smem) {
-  auto k = deconv3x3_simt_kernel<OCB>;
-  static SmemAttrCache cache;
-  TIC_CUDA(h, cache.ensure(reinterpret_cast<const void*>(k), smem, 48 * 1024));
-  k<<<grid, kThreads, smem, h->stream>>>(a, sp);
-  return TIC_OK;
-}
-
 // Pick the row pitch so that the (up to four) row groups a warp spans land in distinct banks.
 int pick_pitch(int iw, int lanes_x, int row_words /* words between a warp's row groups, per pitch unit */, int s) {
   if (lanes_x * s >= 32) return iw | 1;
@@ -263,34 +229,24 @@ int launch_simt(tic_codec* h, LayerArgs a, int kind, int stride) {
   dim3 grid((unsigned)gx, (unsigned)grid_y);
   const size_t smem = ((size_t)a.TP * sp.pstr + 9 * kIcc * ocb) * sizeof(float);
   if (smem > 200 * 1024) return fail(h, TIC_ERR_UNSUPPORTED, "tile needs %zu B shared memory", smem);
-  int rc = TIC_OK;
-  if (kind == TIC_CONV) {
-    if (stride == 1) {
-      switch (ocb) {
-        case 64: rc = launch_conv_t<64, 1>(h, a, sp, grid, smem); break;
-        case 32: rc = launch_conv_t<32, 1>(h, a, sp, grid, smem); break;
-        case 16: rc = launch_conv_t<16, 1>(h, a, sp, grid, smem); break;
-        default: rc = launch_conv_t<8, 1>(h, a, sp, grid, smem); break;
-      }
-    } else {
-      switch (ocb) {
-        case 64: rc = launch_conv_t<64, 2>(h, a, sp, grid, smem); break;
-        case 32: rc = launch_conv_t<32, 2>(h, a, sp, grid, smem); break;
-        case 16: rc = launch_conv_t<16, 2>(h, a, sp, grid, smem); break;
-        default: rc = launch_conv_t<8, 2>(h, a, sp, grid, smem); break;
-      }
-    }
-  } else {
-    switch (ocb) {
-      case 32: rc = launch_deconv_t<32>(h, a, sp, grid, smem); break;
-      case 16: rc = launch_deconv_t<16>(h, a, sp, grid, smem); break;
-      case 8: rc = launch_deconv_t<8>(h, a, sp, grid, smem); break;
-      default: rc = launch_deconv_t<4>(h, a, sp, grid, smem); break;
-    }
-  }
-  if (rc != TIC_OK) return rc;
+  void (*kernel)(LayerArgs, SmemPlan);
+  if (kind != TIC_CONV)
+    kernel = ocb == 32   ? deconv3x3_simt_kernel<32>
+             : ocb == 16 ? deconv3x3_simt_kernel<16>
+             : ocb == 8  ? deconv3x3_simt_kernel<8>
+                         : deconv3x3_simt_kernel<4>;
+  else if (stride == 1)
+    kernel = ocb == 64   ? conv3x3_simt_kernel<64, 1>
+             : ocb == 32 ? conv3x3_simt_kernel<32, 1>
+             : ocb == 16 ? conv3x3_simt_kernel<16, 1>
+                         : conv3x3_simt_kernel<8, 1>;
+  else
+    kernel = ocb == 64   ? conv3x3_simt_kernel<64, 2>
+             : ocb == 32 ? conv3x3_simt_kernel<32, 2>
+             : ocb == 16 ? conv3x3_simt_kernel<16, 2>
+                         : conv3x3_simt_kernel<8, 2>;
   h->launches++;
-  TIC_CUDA(h, cudaGetLastError());
+  TIC_CUDA(h, launch_dyn(kernel, grid, kThreads, smem, h->stream, a, sp));
   return TIC_OK;
 }
 
@@ -405,6 +361,7 @@ int run_graph(tic_codec* h, int gi, const IoSpec& io_in, const IoSpec& io_out, i
     TIC_CUDA(h, cudaGetLastError());
     cur = 0;
   }
+  const LaunchCtx ctx{h->stream, h->num_sms, &h->err, &h->launches};
   for (int i = 0; i < L; ++i) {
     Layer& ly = g.layers[i];
     const tic_layer_desc& d = ly.d;
@@ -480,9 +437,7 @@ int run_graph(tic_codec* h, int gi, const IoSpec& io_in, const IoSpec& io_out, i
       a2.out = io_out.mode == IO_ACT ? nullptr : io_out.out;
       a2.geo = io_out.geo;
       if (a2.out && fused_dec_supported(a, d.kind, a2, ly2.d.kind)) {
-        int nl = 0;
-        rc = launch_fused_dec(h->stream, a, a2, ly.w, ly2.w, ly.hb.data(), ly2.hb.data(), &ly.fdw, h->num_sms, &h->err, &nl);
-        h->launches += nl;
+        rc = launch_fused_dec(ctx, a, a2, ly.w, ly2.w, ly.hb.data(), ly2.hb.data(), ly.fused());
         fused = true;
       }
     }
@@ -498,9 +453,7 @@ int run_graph(tic_codec* h, int gi, const IoSpec& io_in, const IoSpec& io_out, i
       a2.out = h->act[0].p;
       a2.out_lo_off = (long long)n * a2.hout * a2.wout * a2.cout;
       if (fused_enc_supported(a, d.kind, d.stride, a2, ly2.d.kind, ly2.d.stride)) {
-        int nl = 0;
-        rc = launch_fused_enc(h->stream, a, a2, ly.w, ly2.w, ly.hb.data(), &ly.few, h->num_sms, &h->err, &nl);
-        h->launches += nl;
+        rc = launch_fused_enc(ctx, a, a2, ly.w, ly2.w, ly.hb.data(), ly.fused());
         fused = true;
         ob = 0;  // the pair's output lives in act[0]
       }
@@ -508,18 +461,11 @@ int run_graph(tic_codec* h, int gi, const IoSpec& io_in, const IoSpec& io_out, i
     if (fused) {
       ++i;  // the next layer ran inside this launch (its time is reported with this layer)
     } else if (pair16 && f16_first_supported(a, d.kind, d.stride)) {
-      int nl = 0;
-      rc = launch_first16(h->stream, a, d.stride, ly.w, &ly.fw16, h->num_sms, &h->err, &nl);
-      h->launches += nl;
+      rc = launch_first16(ctx, a, d.stride, ly.w, ly.first16());
     } else if (pair16 && u16_supported(a, d.kind, d.stride)) {
-      int nl = 0;
-      rc = launch_u16(h->stream, a, d.kind, d.stride, ly.w, &ly.uw16, h->num_sms, &h->err, &nl);
-      h->launches += nl;
+      rc = launch_u16(ctx, a, d.kind, d.stride, ly.w, ly.pair16());
     } else if (h->mode != TIC_COMPUTE_FP32 && !pair16 && umma_supported(a, d.kind, d.stride)) {
-      int nl = 0;
-      rc = launch_umma(h->stream, a, d.kind, d.stride, ly.w, &ly.uw, h->mode == TIC_COMPUTE_TENSOR_3XTF32, h->num_sms,
-                       &h->err, &nl);
-      h->launches += nl;
+      rc = launch_umma(ctx, a, d.kind, d.stride, ly.w, ly.tf32(), h->mode == TIC_COMPUTE_TENSOR_3XTF32);
     } else {
       rc = launch_simt(h, a, d.kind, d.stride);
     }
@@ -527,7 +473,7 @@ int run_graph(tic_codec* h, int gi, const IoSpec& io_in, const IoSpec& io_out, i
       cudaEventRecord(pr.e1, h->stream);
       h->prof_pending.push_back(pr);
     }
-    if (rc != TIC_OK) return rc < 0 && rc >= TIC_ERR_UNSUPPORTED ? rc : TIC_ERR_CUDA;
+    if (rc != TIC_OK) return rc;
     if (d.res_end) {
       res_buf = -1;
       res_ptr = nullptr;
@@ -759,12 +705,11 @@ int image_shapes(tic_codec* h, int H, int W, int P, bool enc, bool dec, ImageSha
   return TIC_OK;
 }
 
-// Frees a graph's weights and operand images.
+// Frees a graph's weights (its layers' operand images go with the layers).
 void free_layers(Graph& g) {
   for (auto& l : g.layers) {
     cudaFree(l.w);
     cudaFree(l.b);
-    l.release();
   }
   g.layers.clear();
 }
@@ -962,10 +907,8 @@ int tic_load_weights(tic_codec* h, int graph, int layer, const float* kernel, co
   TIC_CUDA(h, cudaMemcpy(l.b, bias, (size_t)cout * sizeof(float), cudaMemcpyHostToDevice));
   l.hb.assign(bias, bias + cout);
   l.release();
-  if (layer > 0) {  // the fused pair kernels keep this layer's operand image with the previous layer
-    g.layers[layer - 1].fdw.release();
-    g.layers[layer - 1].few.release();
-  }
+  if (layer > 0)  // the fused pair kernels keep this layer's operand image with the previous layer
+    for (int k = 0; k < 2; ++k) g.layers[layer - 1].fused()[k].release();
   l.loaded = true;
   return TIC_OK;
 }

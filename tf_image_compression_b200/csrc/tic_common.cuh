@@ -5,7 +5,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdlib.h>
-#include <mutex>
 #include "../../include/tic_math.h"
 
 namespace tic {
@@ -45,26 +44,6 @@ inline int tic_env_int(const char* name, int dflt) {
 inline int tic_env_int(const char*, int dflt) { return dflt; }
 #define TIC_DBG_BITS(x) 0
 #endif
-
-// cudaFuncAttributeMaxDynamicSharedMemorySize is a PER-DEVICE attribute of a kernel: the "already configured" cache of a
-// launcher is keyed by the current device (one handle per device, several devices per process), and guarded by a mutex
-// because handles of different devices may launch from different threads.
-struct SmemAttrCache {
-  static constexpr int kMaxDevices = 64;
-  size_t have[kMaxDevices] = {};
-  std::mutex mu;
-  cudaError_t ensure(const void* kernel, size_t smem, size_t always_above = 0) {
-    if (smem <= always_above) return cudaSuccess;
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return e;
-    std::lock_guard<std::mutex> lock(mu);
-    if (dev >= 0 && dev < kMaxDevices && smem <= have[dev]) return cudaSuccess;
-    e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess && dev >= 0 && dev < kMaxDevices) have[dev] = smem;
-    return e;
-  }
-};
 
 // How the first layer reads its input / the last layer writes its output.
 enum IoMode : int {

@@ -11,6 +11,7 @@
 // latency-bound, all 27 loads of a pixel are issued before any is used), 8-15 epilogue (shared with
 // tic_umma16.cuh), 16 MMA issuer + TMEM.
 #pragma once
+#include "tic_launch.cuh"
 #include "tic_umma16.cuh"
 
 namespace tic {
@@ -1031,21 +1032,7 @@ inline bool f16_first_tma_ok(const LayerArgs& a) {
   return true;
 }
 
-struct F16Weights {
-  uint8_t* img = nullptr;
-  bool windowed = false;
-  void release() {
-    if (img) cudaFree(img);
-    img = nullptr;
-  }
-};
-
-inline int launch_first16(cudaStream_t stream, const LayerArgs& a, int stride, const float* w_dev, F16Weights* fw, int num_sms,
-                          std::string* err, int* launches) {
-  auto fail = [&](const std::string& what, int code) {
-    if (err) *err = what;
-    return code;
-  };
+inline tic_status launch_first16(const LaunchCtx& c, const LayerArgs& a, int stride, const float* w_dev, OperandImage& img) {
   F16Params p{};
   p.n = a.n;
   p.P = a.hin;
@@ -1056,7 +1043,7 @@ inline int launch_first16(cudaStream_t stream, const LayerArgs& a, int stride, c
   p.tiles_x = a.wout / 8;
   p.tiles_y = a.hout / p.bh;
   p.num_tiles = (long long)p.tiles_x * p.tiles_y * ((a.n + p.bn - 1) / p.bn);
-  if (p.num_tiles >= (1LL << 31) - 65536) return fail("too many tiles for one launch", -5);
+  if (p.num_tiles >= (1LL << 31) - 65536) return c.fail("too many tiles for one launch", TIC_ERR_UNSUPPORTED);
   p.tx_d = make_fastdiv((uint32_t)p.tiles_x);
   p.ty_d = make_fastdiv((uint32_t)p.tiles_y);
   p.txy_d = make_fastdiv((uint32_t)(p.tiles_x * p.tiles_y));
@@ -1064,92 +1051,49 @@ inline int launch_first16(cudaStream_t stream, const LayerArgs& a, int stride, c
   p.dbg = tic_env_int("TIC_DBG", 0);  // -DTIC_ABLATE builds only
   p.nbuf = std::min(4, 512 / (2 * p.npad));
   const bool windowed = stride == 2 && p.bn == 1;  // operands straight from the staged input tile (no im2col)
-  if (!fw->img || fw->windowed != windowed) {
-    fw->release();
-    if (cudaMalloc(&fw->img, 192 * 64) != cudaSuccess) return fail("cudaMalloc for first-layer weight image failed", -4);
-    fw->windowed = windowed;
-    cudaMemsetAsync(fw->img, 0, 192 * 64, stream);
-    if (windowed)
-      f16_build_weights_s2_kernel<<<8, 256, 0, stream>>>(w_dev, a.cout, p.npad, fw->img);
-    else
-      f16_build_weights_kernel<<<8, 256, 0, stream>>>(w_dev, a.cout, p.npad, fw->img);
-    if (cudaGetLastError() != cudaSuccess) return fail("first-layer weight image kernel failed", -2);
+  auto builder = windowed ? f16_build_weights_s2_kernel : f16_build_weights_kernel;
+  bool build;
+  if (img.ensure(image_key(builder, w_dev, a.cout, p.npad), 192 * 64, &build) != TIC_OK)
+    return c.fail("cudaMalloc for first-layer weight image failed", TIC_ERR_NOMEM);
+  if (build) {
+    if (cudaMemsetAsync(img.buf.p, 0, 192 * 64, c.stream) != cudaSuccess)
+      return c.fail("cudaMemsetAsync of the first-layer weight image failed", TIC_ERR_CUDA);
+    builder<<<8, 256, 0, c.stream>>>(w_dev, a.cout, p.npad, img.buf.as<uint8_t>());
+    if (cudaGetLastError() != cudaSuccess) return c.fail("first-layer weight image kernel failed", TIC_ERR_CUDA);
   }
-  p.wimg = fw->img;
-  const size_t smem = kF16Stages * kF16StageBytes + 2 * 64 * 64 + kU16StageBytes + sizeof(F16SmemBars) + 1024;
-  const size_t smem_w2 = kW2Stages * 10240 + 192 * 64 + kU16StageBytes + kRawStages * kRawStage + sizeof(W2SmemBars) + 1024;
+  p.wimg = img.img();
   CUtensorMap tm_img{};
-  p.use_tma = 0;
-  if (windowed && f16_first_tma_ok(a)) {
-    auto encode = umma_encode_fn();
-    if (encode) {
-      const Geo& g = a.geo;
-      const long long per_img = (long long)g.gh * g.gw;
-      const cuuint64_t nimg = (cuuint64_t)((g.n0 + a.n + per_img - 1) / per_img);
-      const bool f32in = a.in_mode == IO_F32_NORM;
-      const cuuint64_t eb = f32in ? 4 : 1;
-      cuuint64_t dims[3] = {(cuuint64_t)g.W * 3, (cuuint64_t)g.H, nimg};
-      cuuint64_t strides[2] = {(cuuint64_t)g.W * 3 * eb, (cuuint64_t)g.H * g.W * 3 * eb};
-      cuuint32_t box[3] = {f32in ? kRawRowF32 / 4 : kRawRow, (cuuint32_t)kW2Rows, 1};
-      cuuint32_t es[3] = {1, 1, 1};
-      CUresult r = encode(&tm_img, f32in ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 3,
-                          const_cast<void*>(a.in), dims, strides, box, es,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r == CUDA_SUCCESS) p.use_tma = 1;
-    }
-  }
-  const int grid = (int)std::min<long long>(p.num_tiles, num_sms);
-  static SmemAttrCache cache_k1, cache_k2, cache_w2;
-  if (cache_k1.ensure(reinterpret_cast<const void*>(f16_first_kernel<1>), smem) != cudaSuccess ||
-      cache_k2.ensure(reinterpret_cast<const void*>(f16_first_kernel<2>), smem) != cudaSuccess ||
-      cache_w2.ensure(reinterpret_cast<const void*>(f16_first_s2_kernel), smem_w2) != cudaSuccess)
-    return fail("cudaFuncSetAttribute(first-layer kernel) failed", -2);
+  // raw u8 / f32 image windows by TMA where the geometry allows it (otherwise the builders load them)
+  const bool f32in = a.in_mode == IO_F32_NORM;
+  p.use_tma = windowed && f16_first_tma_ok(a) &&
+              tmap_image_rows(&tm_img, a, f32in, f32in ? kRawRowF32 / 4 : kRawRow, kW2Rows, nullptr, nullptr) == TIC_OK;
+  const int grid = (int)std::min<long long>(p.num_tiles, c.num_sms);
   // the TMA-fed, pair-plane-output kernel (16 epilogue warps) when the launch qualifies
   const bool t2 = windowed && p.use_tma && a.out_mode == IO_ACT16 && (a.cout == 32 || a.cout == 16) && p.nbuf == 4;
   // the general kernel's TMA builders take u8 windows of an un-shifted grid only
   if (!t2 && (a.in_mode != IO_U8_NORM || a.geo.oy != 0 || a.geo.ox != 0)) p.use_tma = 0;
+  cudaError_t e;
   if (t2) {
-    const bool f32in = a.in_mode == IO_F32_NORM;
     const size_t smem_t2 = kT2Stages * 10240 + 192 * 64 + kT2EpiWarps * kT2StagePerWarp +
                            kT2Stages * (f32in ? kRawStageF32 : kRawStage) + sizeof(W2SmemBars) + 1024;
-    static SmemAttrCache cache_t2u, cache_t2f;
-    const size_t big = kT2Stages * 10240 + 192 * 64 + kT2EpiWarps * kT2StagePerWarp + kT2Stages * kRawStageF32 +
-                       sizeof(W2SmemBars) + 1024;
-    if (cache_t2u.ensure(reinterpret_cast<const void*>(f16_first_s2_tma_kernel<false>), big) != cudaSuccess ||
-        cache_t2f.ensure(reinterpret_cast<const void*>(f16_first_s2_tma_kernel<true>), big) != cudaSuccess)
-      return fail("cudaFuncSetAttribute(first-layer TMA kernel) failed", -2);
-    // output tensor maps (hi / lo' plane of the NHWC pair-plane activation): box = one epilogue warp's 4 rows x 8 columns
+    // output tensor maps (hi / lo' plane of the NHWC pair-plane activation)
     CUtensorMap tm_o[2];
-    {
-      auto encode = umma_encode_fn();
-      const cuuint64_t C = a.cout, Wd = a.wout, Hd = a.hout, Nd = a.n;
-      cuuint64_t dims[4] = {C, Wd, Hd, Nd};
-      cuuint64_t strides[3] = {C * 2, Wd * C * 2, Hd * Wd * C * 2};
-      cuuint32_t box[4] = {(cuuint32_t)a.cout, 8, 4, 1};
-      cuuint32_t es[4] = {1, 1, 1, 1};
-      for (int pl = 0; pl < 2; ++pl) {
-        void* base = reinterpret_cast<__half*>(a.out) + (pl ? a.out_lo_off : 0);
-        CUresult r = encode(&tm_o[pl], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                            a.cout == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled (first-layer output) failed (" + std::to_string((int)r) + ")", -2);
-      }
-    }
-    if (f32in)
-      f16_first_s2_tma_kernel<true><<<grid, kT2Threads, smem_t2, stream>>>(tm_img, tm_o[0], tm_o[1], p, a);
-    else
-      f16_first_s2_tma_kernel<false><<<grid, kT2Threads, smem_t2, stream>>>(tm_img, tm_o[0], tm_o[1], p, a);
-  } else if (windowed)
-    f16_first_s2_kernel<<<grid, kW2Threads, smem_w2, stream>>>(tm_img, p, a);
-  else if (stride == 1)
-    f16_first_kernel<1><<<grid, kF16Threads, smem, stream>>>(p, a);
-  else
-    f16_first_kernel<2><<<grid, kF16Threads, smem, stream>>>(p, a);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return fail(std::string("first-layer tensor launch failed: ") + cudaGetErrorString(e), -2);
-  if (launches) ++*launches;
-  return 0;
+    for (int pl = 0; pl < 2; ++pl)
+      if (tic_status s = tmap_pair_out(&tm_o[pl], reinterpret_cast<__half*>(a.out) + (pl ? a.out_lo_off : 0), a.n, a.hout, a.wout, a.cout,
+                                       "first-layer output", c.err))
+        return s;
+    e = launch_dyn(f32in ? f16_first_s2_tma_kernel<true> : f16_first_s2_tma_kernel<false>, grid, kT2Threads, smem_t2, c.stream, tm_img,
+                   tm_o[0], tm_o[1], p, a);
+  } else if (windowed) {
+    const size_t smem_w2 = kW2Stages * 10240 + 192 * 64 + kU16StageBytes + kRawStages * kRawStage + sizeof(W2SmemBars) + 1024;
+    e = launch_dyn(f16_first_s2_kernel, grid, kW2Threads, smem_w2, c.stream, tm_img, p, a);
+  } else {
+    const size_t smem = kF16Stages * kF16StageBytes + 2 * 64 * 64 + kU16StageBytes + sizeof(F16SmemBars) + 1024;
+    e = launch_dyn(stride == 1 ? f16_first_kernel<1> : f16_first_kernel<2>, grid, kF16Threads, smem, c.stream, p, a);
+  }
+  if (e != cudaSuccess) return c.fail(std::string("first-layer tensor launch failed: ") + cudaGetErrorString(e), TIC_ERR_CUDA);
+  ++*c.launches;
+  return TIC_OK;
 }
 
 }  // namespace tic

@@ -23,6 +23,7 @@
 // role code).  The issuer runs MMA1 of tile i + 1 ahead of MMA2 of tile i, and epilogue 1 converts the accumulators
 // while the previous MMA2 still runs, so only the region writes sit between two MMA2s.
 #pragma once
+#include "tic_launch.cuh"
 #include "tic_umma16.cuh"
 
 namespace tic {
@@ -442,53 +443,23 @@ inline bool fused_dec_supported(const LayerArgs& a1, int kind1, const LayerArgs&
   return true;
 }
 
-struct FusedDecWeights {
-  U16WeightSlice w1, w2;
-  void release() {
-    w1.release();
-    w2.release();
-  }
-};
-
-inline int u16_ensure_pair_weights(cudaStream_t stream, const float* w_dev, const LayerArgs& a, const U16Params& p, U16WeightSlice* ws) {
-  const size_t img_bytes = 2 * (size_t)p.w_bytes;
-  if (!ws->img || ws->bytes != img_bytes || ws->mode != p.mode || ws->npad != p.npad || ws->oc0 != 0) {
-    ws->release();
-    if (cudaMalloc(&ws->img, img_bytes) != cudaSuccess) return -4;
-    ws->bytes = img_bytes;
-    ws->mode = p.mode;
-    ws->npad = p.npad;
-    ws->oc0 = 0;
-    u16_build_weights_pair_kernel<<<64, 256, 0, stream>>>(w_dev, a.cin, a.cout, 0, a.cout, p.npad, p.cpad, p.mode == U16_DECONV_PH, p.kc, p.KB,
-                                                          (p.wA_bytes + 1023u) & ~1023u, (p.wB_bytes + 1023u) & ~1023u, ws->img);
-    if (cudaGetLastError() != cudaSuccess) return -2;
-  }
-  return 0;
-}
-
-inline int launch_fused_dec(cudaStream_t stream, const LayerArgs& a1, const LayerArgs& a2, const float* w1_dev, const float* w2_dev,
-                            const float* bias1_host, const float* bias2_host,
-                            FusedDecWeights* fw, int num_sms, std::string* err, int* launches) {
-  auto fail = [&](const std::string& what, int code) {
-    if (err) *err = what;
-    return code;
-  };
-  auto encode = umma_encode_fn();
-  if (!encode) return fail("cuTensorMapEncodeTiled is unavailable (driver too old?)", -2);
-  if (num_sms < 2) return fail("the fused decoder kernel needs CTA pairs", -5);
+// img[0], img[1]: the operand images of the two layers
+inline tic_status launch_fused_dec(const LaunchCtx& c, const LayerArgs& a1, const LayerArgs& a2, const float* w1_dev, const float* w2_dev,
+                                   const float* bias1_host, const float* bias2_host, OperandImage* img) {
+  if (c.num_sms < 2) return c.fail("the fused decoder kernel needs CTA pairs", TIC_ERR_UNSUPPORTED);
   U16Plan pl1{}, pl2{};
-  if (!u16_plan(a1, 1, 2, a1.cout, &pl1) || !u16_plan(a2, 1, 2, a2.cout, &pl2)) return fail("fused decoder plan failed", -5);
+  if (!u16_plan(a1, 1, 2, a1.cout, &pl1) || !u16_plan(a2, 1, 2, a2.cout, &pl2)) return c.fail("fused decoder plan failed", TIC_ERR_UNSUPPORTED);
   U16Params p1 = pl1.p, p2 = pl2.p;
   if (p1.mode != U16_DECONV_PH || p1.cpad != 32 || p2.mode != U16_DECONV_PH || p2.cpad != 4 || p1.ksteps != 2 || p2.ksteps != 2)
-    return fail("fused decoder: unexpected layer plan", -5);
+    return c.fail("fused decoder: unexpected layer plan", TIC_ERR_UNSUPPORTED);
   // layer 2 reads its operand from the region buffer: pitch 17 pixels, views (dy, dx) = rows / columns -1 + dy / dx
   for (int v = 0; v < 4; ++v) p2.a_off[v] = (uint32_t)(((v >> 1) * kFusedRegionCols + (v & 1)) * 64);
   p2.sbo = kFusedRegionPitch;
-  int rc = u16_ensure_pair_weights(stream, w1_dev, a1, p1, &fw->w1);
-  if (rc == 0) rc = u16_ensure_pair_weights(stream, w2_dev, a2, p2, &fw->w2);
-  if (rc != 0) return fail("fused decoder: weight images failed", rc);
-  p1.wimg = fw->w1.img;
-  p2.wimg = fw->w2.img;
+  tic_status s = u16_pair_image(c.stream, img[0], w1_dev, a1, p1, 0, a1.cout);
+  if (s == TIC_OK) s = u16_pair_image(c.stream, img[1], w2_dev, a2, p2, 0, a2.cout);
+  if (s != TIC_OK) return c.fail("fused decoder: weight images failed", s);
+  p1.wimg = img[0].img();
+  p2.wimg = img[1].img();
   p1.dbg = tic_env_int("TIC_DBG", 0);  // -DTIC_ABLATE builds only: 1 no MMA2, 16 no MMA1, 2 no epilogue 2, 4 no region writes
 
   FusedDecParams fp{};
@@ -522,29 +493,18 @@ inline int launch_fused_dec(cudaStream_t stream, const LayerArgs& a1, const Laye
   fp.bars_off = off;
   off += (uint32_t)sizeof(FusedDecBars);
   fp.smem_bytes = off + 1024u;
-  if (fp.smem_bytes > 227u * 1024u - 1024u) return fail("fused decoder: shared memory plan does not fit", -5);
+  if (fp.smem_bytes > 227u * 1024u - 1024u) return c.fail("fused decoder: shared memory plan does not fit", TIC_ERR_UNSUPPORTED);
 
   CUtensorMap tm[2];
-  const cuuint64_t C = a1.cin, W = a1.win, H = a1.hin, N = a1.n;
-  for (int pl = 0; pl < 2; ++pl) {
-    void* base = const_cast<__half*>(reinterpret_cast<const __half*>(a1.in) + (pl ? a1.in_lo_off : 0));
-    cuuint64_t dims[4] = {C, W, N, H};
-    cuuint64_t strides[3] = {C * 2, H * W * C * 2, W * C * 2};
-    cuuint32_t box[4] = {(cuuint32_t)p1.kc, 9, 1, 17};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    CUresult r = encode(&tm[pl], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled failed (" + std::to_string((int)r) + ")", -2);
-  }
-  static SmemAttrCache cache;
-  if (cache.ensure(reinterpret_cast<const void*>(fused_dec_kernel), fp.smem_bytes) != cudaSuccess)
-    return fail("cudaFuncSetAttribute(fused decoder) failed", -2);
-  const int grid = 2 * (int)std::min<long long>(fp.pairs_total, num_sms / 2);
-  fused_dec_kernel<<<grid, kFusedThreads, fp.smem_bytes, stream>>>(tm[0], tm[1], p1, a1, p2, a2, fp);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return fail(std::string("fused decoder launch failed: ") + cudaGetErrorString(e), -2);
-  if (launches) ++*launches;
-  return 0;
+  for (int pl = 0; pl < 2; ++pl)
+    if (tic_status st = tmap_act(&tm[pl], reinterpret_cast<const __half*>(a1.in) + (pl ? a1.in_lo_off : 0), true, a1, false,
+                                 {(cuuint32_t)p1.kc, 9, 1, 17}, CU_TENSOR_MAP_SWIZZLE_64B, c.err))
+      return st;
+  const int grid = 2 * (int)std::min<long long>(fp.pairs_total, c.num_sms / 2);
+  const cudaError_t e = launch_dyn(fused_dec_kernel, grid, kFusedThreads, fp.smem_bytes, c.stream, tm[0], tm[1], p1, a1, p2, a2, fp);
+  if (e != cudaSuccess) return c.fail(std::string("fused decoder launch failed: ") + cudaGetErrorString(e), TIC_ERR_CUDA);
+  ++*c.launches;
+  return TIC_OK;
 }
 
 }  // namespace tic

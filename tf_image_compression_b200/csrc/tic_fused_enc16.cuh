@@ -26,6 +26,7 @@
 #pragma once
 #include "tic_first16.cuh"
 #include "tic_fused16.cuh"
+#include "tic_launch.cuh"
 
 namespace tic {
 
@@ -579,48 +580,32 @@ inline bool fused_enc_supported(const LayerArgs& a1, int kind1, int stride1, con
   return f16_first_tma_ok(a1);
 }
 
-struct FusedEncWeights {
-  uint8_t* w1 = nullptr;
-  FusedEncNorm nm{};        // the normalisation constants folded into w1 (tic_set_norm after the first launch rebuilds it)
-  U16WeightSlice w2;
-  void release() {
-    if (w1) cudaFree(w1);
-    w1 = nullptr;
-    w2.release();
-  }
-};
-
-inline int launch_fused_enc(cudaStream_t stream, const LayerArgs& a1, const LayerArgs& a2, const float* w1_dev, const float* w2_dev,
-                            const float* bias1_host,
-                            FusedEncWeights* fw, int num_sms, std::string* err, int* launches) {
-  auto fail = [&](const std::string& what, int code) {
-    if (err) *err = what;
-    return code;
-  };
-  auto encode = umma_encode_fn();
-  if (!encode) return fail("cuTensorMapEncodeTiled is unavailable (driver too old?)", -2);
-  if (num_sms < 2) return fail("the fused encoder kernel needs CTA pairs", -5);
+// img[0]: the first layer's operand image with the normalisation folded in (f16_build_weights_s2_pair_kernel), img[1]: the
+// second layer's
+inline tic_status launch_fused_enc(const LaunchCtx& c, const LayerArgs& a1, const LayerArgs& a2, const float* w1_dev, const float* w2_dev,
+                                   const float* bias1_host, OperandImage* img) {
+  if (c.num_sms < 2) return c.fail("the fused encoder kernel needs CTA pairs", TIC_ERR_UNSUPPORTED);
   U16Plan pl2{};
-  if (!u16_plan(a2, 0, 2, a2.cout, &pl2)) return fail("fused encoder plan failed", -5);
+  if (!u16_plan(a2, 0, 2, a2.cout, &pl2)) return c.fail("fused encoder plan failed", TIC_ERR_UNSUPPORTED);
   U16Params p2 = pl2.p;
   if (p2.mode != U16_S2 || p2.nbox != 1 || p2.ksteps != 2 || p2.KB != 1 || p2.bn != 1 || p2.npad != 32 || p2.nsplit != 1)
-    return fail("fused encoder: unexpected layer plan", -5);
+    return c.fail("fused encoder: unexpected layer plan", TIC_ERR_UNSUPPORTED);
   FusedEncNorm nm{};
-  for (int c = 0; c < 3; ++c) {
-    nm.mean[c] = a1.mean[c];
-    nm.stdv[c] = a1.stdv[c];
-    nm.m[c] = (int)lrintf(a1.mean[c]);
-    if (!fused_enc_mean_ok(a1.mean[c])) return fail("fused encoder: channel mean outside the exact fp16 integer range", -5);
+  for (int ch = 0; ch < 3; ++ch) {
+    nm.mean[ch] = a1.mean[ch];
+    nm.stdv[ch] = a1.stdv[ch];
+    nm.m[ch] = (int)lrintf(a1.mean[ch]);
+    if (!fused_enc_mean_ok(a1.mean[ch])) return c.fail("fused encoder: channel mean outside the exact fp16 integer range", TIC_ERR_UNSUPPORTED);
   }
-  if (!fw->w1 || memcmp(&fw->nm, &nm, sizeof(nm)) != 0) {
-    // (a rebuild on the same stream is ordered behind the launches that still read the old image)
-    if (!fw->w1 && cudaMalloc(&fw->w1, 2 * 4608) != cudaSuccess) return fail("cudaMalloc for the fused first-layer weight image failed", -4);
-    fw->nm = nm;
-    f16_build_weights_s2_pair_kernel<<<8, 256, 0, stream>>>(w1_dev, a1.cout, fw->w1, nm);
-    if (cudaGetLastError() != cudaSuccess) return fail("fused first-layer weight image kernel failed", -2);
+  bool build;  // (tic_set_norm after the first launch changes nm: the image is rebuilt)
+  if (img[0].ensure(image_key(w1_dev, a1.cout, nm), 2 * 4608, &build) != TIC_OK)
+    return c.fail("cudaMalloc for the fused first-layer weight image failed", TIC_ERR_NOMEM);
+  if (build) {
+    f16_build_weights_s2_pair_kernel<<<8, 256, 0, c.stream>>>(w1_dev, a1.cout, img[0].buf.as<uint8_t>(), nm);
+    if (cudaGetLastError() != cudaSuccess) return c.fail("fused first-layer weight image kernel failed", TIC_ERR_CUDA);
   }
-  if (u16_ensure_pair_weights(stream, w2_dev, a2, p2, &fw->w2) != 0) return fail("fused encoder: weight images failed", -2);
-  p2.wimg = fw->w2.img;
+  if (tic_status s = u16_pair_image(c.stream, img[1], w2_dev, a2, p2, 0, a2.cout)) return c.fail("fused encoder: weight images failed", s);
+  p2.wimg = img[1].img();
   p2.dbg = tic_env_int("TIC_DBG", 0);  // -DTIC_ABLATE builds only: 1 no MMA2, 16 no MMA1, 2 no epilogue 2, 4 no region writes, 8 no builders
 
   FusedEncParams fp{};
@@ -630,8 +615,8 @@ inline int launch_fused_enc(cudaStream_t stream, const LayerArgs& a1, const Laye
   fp.tiles_y = a2.hout / 16;
   fp.tiles_pp = fp.tiles_x * fp.tiles_y;
   fp.pairs_total = ((long long)a1.n + 1) / 2;
-  fp.w1img = fw->w1;
-  for (int c = 0; c < 3; ++c) fp.moff[c] = nm.m[c];
+  fp.w1img = img[0].img();
+  for (int ch = 0; ch < 3; ++ch) fp.moff[ch] = nm.m[ch];
   for (int i = 0; i < 32; ++i) fp.bias1[i] = i < a1.cout ? bias1_host[i] : 0.f;
   auto up = [](uint32_t v) { return (v + 1023u) & ~1023u; };
   uint32_t off = 0;
@@ -656,45 +641,21 @@ inline int launch_fused_enc(cudaStream_t stream, const LayerArgs& a1, const Laye
   fp.bars_off = off;
   off += (uint32_t)sizeof(FusedEncBars);
   fp.smem_bytes = off + 1024u;
-  if (fp.smem_bytes + 1024u /* static: bias, alignment */ > 227u * 1024u) return fail("fused encoder: shared memory plan does not fit", -5);
+  if (fp.smem_bytes + 1024u /* static: bias, alignment */ > 227u * 1024u)
+    return c.fail("fused encoder: shared memory plan does not fit", TIC_ERR_UNSUPPORTED);
 
-  // raw image windows: 3-D map over [B, H, W * 3] bytes, box 65 rows x 112 bytes
+  // raw image windows: box 65 rows x 112 bytes; encode_1's output planes
   CUtensorMap tm_img, tm_o[2];
-  {
-    const Geo& g = a1.geo;
-    const long long per_img = (long long)g.gh * g.gw;
-    const cuuint64_t nimg = (cuuint64_t)((g.n0 + a1.n + per_img - 1) / per_img);
-    cuuint64_t dims[3] = {(cuuint64_t)g.W * 3, (cuuint64_t)g.H, nimg};
-    cuuint64_t strides[2] = {(cuuint64_t)g.W * 3, (cuuint64_t)g.H * g.W * 3};
-    cuuint32_t box[3] = {kFERawRow, (cuuint32_t)kFEOpRows, 1};
-    cuuint32_t es[3] = {1, 1, 1};
-    CUresult r = encode(&tm_img, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(a1.in), dims, strides, box, es,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled (image windows) failed (" + std::to_string((int)r) + ")", -2);
-  }
-  {  // encode_1's output planes: box = one epilogue warp's 4 rows x 8 columns x 32 channels
-    const cuuint64_t C = a2.cout, Wd = a2.wout, Hd = a2.hout, Nd = a2.n;
-    cuuint64_t dims[4] = {C, Wd, Hd, Nd};
-    cuuint64_t strides[3] = {C * 2, Wd * C * 2, Hd * Wd * C * 2};
-    cuuint32_t box[4] = {32, 8, 4, 1};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    for (int pl = 0; pl < 2; ++pl) {
-      void* base = reinterpret_cast<__half*>(a2.out) + (pl ? a2.out_lo_off : 0);
-      CUresult r = encode(&tm_o[pl], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled (fused encoder output) failed (" + std::to_string((int)r) + ")", -2);
-    }
-  }
-  static SmemAttrCache cache;
-  if (cache.ensure(reinterpret_cast<const void*>(fused_enc_kernel), fp.smem_bytes) != cudaSuccess)
-    return fail("cudaFuncSetAttribute(fused encoder) failed", -2);
-  const int grid = 2 * (int)std::min<long long>(fp.pairs_total, num_sms / 2);
-  fused_enc_kernel<<<grid, kFEThreads, fp.smem_bytes, stream>>>(tm_img, tm_o[0], tm_o[1], a1, p2, a2, fp);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return fail(std::string("fused encoder launch failed: ") + cudaGetErrorString(e), -2);
-  if (launches) ++*launches;
-  return 0;
+  if (tic_status s = tmap_image_rows(&tm_img, a1, false, kFERawRow, kFEOpRows, "image windows", c.err)) return s;
+  for (int pl = 0; pl < 2; ++pl)
+    if (tic_status s = tmap_pair_out(&tm_o[pl], reinterpret_cast<__half*>(a2.out) + (pl ? a2.out_lo_off : 0), a2.n, a2.hout, a2.wout,
+                                     a2.cout, "fused encoder output", c.err))
+      return s;
+  const int grid = 2 * (int)std::min<long long>(fp.pairs_total, c.num_sms / 2);
+  const cudaError_t e = launch_dyn(fused_enc_kernel, grid, kFEThreads, fp.smem_bytes, c.stream, tm_img, tm_o[0], tm_o[1], a1, p2, a2, fp);
+  if (e != cudaSuccess) return c.fail(std::string("fused encoder launch failed: ") + cudaGetErrorString(e), TIC_ERR_CUDA);
+  ++*c.launches;
+  return TIC_OK;
 }
 
 }  // namespace tic

@@ -22,11 +22,11 @@
 // 3 TMEM allocator, 4-7 lo-converters, 8-11 epilogue (TMEM -> registers -> bias/act/residual/quantise -> global).
 #pragma once
 #include <cuda.h>
-#include <cudaTypedefs.h>
 
 #include <string>
 
 #include "tic_common.cuh"
+#include "tic_launch.cuh"
 #include "tic_ptx.cuh"
 #include "tic_simt.cuh"
 
@@ -64,24 +64,6 @@ struct UmmaParams {
   int three_pass;
   const uint8_t* wimg;     // weight images, groups consecutive
   int oc0;                 // first output channel of this launch (layers with cout > 64 run in 64-channel slices)
-};
-
-struct UmmaWeightSlice {
-  uint8_t* img = nullptr;
-  size_t bytes = 0;
-  int mode = -1;
-  void release() {
-    if (img) cudaFree(img);
-    img = nullptr;
-    bytes = 0;
-    mode = -1;
-  }
-};
-struct UmmaWeights {
-  UmmaWeightSlice slice[4];  // layers with cout > 64 run as 64-channel slices
-  void release() {
-    for (auto& sl : slice) sl.release();
-  }
 };
 
 // Tap order inside a weight group.  S1/S2 group (kb, kw): kh = 0,1,2.  DECONV group (kb, 0) = input
@@ -459,18 +441,6 @@ umma_conv_kernel(const __grid_constant__ CUtensorMap tmap, const UmmaParams p, c
 }
 
 // ---- host side -------------------------------------------------------------------------------
-inline PFN_cuTensorMapEncodeTiled_v12000 umma_encode_fn() {
-  static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(p);
-  }
-  return fn;
-}
-
 inline int umma_mode_of(int kind, int stride) { return kind == 1 ? UMMA_DECONV : (stride == 2 ? UMMA_S2 : UMMA_S1); }
 
 // Which layers the tensor path takes; everything else (first layer with 3 input channels, fused u8
@@ -491,27 +461,8 @@ inline bool umma_supported(const LayerArgs& a, int kind, int stride) {
   return true;
 }
 
-template <int MODE, bool THREE_PASS>
-inline cudaError_t umma_launch_t(cudaStream_t stream, const CUtensorMap& tm, const UmmaParams& p, const LayerArgs& a, int grid,
-                                 size_t smem) {
-  auto k = umma_conv_kernel<MODE, THREE_PASS>;
-  static SmemAttrCache cache;
-  {
-    cudaError_t e = cache.ensure(reinterpret_cast<const void*>(k), smem);
-    if (e != cudaSuccess) return e;
-  }
-  k<<<grid, kUmmaThreads, smem, stream>>>(tm, p, a);
-  return cudaGetLastError();
-}
-
-inline int launch_umma_slice(cudaStream_t stream, const LayerArgs& a, int kind, int stride, const float* w_dev,
-                             UmmaWeightSlice* uw, int oc0, int cs, bool three_pass, int num_sms, std::string* err) {
-  auto fail = [&](const char* what, int code) {
-    if (err) *err = what;
-    return code;
-  };
-  auto encode = umma_encode_fn();
-  if (!encode) return fail("cuTensorMapEncodeTiled is unavailable (driver too old?)", -2);
+inline tic_status launch_umma_slice(const LaunchCtx& c, const LayerArgs& a, int kind, int stride, const float* w_dev,
+                                    OperandImage& img, int oc0, int cs, bool three_pass) {
   UmmaParams p{};
   p.mode = umma_mode_of(kind, stride);
   p.n = a.n;
@@ -539,7 +490,7 @@ inline int launch_umma_slice(cudaStream_t stream, const LayerArgs& a, int kind, 
     p.nacc = (p.split_kw ? 3 : 1) + p.split_lo;
   }
   p.T = std::min(kMaxTiles, 512 / (p.npad * p.nacc));
-  if (p.T < 1) return fail("accumulators do not fit TMEM", -5);
+  if (p.T < 1) return c.fail("accumulators do not fit TMEM", TIC_ERR_UNSUPPORTED);
   p.num_super = (p.num_tiles + p.T - 1) / p.T;
   p.three_pass = three_pass ? 1 : 0;
   p.tap_bytes = 2u * p.npad * 128u;
@@ -572,75 +523,47 @@ inline int launch_umma_slice(cudaStream_t stream, const LayerArgs& a, int kind, 
   p.S = (int)std::min<size_t>(kMaxStages, (budget - 2 * (size_t)p.wbuf_bytes) / stage);
   if (budget < 2 * (size_t)p.wbuf_bytes || p.S < 2) {
     p.WB = 1;
-    if (budget < p.wbuf_bytes) return fail("weight group does not fit shared memory", -5);
+    if (budget < p.wbuf_bytes) return c.fail("weight group does not fit shared memory", TIC_ERR_UNSUPPORTED);
     p.S = (int)std::min<size_t>(kMaxStages, (budget - p.wbuf_bytes) / stage);
   }
-  if (p.S < 1) return fail("A stages do not fit shared memory", -5);
+  if (p.S < 1) return c.fail("A stages do not fit shared memory", TIC_ERR_UNSUPPORTED);
   const size_t smem = (size_t)p.WB * p.wbuf_bytes + (size_t)p.S * stage + sizeof(UmmaSmemBars) + 1024;
 
   // weight images (once per layer and mode)
-  const size_t wbytes = (size_t)p.KB * 9 * p.tap_bytes;
-  if (!uw->img || uw->bytes != wbytes || uw->mode != p.mode) {
-    uw->release();
-    if (cudaMalloc(&uw->img, wbytes) != cudaSuccess) return fail("cudaMalloc for weight images failed", -4);
-    uw->bytes = wbytes;
-    uw->mode = p.mode;
-    umma_build_weights_kernel<<<64, 256, 0, stream>>>(w_dev, a.cin, a.cout, oc0, p.npad, p.mode, p.KB, p.gw, uw->img);
-    if (cudaGetLastError() != cudaSuccess) return fail("weight image kernel failed", -2);
+  bool build;
+  if (img.ensure(image_key(w_dev, a.cin, a.cout, oc0, p.npad, p.mode, p.KB, p.gw), (size_t)p.KB * 9 * p.tap_bytes, &build) != TIC_OK)
+    return c.fail("cudaMalloc for weight images failed", TIC_ERR_NOMEM);
+  if (build) {
+    umma_build_weights_kernel<<<64, 256, 0, c.stream>>>(w_dev, a.cin, a.cout, oc0, p.npad, p.mode, p.KB, p.gw, img.buf.as<uint8_t>());
+    if (cudaGetLastError() != cudaSuccess) return c.fail("weight image kernel failed", TIC_ERR_CUDA);
   }
-  p.wimg = uw->img;
+  p.wimg = img.img();
 
   // tensor map over the input activation [n, hin, win, cin] fp32
   CUtensorMap tm;
-  CUresult r;
-  const cuuint64_t C = a.cin, W = a.win, H = a.hin, N = a.n;
-  if (p.mode != UMMA_S2) {
-    cuuint64_t dims[4] = {C, W, N, H};
-    cuuint64_t strides[3] = {C * 4, H * W * C * 4, W * C * 4};
-    cuuint32_t box[4] = {32, 8, (cuuint32_t)p.bn, (cuuint32_t)(p.bh + (p.mode == UMMA_S1 ? 2 : 1))};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    r = encode(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<void*>(a.in), dims, strides, box, es,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  } else {
-    cuuint64_t dims[5] = {2 * C, W / 2, 2, N, H / 2};
-    cuuint64_t strides[4] = {2 * C * 4, W * C * 4, H * W * C * 4, 2 * W * C * 4};
-    cuuint32_t box[5] = {32, 8, 2, (cuuint32_t)p.bn, (cuuint32_t)(p.bh + 1)};
-    cuuint32_t es[5] = {1, 1, 1, 1, 1};
-    r = encode(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, const_cast<void*>(a.in), dims, strides, box, es,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  }
-  if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled failed", -2);
+  const cuuint32_t box[4] = {32, 8, (cuuint32_t)p.bn, (cuuint32_t)(p.bh + (p.mode == UMMA_S1 ? 2 : 1))};
+  if (tic_status s = tmap_act(&tm, a.in, false, a, p.mode == UMMA_S2, box, CU_TENSOR_MAP_SWIZZLE_128B, c.err)) return s;
 
-  const int grid = (int)std::min<long long>(p.num_super, num_sms);
-  cudaError_t e;
-  if (p.mode == UMMA_S1)
-    e = three_pass ? umma_launch_t<UMMA_S1, true>(stream, tm, p, a, grid, smem) : umma_launch_t<UMMA_S1, false>(stream, tm, p, a, grid, smem);
-  else if (p.mode == UMMA_S2)
-    e = three_pass ? umma_launch_t<UMMA_S2, true>(stream, tm, p, a, grid, smem) : umma_launch_t<UMMA_S2, false>(stream, tm, p, a, grid, smem);
-  else
-    e = three_pass ? umma_launch_t<UMMA_DECONV, true>(stream, tm, p, a, grid, smem)
-                   : umma_launch_t<UMMA_DECONV, false>(stream, tm, p, a, grid, smem);
-  if (e != cudaSuccess) {
-    if (err) *err = std::string("tensor-path launch failed: ") + cudaGetErrorString(e);
-    return -2;
-  }
-  return 0;
+  const int grid = (int)std::min<long long>(p.num_super, c.num_sms);
+  auto kernel = p.mode == UMMA_S1 ? (three_pass ? umma_conv_kernel<UMMA_S1, true> : umma_conv_kernel<UMMA_S1, false>)
+                : p.mode == UMMA_S2 ? (three_pass ? umma_conv_kernel<UMMA_S2, true> : umma_conv_kernel<UMMA_S2, false>)
+                                    : (three_pass ? umma_conv_kernel<UMMA_DECONV, true> : umma_conv_kernel<UMMA_DECONV, false>);
+  const cudaError_t e = launch_dyn(kernel, grid, kUmmaThreads, smem, c.stream, tm, p, a);
+  if (e != cudaSuccess) return c.fail(std::string("tensor-path launch failed: ") + cudaGetErrorString(e), TIC_ERR_CUDA);
+  return TIC_OK;
 }
 
 // A layer with more than 64 output channels runs as 64-channel slices (same A tiles, disjoint weight
 // rows and output channels): N = 64 keeps four split accumulators x two tiles inside the 512 TMEM columns.
-inline int launch_umma(cudaStream_t stream, const LayerArgs& a, int kind, int stride, const float* w_dev, UmmaWeights* uw,
-                       bool three_pass, int num_sms, std::string* err, int* launches) {
+inline tic_status launch_umma(const LaunchCtx& c, const LayerArgs& a, int kind, int stride, const float* w_dev, OperandImage* slices,
+                              bool three_pass) {
   int si = 0;
   for (int oc0 = 0; oc0 < a.cout; oc0 += 64, ++si) {
     const int cs = std::min(64, a.cout - oc0);
-    int rc = launch_umma_slice(stream, a, kind, stride, w_dev, &uw->slice[si], oc0, cs, three_pass, num_sms, err);
-    if (rc != 0) return rc;
-    if (launches) ++*launches;
+    if (tic_status s = launch_umma_slice(c, a, kind, stride, w_dev, slices[si], oc0, cs, three_pass)) return s;
+    ++*c.launches;
   }
-  return 0;
+  return TIC_OK;
 }
 
 }  // namespace tic

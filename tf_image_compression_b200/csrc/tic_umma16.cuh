@@ -33,12 +33,12 @@
 // lane quadrant, alternating 16-column chunks).
 #pragma once
 #include <cuda.h>
-#include <cudaTypedefs.h>
 #include <cuda_fp16.h>
 
 #include <string>
 
 #include "tic_common.cuh"
+#include "tic_launch.cuh"
 #include "tic_ptx.cuh"
 #include "tic_simt.cuh"
 
@@ -92,24 +92,6 @@ struct U16Params {
   uint32_t wB_bytes;     // pair: per-CTA bytes of its half of W_hi for the A_lo' x W_hi product
   long long in_lo_off;   // elements between the hi and lo' planes of the input (unused by the kernel: second tensor map)
   int dbg;               // measurement aid (env TIC_DBG, pair kernel): 1 = no MMA issue, 2 = no TMA loads, 4 = no epilogue work
-};
-
-struct U16WeightSlice {
-  uint8_t* img = nullptr;
-  size_t bytes = 0;
-  int mode = -1, npad = 0, oc0 = -1;
-  void release() {
-    if (img) cudaFree(img);
-    img = nullptr;
-    bytes = 0;
-    mode = -1;
-  }
-};
-struct U16Weights {
-  U16WeightSlice slice[16];
-  void release() {
-    for (auto& sl : slice) sl.release();
-  }
 };
 
 __host__ __device__ inline uint32_t u16_swz(uint32_t off, uint32_t rowbytes) {
@@ -1013,14 +995,8 @@ inline bool u16_supported(const LayerArgs& a, int kind, int stride) {
 template <int MODE, int PPS, int EW>
 inline cudaError_t u16_launch_pair_ew(cudaStream_t stream, const CUtensorMap& th, const CUtensorMap& tl, const U16Params& p,
                                       const LayerArgs& a, int grid, size_t smem) {
-  auto k = u16_pair_kernel<MODE, PPS, EW>;
-  static SmemAttrCache cache;
-  {
-    cudaError_t e = cache.ensure(reinterpret_cast<const void*>(k), smem);
-    if (e != cudaSuccess) return e;
-  }
-  k<<<grid, 128 + 32 * EW, smem, stream>>>(th, tl, p, a);  // __cluster_dims__(2, 1, 1): grid is even
-  return cudaGetLastError();
+  // __cluster_dims__(2, 1, 1): grid is even
+  return launch_dyn(u16_pair_kernel<MODE, PPS, EW>, grid, 128 + 32 * EW, smem, stream, th, tl, p, a);
 }
 template <int MODE, int PPS>
 inline cudaError_t u16_launch_pair_pps(cudaStream_t stream, const CUtensorMap& th, const CUtensorMap& tl, const U16Params& p,
@@ -1175,15 +1151,25 @@ inline bool u16_plan(const LayerArgs& a, int kind, int stride, int cs, U16Plan* 
   return true;
 }
 
-inline int launch_u16(cudaStream_t stream, const LayerArgs& a, int kind, int stride, const float* w_dev, U16Weights* uw,
-                      int num_sms, std::string* err, int* launches) {
-  auto fail = [&](const std::string& what, int code) {
-    if (err) *err = what;
-    return code;
-  };
-  auto encode = umma_encode_fn();
-  if (!encode) return fail("cuTensorMapEncodeTiled is unavailable (driver too old?)", -2);
-  if (num_sms < 2) return fail("the fp16-pair tensor kernels need CTA pairs", -5);
+// The CTA-pair weight image of output channels [oc0, oc0 + cs) of a layer for plan p (u16_build_weights_pair_kernel).
+inline tic_status u16_pair_image(cudaStream_t stream, OperandImage& img, const float* w_dev, const LayerArgs& a, const U16Params& p,
+                                 int oc0, int cs) {
+  const uint32_t regA = (p.wA_bytes + 1023u) & ~1023u, regB = (p.wB_bytes + 1023u) & ~1023u;
+  const int ph_mode = p.mode == U16_DECONV_PH;
+  bool build;
+  if (img.ensure(image_key(w_dev, a.cin, a.cout, oc0, cs, p.npad, p.cpad, ph_mode, p.kc, p.KB, regA, regB), 2 * (size_t)p.w_bytes,
+                 &build) != TIC_OK)
+    return TIC_ERR_NOMEM;
+  if (build) {
+    u16_build_weights_pair_kernel<<<64, 256, 0, stream>>>(w_dev, a.cin, a.cout, oc0, cs, p.npad, p.cpad, ph_mode, p.kc, p.KB, regA,
+                                                          regB, img.buf.as<uint8_t>());
+    if (cudaGetLastError() != cudaSuccess) return TIC_ERR_CUDA;
+  }
+  return TIC_OK;
+}
+
+inline tic_status launch_u16(const LaunchCtx& c, const LayerArgs& a, int kind, int stride, const float* w_dev, OperandImage* slices) {
+  if (c.num_sms < 2) return c.fail("the fp16-pair tensor kernels need CTA pairs", TIC_ERR_UNSUPPORTED);
   // widest output-channel slice whose weights stay resident
   U16Plan plan{};
   int cs = std::min(a.cout, 128);
@@ -1203,76 +1189,48 @@ inline int launch_u16(cudaStream_t stream, const LayerArgs& a, int kind, int str
     if (!ok && small_kc) ok = u16_plan(a, kind, stride, csl, &plan, 1) || u16_plan(a, kind, stride, csl, &plan, 3);
     if (ok) break;
   }
-  if (!ok) return fail("layer does not fit the fp16-pair tensor path", -5);
+  if (!ok) return c.fail("layer does not fit the fp16-pair tensor path", TIC_ERR_UNSUPPORTED);
   cs = plan.cs;
 
   // tensor maps over the two planes of the input activation [n, hin, win, cin] fp16
   CUtensorMap tm[2];
   const U16Params& p0 = plan.p;
-  const cuuint64_t C = a.cin, W = a.win, H = a.hin, N = a.n;
-  for (int pl = 0; pl < 2; ++pl) {
-    void* base = const_cast<__half*>(reinterpret_cast<const __half*>(a.in) + (pl ? a.in_lo_off : 0));
-    CUresult r;
-    const CUtensorMapSwizzle sw = p0.a_layout == 2 ? CU_TENSOR_MAP_SWIZZLE_128B
-                                  : p0.a_layout == 4 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
-    if (p0.mode != U16_S2) {
-      cuuint64_t dims[4] = {C, W, N, H};
-      cuuint64_t strides[3] = {C * 2, H * W * C * 2, W * C * 2};
-      cuuint32_t box[4] = {(cuuint32_t)p0.kc, (cuuint32_t)(p0.mode == U16_S1 ? 10 : 9), (cuuint32_t)p0.bn,
-                           (cuuint32_t)(p0.bh + (p0.mode == U16_S1 ? 2 : 1))};
-      cuuint32_t es[4] = {1, 1, 1, 1};
-      r = encode(&tm[pl], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                 CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    } else {
-      cuuint64_t dims[5] = {2 * C, W / 2, 2, N, H / 2};
-      cuuint64_t strides[4] = {2 * C * 2, W * C * 2, H * W * C * 2, 2 * W * C * 2};
-      cuuint32_t box[5] = {(cuuint32_t)(p0.nbox == 1 ? 2 * p0.kc : p0.kc), 9, 2, (cuuint32_t)p0.bn, (cuuint32_t)(p0.bh + 1)};
-      cuuint32_t es[5] = {1, 1, 1, 1, 1};
-      r = encode(&tm[pl], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                 CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    }
-    if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled failed (" + std::to_string((int)r) + ")", -2);
-  }
+  const CUtensorMapSwizzle sw = p0.a_layout == 2 ? CU_TENSOR_MAP_SWIZZLE_128B
+                                : p0.a_layout == 4 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
+  const cuuint32_t box[4] = {(cuuint32_t)(p0.mode == U16_S2 && p0.nbox == 1 ? 2 * p0.kc : p0.kc), (cuuint32_t)(p0.mode == U16_S1 ? 10 : 9),
+                             (cuuint32_t)p0.bn, (cuuint32_t)(p0.bh + (p0.mode == U16_S1 ? 2 : 1))};
+  for (int pl = 0; pl < 2; ++pl)
+    if (tic_status s = tmap_act(&tm[pl], reinterpret_cast<const __half*>(a.in) + (pl ? a.in_lo_off : 0), true, a, p0.mode == U16_S2, box,
+                                sw, c.err))
+      return s;
 
   int si = 0;
   for (int oc0 = 0; oc0 < a.cout; oc0 += cs, ++si) {
-    if (si >= 16) return fail("too many output-channel slices", -5);
+    if (si >= 16) return c.fail("too many output-channel slices", TIC_ERR_UNSUPPORTED);
     const int csl = std::min(cs, a.cout - oc0);
     U16Plan pl{};
-    if (!u16_plan(a, kind, stride, csl, &pl, plan.variant)) return fail("slice plan failed", -5);
+    if (!u16_plan(a, kind, stride, csl, &pl, plan.variant)) return c.fail("slice plan failed", TIC_ERR_UNSUPPORTED);
     U16Params p = pl.p;
     p.oc0 = oc0;
-    U16WeightSlice* ws = &uw->slice[si];
-    const size_t img_bytes = 2 * (size_t)p.w_bytes;
-    if (!ws->img || ws->bytes != img_bytes || ws->mode != p.mode || ws->npad != p.npad || ws->oc0 != oc0) {
-      ws->release();
-      if (cudaMalloc(&ws->img, img_bytes) != cudaSuccess) return fail("cudaMalloc for weight images failed", -4);
-      ws->bytes = img_bytes;
-      ws->mode = p.mode;
-      ws->npad = p.npad;
-      ws->oc0 = oc0;
-      u16_build_weights_pair_kernel<<<64, 256, 0, stream>>>(w_dev, a.cin, a.cout, oc0, csl, p.npad, p.cpad, p.mode == U16_DECONV_PH,
-                                                            p.kc, p.KB, (p.wA_bytes + 1023u) & ~1023u,
-                                                            (p.wB_bytes + 1023u) & ~1023u, ws->img);
-      if (cudaGetLastError() != cudaSuccess) return fail("weight image kernel failed", -2);
-    }
-    p.wimg = ws->img;
-    const int grid = 2 * (int)std::min<long long>((p.num_tiles + 1) / 2, num_sms / 2);
+    if (tic_status s = u16_pair_image(c.stream, slices[si], w_dev, a, p, oc0, csl))
+      return c.fail(s == TIC_ERR_NOMEM ? "cudaMalloc for weight images failed" : "weight image kernel failed", s);
+    p.wimg = slices[si].img();
+    const int grid = 2 * (int)std::min<long long>((p.num_tiles + 1) / 2, c.num_sms / 2);
     cudaError_t e;
     if (p.mode == U16_S1)
-      e = u16_launch_pair_t<U16_S1>(stream, tm[0], tm[1], p, a, grid, pl.smem);
+      e = u16_launch_pair_t<U16_S1>(c.stream, tm[0], tm[1], p, a, grid, pl.smem);
     else if (p.mode == U16_S2)
-      e = u16_launch_pair_t<U16_S2>(stream, tm[0], tm[1], p, a, grid, pl.smem);
+      e = u16_launch_pair_t<U16_S2>(c.stream, tm[0], tm[1], p, a, grid, pl.smem);
     else if (p.mode == U16_DECONV_PH && p.cpad == 4)
-      e = u16_launch_pair_t<U16_DECONV_RGB>(stream, tm[0], tm[1], p, a, grid, pl.smem);
+      e = u16_launch_pair_t<U16_DECONV_RGB>(c.stream, tm[0], tm[1], p, a, grid, pl.smem);
     else if (p.mode == U16_DECONV_PH)
-      e = u16_launch_pair_t<U16_DECONV_PH>(stream, tm[0], tm[1], p, a, grid, pl.smem);
+      e = u16_launch_pair_t<U16_DECONV_PH>(c.stream, tm[0], tm[1], p, a, grid, pl.smem);
     else
-      e = u16_launch_pair_t<U16_DECONV>(stream, tm[0], tm[1], p, a, grid, pl.smem);
-    if (e != cudaSuccess) return fail(std::string("fp16-pair tensor launch failed: ") + cudaGetErrorString(e), -2);
-    if (launches) ++*launches;
+      e = u16_launch_pair_t<U16_DECONV>(c.stream, tm[0], tm[1], p, a, grid, pl.smem);
+    if (e != cudaSuccess) return c.fail(std::string("fp16-pair tensor launch failed: ") + cudaGetErrorString(e), TIC_ERR_CUDA);
+    ++*c.launches;
   }
-  return 0;
+  return TIC_OK;
 }
 
 }  // namespace tic
